@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s (primary + shadow) and ms/frame of the lasgun render loop on 1/2/4/8 B200.
 
-  python bench.py --gpus N --steps K --warmup W [--workload mixed4k] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--workload mixed4k] [--impl reference] [--dump-outputs DIR]
 
 A step is one full frame of the workload (default: BASELINE.json's config 5, `mixed4k`, 3840x2160 at
 16 spp — the config the 1/2/4/8-GPU metric is quoted on; it fits one GPU).  Rays are counted with the
@@ -19,6 +19,8 @@ reference's semantics: primary = w*h*spp, shadow = lights * primary hits (integr
          no microbenchmark in any denominator.
 --impl reference times the CPU oracle (C++ restatement of the reference algorithm — the Rust build
 cannot be compiled here) on all host threads over a bounded sample of the same frame.
+--dump-outputs DIR writes the film of the last timed step (see dump_outputs), so that two builds run with the same arguments can be
+compared pixel for pixel.
 """
 from __future__ import annotations
 
@@ -34,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -45,6 +48,7 @@ OPS = {"node": 26, "sphere": (26, 39), "tri": (47, 68), "cuboid": 31, "camera": 
        "background": 15, "film": 12}
 BYTES = {"node": 32, "sphere": 16, "tri": 48, "cuboid": 32, "ref": 4, "film": 4}
 OTHER_CONFIGS = ("simple", "mesh1m", "cornell", "spheres1m")
+DUMP_PIXELS = 1 << 21      # --dump-outputs: 32 MiB of f32 RGBA + 16 MiB of f64 pixel indices at most
 
 
 def load_peaks():
@@ -123,6 +127,19 @@ class ClockSampler:
         return out
 
 
+def dump_outputs(path, rgba, pixels=None):
+    """The film a step delivered: DIR/film_rgba.npy (k, 4) float32 RGBA8 values and DIR/film_pixel_index.npy (k,) float64 row-major
+    pixel indices y * width + x.  `pixels` are the indices the step rendered (default: all); of more than DUMP_PIXELS a fixed,
+    seeded sample is kept, so that runs with the same arguments write the same pixels."""
+    flat = np.asarray(rgba).reshape(-1, 4)
+    idx = np.arange(len(flat)) if pixels is None else np.sort(pixels)
+    if len(idx) > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(idx, DUMP_PIXELS, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "film_rgba.npy"), flat[idx].astype(np.float32))
+    np.save(os.path.join(path, "film_pixel_index.npy"), idx.astype(np.float64))
+
+
 def workload(name, args):
     if name == "mixed4k" and args.small:
         return scenes.mixed4k(mesh_n=80, nspheres=8000, res=(480, 270), supersampling=1)
@@ -179,6 +196,8 @@ def run_reference(args):
         r = osc.capture(w, h, threads=threads, counters=True, subset=(n, 0, threads))
         if i >= args.warmup:
             times.append(r["render_ms"]); rays = r["counters"]["primary"] + r["counters"]["shadow"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["rgba"], np.concatenate([np.arange(k, w * h, n) for k in range(threads)]))
     ms = sum(times) / len(times)
     value = rays / (ms * 1e-3) / 1e6
     frame_rays_est = rays * (n / threads)
@@ -334,7 +353,7 @@ def run_gpu(args):
     shared = multi.SharedFilm(ctx, w, h, rank, world, N) if (world > 1 and args.gather == "p2p") else None
 
     def step():
-        multi.capture_distributed(dev, w, h, film, rank, world, stream, shared=shared)
+        return multi.capture_distributed(dev, w, h, film, rank, world, stream, shared=shared)
 
     # one counted frame (not timed): ray counts of the frame, summed over ranks
     st = dev.capture_device(w, h, film.data_ptr(), rank=rank, ranks=world, stream=stream, want_stats=True)
@@ -356,10 +375,12 @@ def run_gpu(args):
     t_region0 = sampler.mark()
     ev[0].record()
     for _ in range(args.steps):
-        step()
+        last = step()
     ev[1].record()
     torch.cuda.synchronize()
     t_region1 = sampler.mark()
+    # the whole frame is on rank 0; copied now, before the measurements below render into the same film
+    last_film = last.cpu().numpy() if args.dump_outputs and rank == 0 else None
     if world > 1:
         dist.barrier()
     clocks = sampler.stop(t_region0, t_region1)
@@ -597,6 +618,8 @@ def run_gpu(args):
                 except Exception as e:      # a failing side measurement must not take the headline line down with it
                     others[name] = {"error": repr(e)}
             line["other_configs"] = others
+        if last_film is not None:
+            dump_outputs(args.dump_outputs, last_film)
         print(json.dumps(line))
     dev.destroy()
     if shared is not None:
@@ -625,7 +648,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-group", action="store_true", help="N>1: skip the one-process device-group measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the film of the last timed step as .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
