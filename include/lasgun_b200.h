@@ -312,8 +312,15 @@ typedef struct lgb_kernel_time {
 int lgb_capture_profile(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, void* d_film,
                         lgb_kernel_time* out, uint32_t cap, uint32_t* n_out, lgb_stats* stats);
 
-/* Trace caller-supplied rays (o[3], d[3] f64 each) through the scene: closest-hit id and t.
- * Used by the known-answer and random-ray parity tests. */
+/* Trace caller-supplied rays (o[3], d[3] f64 each) through the scene: closest-hit id, t and the world-space
+ * RayIntersection::ng() / ns() (surface.rs:107-118; any output pointer may be NULL).
+ * The f32 error bound of the traversal is derived from the world box of the scene and its camera (the reference root box,
+ * through the root transform, united with the camera origin).  The f32 culling ray of an origin outside that box starts where
+ * the ray enters it (grown by 1/64 of its extent), and a direction with max |d_k| outside [2^-40, 2^40] is traced scaled by
+ * an exact power of two; the exact f64 tests give the reference's t either way.  Precondition: every origin lies within one
+ * box extent of that box (so no coordinate is NaN or infinite); otherwise the whole batch is refused with LGB_ERR_UNSUPPORTED
+ * and lgb_last_error names the box.
+ * Used by the known-answer tests (tests/test_gpu_parity.py) and the random-ray parity tests (tests/test_trace_rays.py). */
 int lgb_trace_rays(lgb_ctx* ctx, lgb_scene* scene, const double* rays_od, uint64_t n_rays,
                    uint32_t* prim_id, double* t, double* ng, double* ns);
 

@@ -28,7 +28,7 @@ cudaError_t launch_level(const DevScene&, const DevCamera&, const DevShade&, con
 cudaError_t launch_gather(const SpawnRec* recs, const uint32_t* nspec, double* rad_parent, const double* rad_child, uint64_t n_upper, cudaStream_t);
 cudaError_t launch_resolve(const DevWork&, const DevOut&, cudaStream_t);
 cudaError_t launch_export_li(const DevWork&, const DevOut&, const DevWave&, cudaStream_t);
-cudaError_t launch_trace(const DevScene&, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns, cudaStream_t);
+cudaError_t launch_trace(const DevScene&, const TraceBox&, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns, cudaStream_t);
 cudaError_t launch_l2_read(const void* buf, uint64_t bytes, int iters, float* sink, int sms, cudaStream_t);
 cudaError_t launch_fp32_peak(int iters, float* sink, int sms, cudaStream_t);
 cudaError_t launch_fp64_peak(int iters, double* sink, int sms, cudaStream_t);
@@ -153,6 +153,9 @@ struct lgb_scene {
     DevCamera cam{};
     DevShade shade{};
     double max_abs = 0.0;      // max |coordinate| over geometry, camera origin and lights
+    // world box (scene and camera) the f32 error bound of every space was derived from: the traversal is conservative for rays
+    // whose f32 origin lies inside it, so lgb_trace_rays starts the f32 ray of a caller-supplied origin outside where it enters it
+    double origin_lo[3] = {0, 0, 0}, origin_hi[3] = {0, 0, 0};
     double build_ms = 0.0;     // host time of the device-BVH build inside lgb_scene_create
     double t_validate = 0, t_rank = 0, t_build = 0, t_convert_upload = 0, t_total = 0;   // ms, lgb_scene_create phases
 };
@@ -465,8 +468,8 @@ static int ensure_rank_tables(lgb_ctx* ctx, lgb_scene* s) {
 extern "C" { static int ensure_bvh(lgb_ctx* ctx, lgb_scene* s); }      // (defined inside the extern "C" block below)
 // ---- export / import: the arena is position independent once DevScene's pointers are written as offsets
 namespace {
-struct SceneLayout { uint64_t magic, arena_bytes; DevScene dev; DevCamera cam; DevShade shade; double max_abs; };
-constexpr uint64_t kLayoutMagic = 0x4C47423253434E33ull;       // "LGB2SCN3"
+struct SceneLayout { uint64_t magic, arena_bytes; DevScene dev; DevCamera cam; DevShade shade; double max_abs; double origin_lo[3], origin_hi[3]; };
+constexpr uint64_t kLayoutMagic = 0x4C47423253434E34ull;       // "LGB2SCN4"
 constexpr uint64_t kNullOffset = ~0ull;
 template <class F> void for_each_pointer(DevScene& d, F f) {
     f((const void*&)d.nodes); f((const void*&)d.sph32); f((const void*&)d.sph64); f((const void*&)d.sph_mat); f((const void*&)d.sph_id);
@@ -633,6 +636,7 @@ int lgb_scene_export(const lgb_scene* s, void* layout_out, uint64_t layout_bytes
     if (int rc = ensure_bvh(s->ctx, const_cast<lgb_scene*>(s))) return rc;          // (an importer cannot build the tree: it has no item boxes)
     SceneLayout L{};
     L.magic = kLayoutMagic; L.arena_bytes = s->bytes; L.dev = s->dev; L.cam = s->cam; L.shade = s->shade; L.max_abs = s->max_abs;
+    std::memcpy(L.origin_lo, s->origin_lo, sizeof L.origin_lo); std::memcpy(L.origin_hi, s->origin_hi, sizeof L.origin_hi);
     const char* base = (const char*)s->arena;
     L.dev.grids = nullptr;                             // light grids live outside the arena: the importer builds its own
     for_each_pointer(L.dev, [&](const void*& p) { p = (const void*)(p ? (uint64_t)((const char*)p - base) : kNullOffset); });
@@ -648,6 +652,7 @@ int lgb_scene_import(lgb_ctx* ctx, const void* layout, uint64_t layout_bytes, vo
     lgb_scene* s = new lgb_scene();
     s->ctx = ctx; s->arena = arena_dev; s->owns_arena = false; s->bytes = L.arena_bytes;
     s->dev = L.dev; s->cam = L.cam; s->shade = L.shade; s->max_abs = L.max_abs;
+    std::memcpy(s->origin_lo, L.origin_lo, sizeof s->origin_lo); std::memcpy(s->origin_hi, L.origin_hi, sizeof s->origin_hi);
     const char* base = (const char*)arena_dev;
     bool ok = true;
     // every array must lie inside the arena with its whole extent (counts recomputed from the leaf words would need the nodes:
@@ -832,6 +837,7 @@ static int replicate_to_peers(lgb_ctx* ctx, lgb_scene* s) {
         lgb_scene* r = new lgb_scene();
         r->ctx = p; r->arena = arena; r->owns_arena = true; r->bytes = s->bytes; r->gpu_built = s->gpu_built;
         r->dev = s->dev; r->cam = s->cam; r->shade = s->shade; r->max_abs = s->max_abs;
+        std::memcpy(r->origin_lo, s->origin_lo, sizeof r->origin_lo); std::memcpy(r->origin_hi, s->origin_hi, sizeof r->origin_hi);
         r->lazy_fn = s->lazy_fn; r->lazy_user = s->lazy_user; r->lazy_desc = s->lazy_desc;
         for_each_pointer(r->dev, [&](const void*& q) { if (q) q = (const char*)arena + ((const char*)q - base); });
         s->replicas.push_back(r);
@@ -968,6 +974,7 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
         for (int k = 0; k < 3; k++) {
             if (std::isfinite(d->camera.origin[k])) { wlo[k] = std::min(wlo[k], d->camera.origin[k] - slack); whi[k] = std::max(whi[k], d->camera.origin[k] + slack); }
         }
+        for (int k = 0; k < 3; k++) { s->origin_lo[k] = wlo[k]; s->origin_hi[k] = whi[k]; }
     }
 
     // ---- device acceleration structure: one binned-SAH BVH per space over the same primitives, rank tables from
@@ -1904,6 +1911,29 @@ int lgb_capture_profile(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void* 
 
 int lgb_trace_rays(lgb_ctx* c, lgb_scene* s, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns) {
     if (!c || !s || (!rays && n)) return fail(c, LGB_ERR_INVALID, "lgb_trace_rays: NULL argument");
+    // The f32 error bound of the traversal is derived from the box of the scene and its camera (lgb_scene::origin_lo/hi).  k_trace
+    // starts the f32 ray of an origin outside it where the ray enters the box grown by 1/64 of its extent.  Origins farther out
+    // than one extent E of the box are refused: there the reference's own f64 tests lose so much to cancellation (a sphere's
+    // |o - c|^2 - r^2) that their hits stray from the surface by more than the conservative culls allow for.
+    TraceBox B;
+    double M = 0.0, E = 0.0;
+    for (int k = 0; k < 3; k++) {
+        M = std::max(M, std::max(std::fabs(s->origin_lo[k]), std::fabs(s->origin_hi[k])));
+        E = std::max(E, s->origin_hi[k] - s->origin_lo[k]);
+    }
+    E += M * std::ldexp(1.0, -10);
+    for (int k = 0; k < 3; k++) { B.lo[k] = s->origin_lo[k] - E / 64.0; B.hi[k] = s->origin_hi[k] + E / 64.0; }
+    for (uint64_t i = 0; i < n; i++) {
+        const double* o = rays + 6 * i;
+        for (int k = 0; k < 3; k++) {
+            if (o[k] >= s->origin_lo[k] - E && o[k] <= s->origin_hi[k] + E) continue;
+            char msg[400];
+            std::snprintf(msg, sizeof msg, "lgb_trace_rays: the origin (%.17g, %.17g, %.17g) of ray %llu lies more than %.17g (one extent) outside the box "
+                          "[%.17g, %.17g] x [%.17g, %.17g] x [%.17g, %.17g] of the scene and its camera", o[0], o[1], o[2], (unsigned long long)i, E,
+                          s->origin_lo[0], s->origin_hi[0], s->origin_lo[1], s->origin_hi[1], s->origin_lo[2], s->origin_hi[2]);
+            return fail(c, LGB_ERR_UNSUPPORTED, msg);
+        }
+    }
     CU(c, cudaSetDevice(c->device));
     if (int rc = ensure_bvh(c, s)) return rc;
     if (n == 0) return LGB_OK;
@@ -1914,7 +1944,7 @@ int lgb_trace_rays(lgb_ctx* c, lgb_scene* s, const double* rays, uint64_t n, uin
     uint32_t* d_id = (uint32_t*)(base + n * 104);
     CU(c, cudaMemcpyAsync(d_rays, rays, n * 48, cudaMemcpyHostToDevice, c->stream));
     if (int rc = sync_scene_copy(c, s, c->stream)) return rc;
-    CU(c, launch_trace(s->dev, d_rays, n, d_id, d_t, d_ng, d_ns, c->stream));
+    CU(c, launch_trace(s->dev, B, d_rays, n, d_id, d_t, d_ng, d_ns, c->stream));
     if (ids) CU(c, cudaMemcpyAsync(ids, d_id, n * 4, cudaMemcpyDeviceToHost, c->stream));
     if (ts) CU(c, cudaMemcpyAsync(ts, d_t, n * 8, cudaMemcpyDeviceToHost, c->stream));
     if (ng) CU(c, cudaMemcpyAsync(ng, d_ng, n * 24, cudaMemcpyDeviceToHost, c->stream));

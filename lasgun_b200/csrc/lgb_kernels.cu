@@ -67,9 +67,11 @@ __device__ __forceinline__ float clamp_idir(float d) {
     return fabsf(v) > 1e30f ? copysignf(1e30f, v) : v;
 }
 
-__device__ __forceinline__ RayF make_rayf(const Ray64& r, float err_abs) {
+// The f32 ray starts at `o` (a point of the line of r): r.o itself, or for caller-supplied rays from far away the point where the
+// line enters the scene's box (k_trace).  The f64 exact tests always see r.
+__device__ __forceinline__ RayF make_rayf_at(const Ray64& r, const D3 o, float err_abs) {
     RayF f;
-    f.ox = (float)r.o.x; f.oy = (float)r.o.y; f.oz = (float)r.o.z;
+    f.ox = (float)o.x; f.oy = (float)o.y; f.oz = (float)o.z;
     f.dx = (float)r.d.x; f.dy = (float)r.d.y; f.dz = (float)r.d.z;
     // dir_is_neg[a] = (1 / d[a] < 0) (bvh.rs:463, ray.rs:28-33) is the sign bit of d[a], -0 included: no f64 division needed
     f.oct = (signbit(r.d.x) ? 1u : 0u) | (signbit(r.d.y) ? 2u : 0u) | (signbit(r.d.z) ? 4u : 0u);
@@ -89,6 +91,12 @@ __device__ __forceinline__ RayF make_rayf(const Ray64& r, float err_abs) {
     f.sx = -fdx * f.sz;
     f.sy = -fdy * f.sz;
     return f;
+}
+__device__ __forceinline__ RayF make_rayf(const Ray64& r, float err_abs) { return make_rayf_at(r, r.o, err_abs); }
+// The f32 ray of r advanced to parameter t0 >= 0 (k_trace).  Its t values are those of r minus t0: every cull that compares them
+// with the best hit only gets weaker, and nothing the scene holds lies before t0 (t0 is the entry into a box around the scene).
+__device__ __forceinline__ RayF make_rayf(const Ray64& r, float err_abs, double t0) {
+    return make_rayf_at(r, d3(r.o.x + t0 * r.d.x, r.o.y + t0 * r.d.y, r.o.z + t0 * r.d.z), err_abs);
 }
 
 // Conservative slab test of an f32 ray against a padded f32 box (DESIGN.md §4.1): returns false only if the
@@ -436,9 +444,9 @@ __device__ __forceinline__ bool prim_exact(const DevScene& S, const Ray64& world
 // spaces; entering one defers the rest of the leaf and an exit marker (count field 31, payload = space to return to).
 constexpr uint32_t kInstLeaf = kLeafBit | ((uint32_t)LGB_PRIM_INSTANCE << 29);
 constexpr uint32_t kExitMarker = kInstLeaf | (31u << 24);
-template <bool ANYHIT, bool STATS, bool REFILL, bool INST>
+template <bool ANYHIT, bool STATS, bool REFILL, bool INST, bool SHIFT = false>
 __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, Ray64& ray, RayF& f, Trav& T, uint32_t* stack, float* tstack, double tmax,
-                                         LocalCounters& lc, int refill_below, unsigned octw, const float4* top = nullptr, const int stride = 1) {
+                                         LocalCounters& lc, int refill_below, unsigned octw, const float4* top = nullptr, const int stride = 1, double t0 = 0.0) {
     Hit& best = T.best;
     float& best_tf = T.best_tf; float& best_up = T.best_up;
     uint32_t& cur = T.cur; int& sp = T.sp;
@@ -461,7 +469,7 @@ __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, 
                 if (count == 32u) {                                   // exit marker: the nested level is done
                     T.space = first;
                     ray = ray_to_space(S, first, world);
-                    f = make_rayf(ray, S.spaces[first].err_abs);
+                    f = SHIFT ? make_rayf(ray, S.spaces[first].err_abs, t0) : make_rayf(ray, S.spaces[first].err_abs);
                 } else {
                     if (count > 1u) { if (!ANYHIT && LGB_TSTACK) tstack[LGB_STK(sp)] = -CUDART_INF_F; stack[LGB_STK(sp)] = kInstLeaf | ((count - 2u) << 24) | (first + 1u); sp++; }
                     if (!ANYHIT && LGB_TSTACK) tstack[LGB_STK(sp)] = -CUDART_INF_F;
@@ -469,7 +477,7 @@ __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, 
                     const uint32_t child = __ldg(&S.inst_space[first]);
                     const DevSpace& c = S.spaces[child];
                     if (!(c.flags & kSpaceIdentity)) ray = ray_into(c, ray);
-                    f = make_rayf(ray, c.err_abs);
+                    f = SHIFT ? make_rayf(ray, c.err_abs, t0) : make_rayf(ray, c.err_abs);
                     T.space = child;
                     cur = c.root_node;
                     continue;
@@ -482,8 +490,8 @@ __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, 
 }
 
 // First ray of a traversal: the world ray in space 0 (the root aggregate may itself be transformed).
-template <bool INST>
-__device__ __forceinline__ void enter_root(const DevScene& S, const Ray64& world, Ray64& ray, RayF& f, Trav& T, double tmax) {
+template <bool INST, bool SHIFT = false>
+__device__ __forceinline__ void enter_root(const DevScene& S, const Ray64& world, Ray64& ray, RayF& f, Trav& T, double tmax, double t0 = 0.0) {
     ray = world;
     float err = S.err_abs;
     uint32_t root = 0;
@@ -492,16 +500,16 @@ __device__ __forceinline__ void enter_root(const DevScene& S, const Ray64& world
         if (!(s0.flags & kSpaceIdentity)) ray = ray_into(s0, world);
         err = s0.err_abs; root = s0.root_node;
     }
-    f = make_rayf(ray, err);
+    f = SHIFT ? make_rayf(ray, err, t0) : make_rayf(ray, err);
     T.init(tmax, root);
 }
-template <bool ANYHIT, bool STATS, bool INST>
-__device__ Hit traverse(const DevScene& S, const Ray64& world, double tmax, LocalCounters& lc) {
+template <bool ANYHIT, bool STATS, bool INST, bool SHIFT = false>
+__device__ Hit traverse(const DevScene& S, const Ray64& world, double tmax, LocalCounters& lc, double t0 = 0.0) {
     Ray64 ray; RayF f; Trav T;
-    enter_root<INST>(S, world, ray, f, T, tmax);
+    enter_root<INST, SHIFT>(S, world, ray, f, T, tmax, t0);
     uint32_t stack[kStackDepth];      // depth is bounded at scene creation (lgb_api.cu), so pushes are unchecked
     float tstack[(ANYHIT || !LGB_TSTACK) ? 1 : kStackDepth];
-    trav_run<ANYHIT, STATS, false, INST>(S, world, ray, f, T, stack, tstack, tmax, lc, 0, 8u);
+    trav_run<ANYHIT, STATS, false, INST, SHIFT>(S, world, ray, f, T, stack, tstack, tmax, lc, 0, 8u, nullptr, 1, t0);
     return T.best;
 }
 
@@ -2760,13 +2768,45 @@ __global__ void __launch_bounds__(256) k_export_li(DevWork W, DevOut O, DevWave 
 }
 
 // Caller-supplied rays (lgb_trace_rays): closest hit id, t, RayIntersection::ng()/ns() (surface.rs:107-118)
+// Parameter at which r enters B, or 0 if r starts inside B or misses it (f64 slab test; a zero direction component keeps its slab
+// only if the origin lies in it).
+__device__ __forceinline__ double entry_param(const TraceBox& B, const Ray64& r) {
+    double tn = 0.0, tf = CUDART_INF;
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        const double o = comp(r.o, k), d = comp(r.d, k);
+        if (d == 0.0) { if (o < B.lo[k] || o > B.hi[k]) return 0.0; continue; }
+        const double t1 = (B.lo[k] - o) / d, t2 = (B.hi[k] - o) / d;
+        tn = fmax(tn, fmin(t1, t2)); tf = fmin(tf, fmax(t1, t2));
+    }
+    return tn <= tf ? tn : 0.0;
+}
 template <bool INST>
-__global__ void __launch_bounds__(128) k_trace(DevScene S, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ngs, double* nss) {
+__global__ void __launch_bounds__(128) k_trace(DevScene S, TraceBox B, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ngs, double* nss) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     Ray64 ray; ray.o = d3(rays[6 * i], rays[6 * i + 1], rays[6 * i + 2]); ray.d = d3(rays[6 * i + 3], rays[6 * i + 4], rays[6 * i + 5]);
+    // The reference takes every ray through the root's Transform3, the identity included (bvh.rs:462): c0 x + c1 y + c2 z + c3 w
+    // ends in + 0, which turns a -0 component into +0 (and so the octant, dinv = +inf, and the slab of an in-plane ray).
+    if (!INST || (S.spaces[0].flags & kSpaceIdentity)) {
+        ray.o = d3(__dadd_rn(ray.o.x, 0.0), __dadd_rn(ray.o.y, 0.0), __dadd_rn(ray.o.z, 0.0));
+        ray.d = d3(__dadd_rn(ray.d.x, 0.0), __dadd_rn(ray.d.y, 0.0), __dadd_rn(ray.d.z, 0.0));
+    }
+    // |d| far from 1: the f32 ray cannot carry it (components overflow to inf, or several reciprocals clamp to the same 1e30), so
+    // the ray is traced as (o, d 2^e) with max |d_k| 2^e in [1, 2).  Every exact test then returns t 2^-e bit for bit (each of
+    // their operations scales exactly by a power of two, and |d| in 2^[-1022/2, 1023/2] keeps the reference's own products
+    // normal), so t comes back exactly; the octant is unchanged.
+    const double dm = fmax(fabs(ray.d.x), fmax(fabs(ray.d.y), fabs(ray.d.z)));
+    const int e = (dm > 0.0 && (dm < 0x1p-40 || dm > 0x1p40)) ? -ilogb(dm) : 0;
+    Ray64 rs = ray;
+    if (e) rs.d = d3(ldexp(ray.d.x, e), ldexp(ray.d.y, e), ldexp(ray.d.z, e));
+    // An origin outside the box of the scene and its camera (lgb_trace_rays admits it up to one box extent away): its f32
+    // rounding could move the ray by more than the node padding and the filter bands allow (they are derived from that box), so
+    // the f32 ray starts where the ray enters the box, grown by a margin.  The exact tests still see the ray as given.
+    const double t0 = entry_param(B, rs);
     LocalCounters lc = {};
-    Hit h = traverse<false, false, INST>(S, ray, CUDART_INF, lc);
+    Hit h = t0 > 0.0 ? traverse<false, false, INST, true>(S, rs, CUDART_INF, lc, t0) : traverse<false, false, INST>(S, rs, CUDART_INF, lc);
+    if (e && h.ref != LGB_MISS) h.t = ldexp(h.t, e);
     uint32_t id = LGB_MISS; D3 ng = d3(0, 0, 0), ns = d3(0, 0, 0);
     if (h.ref != LGB_MISS) {
         Surf sf; double t = h.t;
@@ -3084,10 +3124,10 @@ cudaError_t launch_resolve(const DevWork& W, const DevOut& O, cudaStream_t strea
     k_resolve<<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O);
     return cudaGetLastError();
 }
-cudaError_t launch_trace(const DevScene& S, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns, cudaStream_t stream) {
+cudaError_t launch_trace(const DevScene& S, const TraceBox& B, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns, cudaStream_t stream) {
     if (n == 0) return cudaSuccess;
-    if (S.instanced) k_trace<true><<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(S, rays, n, ids, ts, ng, ns);
-    else k_trace<false><<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(S, rays, n, ids, ts, ng, ns);
+    if (S.instanced) k_trace<true><<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(S, B, rays, n, ids, ts, ng, ns);
+    else k_trace<false><<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(S, B, rays, n, ids, ts, ng, ns);
     return cudaGetLastError();
 }
 cudaError_t launch_l2_read(const void* buf, uint64_t bytes, int iters, float* sink, int sms, cudaStream_t stream) {

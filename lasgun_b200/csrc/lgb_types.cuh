@@ -22,6 +22,10 @@ constexpr int kMaxSpaceDepth = 8;                // nested transformed aggregate
 constexpr uint32_t kSpaceIdentity = 1u, kSpaceSwap = 2u;
 constexpr uint32_t kNoParent = 0xFFFFFFFFu;
 
+// World box of the scene and its camera (lgb_scene::origin_lo/hi) grown by a margin: k_trace starts the f32 ray of a caller-supplied
+// ray whose origin lies outside it where the ray enters it.
+struct TraceBox { double lo[3], hi[3]; };
+
 // One coordinate system of the scene (lgb_build.hpp): cgmath column-major Transform3 of the aggregate that opens it.
 struct DevSpace {
     double m[16], minv[16];

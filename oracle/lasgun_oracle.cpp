@@ -1478,7 +1478,9 @@ double orc_retest_prim(void* accel, uint32_t prim_id, const double* o, const dou
     return INF;
 }
 // Closest hit of caller-supplied rays (Accel::intersect, bvh.rs:461-522): ids = canonical primitive id or 0xFFFFFFFF, t = isect.t.
-void orc_trace_rays(void* accel, const double* rays, uint64_t n, uint32_t* ids, double* ts) {
+// ng / ns (3 doubles per ray, NULL = not wanted): RayIntersection::ng() / ns() (surface.rs:107-118) of the world-space record the
+// root returns, i.e. after transform_isect and the swap_backface flips of every level; zeros on a miss.
+void orc_trace_rays(void* accel, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns) {
     Accel* acc = (Accel*)accel;
     for (uint64_t i = 0; i < n; i++) {
         Ray r = ray_new(v3(rays[6 * i], rays[6 * i + 1], rays[6 * i + 2]), v3(rays[6 * i + 3], rays[6 * i + 4], rays[6 * i + 5]));
@@ -1486,6 +1488,9 @@ void orc_trace_rays(void* accel, const double* rays, uint64_t n, uint32_t* ids, 
         const Primitive* shape = acc->root->intersect(r, is);
         ids[i] = shape ? is.prim_id : 0xFFFFFFFFu;
         ts[i] = shape ? is.t : INF;
+        const V3 g = shape ? isect_ng(is) : v3(0, 0, 0), s = shape ? isect_ns(is) : v3(0, 0, 0);
+        if (ng) { ng[3 * i] = g.x; ng[3 * i + 1] = g.y; ng[3 * i + 2] = g.z; }
+        if (ns) { ns[3 * i] = s.x; ns[3 * i + 1] = s.y; ns[3 * i + 2] = s.z; }
     }
 }
 // li() of one ray with a trace of every ray cast below it (10 doubles each, see trace_ray); returns the number of rays, out_li = radiance.

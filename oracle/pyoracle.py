@@ -73,7 +73,7 @@ def lib():
         "orc_retest_prim": (C.c_double, [vp, C.c_uint32, dp, dp]),
         "orc_camera_sample": (None, [vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, dp]),
         "orc_hardware_threads": (C.c_int, []),
-        "orc_trace_rays": (None, [vp, dp, C.c_uint64, u32p, dp]),
+        "orc_trace_rays": (None, [vp, dp, C.c_uint64, u32p, dp, dp, dp]),
         "orc_debug_li": (C.c_uint64, [vp, dp, dp, dp, C.c_uint64]),
     }
     for name, (res, args) in sig.items():
@@ -209,12 +209,16 @@ class OracleScene:
         n = lib().orc_debug_li(self.accel, _ptr(r, C.c_double), _ptr(out, C.c_double), _ptr(tr, C.c_double), cap)
         return out, tr[:min(n, cap)]
 
-    def trace_rays(self, rays_od):
-        """Closest hit (canonical id, t) of rays given as (n, 6) origin + direction."""
+    def trace_rays(self, rays_od, normals=False):
+        """Closest hit (canonical id, t) of rays given as (n, 6) origin + direction; normals=True also returns the world-space
+        RayIntersection::ng() and ns() of each hit, (n, 3) each (zeros on a miss): (ids, t, ng, ns)."""
         rays = np.ascontiguousarray(rays_od, np.float64).reshape(-1, 6)
         ids = np.zeros((len(rays),), np.uint32); t = np.zeros((len(rays),), np.float64)
-        lib().orc_trace_rays(self.accel, _ptr(rays, C.c_double), len(rays), _ptr(ids, C.c_uint32), _ptr(t, C.c_double))
-        return ids, t
+        ng = np.zeros((len(rays), 3)) if normals else None
+        ns = np.zeros((len(rays), 3)) if normals else None
+        lib().orc_trace_rays(self.accel, _ptr(rays, C.c_double), len(rays), _ptr(ids, C.c_uint32), _ptr(t, C.c_double),
+                             _ptr(ng, C.c_double), _ptr(ns, C.c_double))
+        return (ids, t, ng, ns) if normals else (ids, t)
 
     def camera_sample(self, x, y, w, h):
         out = np.zeros((self.spp, 6), np.float64)
