@@ -22,8 +22,6 @@ namespace lgb {
 constexpr int kRenderEvents = 7;
 cudaError_t launch_render(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, bool stats, bool all_shadows, int sms, cudaStream_t, cudaEvent_t* ev, int part, const SideStreams* side, KernelLog* klog, ShadeChunks* chunks = nullptr);
 bool render_fused(uint32_t spp);
-bool surface_fused(const DevScene&, const DevWork&, const DevOut&, bool all_shadows);
-bool setup_fused(const DevScene&, const DevWork&, const DevOut&, bool all_shadows);
 cudaError_t launch_level(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, int sms, cudaStream_t, DevCounters* shadow_counters);
 cudaError_t launch_gather(const SpawnRec* recs, const uint32_t* nspec, double* rad_parent, const double* rad_child, uint64_t n_upper, cudaStream_t);
 cudaError_t launch_resolve(const DevWork&, const DevOut&, cudaStream_t);
@@ -1641,10 +1639,8 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
                 }
                 W.setup_in_primary = 0;                          // the re-traced slots change their hits: k_setup runs over the band after all
                 DevWork W2 = W;
-                DevCounters before{};
                 if (ties <= V.tie_cap) { W2.slot_list = V.tie_list; W2.n_list = ties; }
                 else if (band == 0) CU(c, cudaMemsetAsync(c->counters.p, 0, kCtrBytes, st));          // too many to list: the whole band again
-                (void)before;
                 if (int rc = sync_scene_copy(c, s, st)) return rc;
                 CU(c, launch_render(s->dev, s->cam, s->shade, W2, O, V, st_on, a.aov, c->sm_count, st, ties <= V.tie_cap ? nullptr : pev, 1, side, a.klog));
             }
@@ -1704,13 +1700,12 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
         for (int k = 0; k < 3; k++) { stats->filter_tests[k] = hc.filter[k]; stats->exact_tests[k] = hc.exact[k]; }
         stats->stack_overflow = hc.stack_overflow;
         stats->beams = W.beams; stats->tie_retraces = tie_slots; stats->secondary_rays = hc.secondary_rays + level_rays;
-        const bool one_kernel = surface_fused(S, W, O, a.aov);              // k_surface: setup + shadows + shade + film
         const uint32_t shadow_launches = grid_shadows ? 1u                                                                // k_gshadow
                                          : s->dev.n_lights * (W.spp > 1 ? 3 : 1) + ((W.beams && W.spp > 1 && !S.instanced) ? 2 * s->dev.n_lights : 0);      // + k_sbeam + k_swalk per light
         const uint32_t primary_launches = W.cg_start ? 1u : (W.beams && W.spp >= 4 && !S.instanced) ? 3u : 1u;           // k_cprimary | k_beam + k_leafp + fallback | k_primary
         const uint32_t shade_launches = S.general ? (S.specular && S.recursion && !wf ? 3u : 2u) : (render_fused(W.spp) && !O.aov_li) ? 1u : 2u;
-        const uint32_t setup_launches = (W.setup_in_primary || setup_fused(S, W, O, a.aov)) ? 0u : 1u;                                          // (inside k_gshadow otherwise)
-        stats->kernel_launches = total_all ? level_launches + (uint32_t)n_bands * (primary_launches + (one_kernel ? 1u : setup_launches + shadow_launches + shade_launches)) : 0;
+        const uint32_t setup_launches = W.setup_in_primary ? 0u : 1u;                                                                           // 0 when k_cprimary<SETUP> did it
+        stats->kernel_launches = total_all ? level_launches + (uint32_t)n_bands * (primary_launches + setup_launches + shadow_launches + shade_launches) : 0;
         if (chunks && chunks->launched) stats->kernel_launches += chunks->launched - 1;
         stats->bands = (uint32_t)n_bands;
         float ms = 0.f; CU(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));

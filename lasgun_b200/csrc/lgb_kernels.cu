@@ -12,42 +12,12 @@
 
 #include "lgb_math.cuh"
 
-// The two traversal prescriptions of the north star that measurements rejected (DESIGN.md 6), kept as build variants:
-#ifndef LGB_SMEM_STACK
-#define LGB_SMEM_STACK 0             // 1: the per-ray traversal stacks of k_primary / k_shadow in shared memory ([entry][thread], conflict-free) instead of local memory
-#endif
-#ifndef LGB_SMEM_TOP
-#define LGB_SMEM_TOP 0               // N > 0: the first N nodes of the device BVH (its top levels: nodes are numbered level by level) staged in shared memory per block
-#endif
-#define LGB_STK(i) ((i) * stride)      // entry i of a traversal stack: stride 1 in local memory, the block size in shared memory
-#ifndef LGB_WALK_PREFETCH
-#define LGB_WALK_PREFETCH 0          // grid walks (k_cprimary, k_gshadow): load entry i + 1 while entry i is tested
-#endif
-#ifndef LGB_CP_STAGE
-#define LGB_CP_STAGE 0               // k_cprimary: a warp whose lanes share a tile stages the list's first 32 entries + filter records in shared memory (needs LGB_WALK_SPLIT).
-                                     // Worth 0.08 ms at 64 registers / 1024 threads per SM; at 48 registers / 1280 threads it COSTS 1.0 ms (6.53 vs 5.54 ms on mixed4k): the
-                                     // 70 KB of slabs per SM come out of the L1 that holds the spill frames (profiles/r2_v47_stage.txt)
-#endif
-#ifndef LGB_WAVE_STREAM
-#define LGB_WAVE_STREAM 1            // wavefront entries (6 GB per mixed4k frame, each written once and read once) are stored / loaded with the streaming
-#endif                               // hint (st.global.cs / ld.global.cs: evict-first in L2), so they do not push the scene and the grids (~100-160 MB) out of the 126 MB L2
-#ifndef LGB_WALK_SPLIT
-#define LGB_WALK_SPLIT 1             // camera-grid walk: filters run down the list until one passes, then the warp meets for the exact test (prim_filter / prim_exact)
-#endif
-#ifndef LGB_WALK_SPLIT_SHADOW
-#define LGB_WALK_SPLIT_SHADOW 0      // the same for the light-grid walk.  Split / fused at 40-48 registers: k_cprimary 5.55 / 5.78 ms, k_gshadow 6.02 / 5.75 (at 64 registers
-                                     // the split won both: 19.47 vs 19.76 ms per frame); an any-hit walk ends at its first exact hit, there is less to converge for
-#endif
-
 namespace lgb {
 
-#if LGB_WAVE_STREAM
+// Wavefront entries (6 GB per mixed4k frame, each written once and read once) are stored / loaded with the streaming hint
+// (st.global.cs / ld.global.cs: evict-first in L2), so they do not push the scene and the grids (~100-160 MB) out of the 126 MB L2.
 template <class T> __device__ __forceinline__ void wst(T* p, T v) { __stcs(p, v); }
 template <class T> __device__ __forceinline__ T wld(const T* p) { return __ldcs(p); }
-#else
-template <class T> __device__ __forceinline__ void wst(T* p, T v) { *p = v; }
-template <class T> __device__ __forceinline__ T wld(const T* p) { return *p; }
-#endif
 
 // ------------------------------------------------------------------ per-ray f32 state
 struct RayF {
@@ -246,29 +216,22 @@ struct Trav {                 // resumable traversal state of one ray
 
 // Inner loop of the while-while traversal: descend interior nodes until `cur` is a leaf or kDone.
 // OCT < 8: every ray of the warp has that direction octant (slab_oct); OCT == 8: mixed warp (slab2).
-#ifndef LGB_TSTACK
-#define LGB_TSTACK 1
-#endif
 // TSTACK (closest-hit rays): the entry distance of a deferred child is kept beside it, and a popped entry
 // that now starts beyond the best hit is dropped without fetching its node.
 template <bool TSTACK>
-__device__ __forceinline__ uint32_t stack_pop(int& sp, const uint32_t* stack, const float* tstack, float best_up, const int stride = 1) {
+__device__ __forceinline__ uint32_t stack_pop(int& sp, const uint32_t* stack, const float* tstack, float best_up) {
     while (sp) {
         --sp;
-        if (!TSTACK || tstack[LGB_STK(sp)] <= best_up) return stack[LGB_STK(sp)];
+        if (!TSTACK || tstack[sp] <= best_up) return stack[sp];
     }
     return kDone;
 }
 template <int OCT, bool STATS, bool TSTACK>
-__device__ __forceinline__ void node_loop(const DevScene& S, const RayF& f, float best_up, uint32_t& cur, int& sp, uint32_t* stack, float* tstack, LocalCounters& lc, const float4* top = nullptr, const int stride = 1) {
+__device__ __forceinline__ void node_loop(const DevScene& S, const RayF& f, float best_up, uint32_t& cur, int& sp, uint32_t* stack, float* tstack, LocalCounters& lc) {
     while (!(cur & kLeafBit) && cur != kDone) {
         const float4* np = S.nodes + 4 * (size_t)cur;
-        float4 n0, n1, n2; float2 n3;
-#if LGB_SMEM_TOP
-        if (top && cur < (uint32_t)LGB_SMEM_TOP) { const float4* tp = top + 4 * cur; n0 = tp[0]; n1 = tp[1]; n2 = tp[2]; n3 = make_float2(tp[3].x, tp[3].y); }
-        else
-#endif
-        { n0 = __ldg(np); n1 = __ldg(np + 1); n2 = __ldg(np + 2); n3 = __ldg(reinterpret_cast<const float2*>(np + 3)); }
+        const float4 n0 = __ldg(np), n1 = __ldg(np + 1), n2 = __ldg(np + 2);
+        const float2 n3 = __ldg(reinterpret_cast<const float2*>(np + 3));
         if (STATS) lc.node_tests++;
         float tn0, tn1;
         bool h0, h1;
@@ -283,11 +246,11 @@ __device__ __forceinline__ void node_loop(const DevScene& S, const RayF& f, floa
         if (h0 && h1) {
             const bool swap = tn1 < tn0;
             cur = swap ? c1 : c0;
-            if (TSTACK) tstack[LGB_STK(sp)] = swap ? tn0 : tn1;
-            stack[LGB_STK(sp)] = swap ? c0 : c1; sp++;
+            if (TSTACK) tstack[sp] = swap ? tn0 : tn1;
+            stack[sp] = swap ? c0 : c1; sp++;
         } else if (h0) cur = c0;
         else if (h1) cur = c1;
-        else cur = stack_pop<TSTACK>(sp, stack, tstack, best_up, stride);
+        else cur = stack_pop<TSTACK>(sp, stack, tstack, best_up);
     }
 }
 
@@ -363,7 +326,7 @@ __device__ __forceinline__ bool leaf_prims(const DevScene& S, const Ray64& world
     return false;
 }
 
-// The two halves of leaf_prims for ONE primitive, for the grid walks (k_cprimary, k_gshadow; LGB_WALK_SPLIT): a lane first runs
+// The two halves of leaf_prims for ONE primitive, for the camera-grid walk (k_cprimary): a lane first runs
 // filters down its list until one passes, then the warp meets for the exact f64 test.  In the fused form a warp ran the exact test
 // -- by far the longest stretch of the loop body -- in nearly every iteration for whichever lanes happened to pass in that one.
 // the filter of one primitive given its f32 record (sphere: q0 = {c, r}; cuboid: q0, q1 = padded lo, hi; triangle: q0..q2 = vertices)
@@ -437,8 +400,9 @@ __device__ __forceinline__ bool prim_exact(const DevScene& S, const Ray64& world
 }
 
 // Runs until the ray is finished (returns true; T.cur == kDone) or, with REFILL, until fewer than
-// `refill_below` lanes of the warp are still traversing (returns false: the caller tops the warp up with
-// new rays and calls again; persistent threads with dynamic fetch).
+// `refill_below` lanes of the warp are still traversing (returns false).  Every caller passes 0: a warp takes new
+// rays only once all its lanes are done (topping it up earlier was measured slower, DESIGN.md §6).  The REFILL
+// form stays because the persistent kernels schedule differently without it.
 // INST (scenes with transformed aggregates): `ray` / `f` are the ray in the CURRENT space and change when the
 // traversal enters or leaves a nested level; `world` is the ray as cast.  A leaf of type LGB_PRIM_INSTANCE lists child
 // spaces; entering one defers the rest of the leaf and an exit marker (count field 31, payload = space to return to).
@@ -446,21 +410,21 @@ constexpr uint32_t kInstLeaf = kLeafBit | ((uint32_t)LGB_PRIM_INSTANCE << 29);
 constexpr uint32_t kExitMarker = kInstLeaf | (31u << 24);
 template <bool ANYHIT, bool STATS, bool REFILL, bool INST, bool SHIFT = false>
 __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, Ray64& ray, RayF& f, Trav& T, uint32_t* stack, float* tstack, double tmax,
-                                         LocalCounters& lc, int refill_below, unsigned octw, const float4* top = nullptr, const int stride = 1, double t0 = 0.0) {
+                                         LocalCounters& lc, int refill_below, unsigned octw, double t0 = 0.0) {
     Hit& best = T.best;
     float& best_tf = T.best_tf; float& best_up = T.best_up;
     uint32_t& cur = T.cur; int& sp = T.sp;
     for (;;) {
         switch (INST ? f.oct : octw) {   // octw is warp-uniform: the octant shared by every ray of the warp, or 8 (mixed)
-        case 0: node_loop<0, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 1: node_loop<1, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 2: node_loop<2, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 3: node_loop<3, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 4: node_loop<4, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 5: node_loop<5, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 6: node_loop<6, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        case 7: node_loop<7, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
-        default: node_loop<8, STATS, (!ANYHIT && LGB_TSTACK)>(S, f, best_up, cur, sp, stack, tstack, lc, top, stride); break;
+        case 0: node_loop<0, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 1: node_loop<1, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 2: node_loop<2, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 3: node_loop<3, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 4: node_loop<4, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 5: node_loop<5, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 6: node_loop<6, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        case 7: node_loop<7, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
+        default: node_loop<8, STATS, !ANYHIT>(S, f, best_up, cur, sp, stack, tstack, lc); break;
         }
         if (cur == kDone) return true;
         {
@@ -471,9 +435,9 @@ __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, 
                     ray = ray_to_space(S, first, world);
                     f = SHIFT ? make_rayf(ray, S.spaces[first].err_abs, t0) : make_rayf(ray, S.spaces[first].err_abs);
                 } else {
-                    if (count > 1u) { if (!ANYHIT && LGB_TSTACK) tstack[LGB_STK(sp)] = -CUDART_INF_F; stack[LGB_STK(sp)] = kInstLeaf | ((count - 2u) << 24) | (first + 1u); sp++; }
-                    if (!ANYHIT && LGB_TSTACK) tstack[LGB_STK(sp)] = -CUDART_INF_F;
-                    stack[LGB_STK(sp)] = kExitMarker | T.space; sp++;
+                    if (count > 1u) { if (!ANYHIT) tstack[sp] = -CUDART_INF_F; stack[sp] = kInstLeaf | ((count - 2u) << 24) | (first + 1u); sp++; }
+                    if (!ANYHIT) tstack[sp] = -CUDART_INF_F;
+                    stack[sp] = kExitMarker | T.space; sp++;
                     const uint32_t child = __ldg(&S.inst_space[first]);
                     const DevSpace& c = S.spaces[child];
                     if (!(c.flags & kSpaceIdentity)) ray = ray_into(c, ray);
@@ -484,7 +448,7 @@ __device__ __forceinline__ bool trav_run(const DevScene& S, const Ray64& world, 
                 }
             } else if (leaf_prims<ANYHIT, STATS, INST>(S, world, ray, f, T, type, count, first, tmax, lc)) { cur = kDone; return true; }
         }
-        cur = stack_pop<(!ANYHIT && LGB_TSTACK)>(sp, stack, tstack, best_up, stride);
+        cur = stack_pop<!ANYHIT>(sp, stack, tstack, best_up);
         if (REFILL && __popc(__activemask()) < refill_below) return cur == kDone;
     }
 }
@@ -508,8 +472,8 @@ __device__ Hit traverse(const DevScene& S, const Ray64& world, double tmax, Loca
     Ray64 ray; RayF f; Trav T;
     enter_root<INST, SHIFT>(S, world, ray, f, T, tmax, t0);
     uint32_t stack[kStackDepth];      // depth is bounded at scene creation (lgb_api.cu), so pushes are unchecked
-    float tstack[(ANYHIT || !LGB_TSTACK) ? 1 : kStackDepth];
-    trav_run<ANYHIT, STATS, false, INST, SHIFT>(S, world, ray, f, T, stack, tstack, tmax, lc, 0, 8u, nullptr, 1, t0);
+    float tstack[ANYHIT ? 1 : kStackDepth];
+    trav_run<ANYHIT, STATS, false, INST, SHIFT>(S, world, ray, f, T, stack, tstack, tmax, lc, 0, 8u, t0);
     return T.best;
 }
 
@@ -1014,9 +978,6 @@ __device__ __forceinline__ bool slot_ray(const DevCamera& C, const DevWork& W, u
     return true;
 }
 
-#ifndef LGB_REFILL_BELOW
-#define LGB_REFILL_BELOW 0       // >0: top a warp up with new rays once fewer lanes than this are still traversing (measured: slower, DESIGN.md §6)
-#endif
 
 // Warp-level work fetch for the persistent kernels: every lane whose `need` is set receives the index of a
 // fresh work item (or >= total when the queue is drained) with one atomic per warp.
@@ -1123,24 +1084,8 @@ __global__ void __launch_bounds__(LGB_TRAV_THREADS, LGB_MIN_BLOCKS) k_primary(De
     const unsigned lane = threadIdx.x & 31u;
     LocalCounters lc = {};
     unsigned int hits = 0, primary = 0;
-#if LGB_SMEM_STACK
-    extern __shared__ uint32_t dyn_smem[];                                   // [entry][thread]: stack words, then entry distances
-    uint32_t* stack = dyn_smem + threadIdx.x;
-    float* tstack = reinterpret_cast<float*>(dyn_smem + (size_t)kStackDepth * LGB_TRAV_THREADS) + threadIdx.x;
-    constexpr int kStride = LGB_TRAV_THREADS;
-#else
     uint32_t stack[kStackDepth];
-    float tstack[LGB_TSTACK ? kStackDepth : 1];
-    constexpr int kStride = 1;
-#endif
-#if LGB_SMEM_TOP
-    __shared__ float4 s_top[4 * LGB_SMEM_TOP];
-    for (uint32_t i = threadIdx.x; i < 4u * min((uint32_t)LGB_SMEM_TOP, S.n_nodes); i += blockDim.x) s_top[i] = __ldg(S.nodes + i);
-    __syncthreads();
-    const float4* top = s_top;
-#else
-    const float4* top = nullptr;
-#endif
+    float tstack[kStackDepth];
     Ray64 world, ray; RayF f; Trav T;      // INST: `ray` is the ray in the current space; otherwise it stays equal to `world`
     uint64_t g = 0;
     bool active = false, drained = false;
@@ -1148,7 +1093,7 @@ __global__ void __launch_bounds__(LGB_TRAV_THREADS, LGB_MIN_BLOCKS) k_primary(De
         // refill: lanes without a ray take the next sample slots
         if (!drained) {
             const unsigned idle = __ballot_sync(0xFFFFFFFFu, !active);
-            if (idle == 0xFFFFFFFFu || __popc(idle) > 32 - LGB_REFILL_BELOW) {
+            if (idle == 0xFFFFFFFFu) {
                 bool need = !active;
                 while (__any_sync(0xFFFFFFFFu, need) && !drained) {
                     const unsigned long long idx = warp_fetch(V.work_counter, need, lane);
@@ -1173,7 +1118,7 @@ __global__ void __launch_bounds__(LGB_TRAV_THREADS, LGB_MIN_BLOCKS) k_primary(De
         const unsigned oct0 = __shfl_sync(0xFFFFFFFFu, f.oct, __ffs(amask) - 1);
         const unsigned octw = __all_sync(0xFFFFFFFFu, !active || f.oct == oct0) ? oct0 : 8u;
         if (active) {
-            const bool done = trav_run<false, STATS, true, INST>(S, world, ray, f, T, stack, tstack, CUDART_INF, lc, drained ? 0 : LGB_REFILL_BELOW, octw, top, kStride);
+            const bool done = trav_run<false, STATS, true, INST>(S, world, ray, f, T, stack, tstack, CUDART_INF, lc, 0, octw);
             if (done) {
                 const bool hit = T.best.ref != LGB_MISS;
                 V.hit_t[g] = hit ? T.best.t : CUDART_INF; V.hit_ref[g] = T.best.ref;
@@ -1262,9 +1207,6 @@ __device__ __forceinline__ bool beam_slab(float lx, float ly, float lz, float hx
 #define LGB_BEAM_MARGIN 1.03125f
 #endif
 constexpr float kBeamMargin = LGB_BEAM_MARGIN;
-#ifndef LGB_BEAM_PRIMS
-#define LGB_BEAM_PRIMS 1             // the bundle lists primitives, not leaves: 52.56 -> 48.44 ms/frame (k_leafp 10.8 -> 6.5, k_beam 4.4 -> 5.2 ms)
-#endif
 #ifndef LGB_BEAM_THREADS
 #define LGB_BEAM_THREADS 64          // as for k_leafp: 256 -> 64 threads per block, 54.02 -> 53.59 ms/frame
 #endif
@@ -1288,11 +1230,9 @@ __global__ void __launch_bounds__(LGB_BEAM_THREADS, 1024 / LGB_BEAM_THREADS) k_b
             uint32_t stack[kStackDepth]; float tstack[kStackDepth]; int sp = 0;
             uint2 list[kBeamList];                     // (leaf word, entry distance) in visiting order: nearer child first, so nearly sorted
             uint32_t cur = 0;
-            float cur_t = 0.0f;                        // bundle entry distance of `cur`
             bool over = false;
             while (cur != kDone && !over) {
                 if (cur & kLeafBit) {                  // a leaf the bundle enters before the bound: list it, test the centre ray
-#if LGB_BEAM_PRIMS
                     // ... primitive by primitive: the bundle against the primitive's own (padded) box, so that the sample rays of
                     // the pixel are handed only the primitives their bundle can reach -- a quarter of a leaf on average
                     const uint32_t type = (cur >> 29) & 3u, count = ((cur >> 24) & 31u) + 1u, first = cur & kLeafFirstMask;
@@ -1326,14 +1266,6 @@ __global__ void __launch_bounds__(LGB_BEAM_THREADS, 1024 / LGB_BEAM_THREADS) k_b
                     }
                     if (over) break;
                     cur = kDone;
-#else
-                    const float t = cur_t;
-                    if (n == (uint32_t)kBeamList) { over = true; break; }
-                    list[n++] = make_uint2(cur, __float_as_uint(t));
-                    leaf_prims<false, STATS, false>(S, world, ray, f, T, (cur >> 29) & 3u, ((cur >> 24) & 31u) + 1u, cur & kLeafFirstMask, CUDART_INF, lc);
-                    bound = T.best_up * kBeamMargin;
-                    cur = kDone;
-#endif
                 } else {
                     const float4* np = S.nodes + 4 * (size_t)cur;
                     const float4 n0 = __ldg(np), n1 = __ldg(np + 1), n2 = __ldg(np + 2);
@@ -1351,15 +1283,15 @@ __global__ void __launch_bounds__(LGB_BEAM_THREADS, 1024 / LGB_BEAM_THREADS) k_b
                     const uint32_t c0 = __float_as_uint(n3.x), c1 = __float_as_uint(n3.y);
                     if (h0 && h1) {
                         const bool swap = t1 < t0;
-                        cur = swap ? c1 : c0; cur_t = swap ? t1 : t0;
+                        cur = swap ? c1 : c0;
                         tstack[sp] = swap ? t0 : t1; stack[sp++] = swap ? c0 : c1;
-                    } else if (h0) { cur = c0; cur_t = t0; }
-                    else if (h1) { cur = c1; cur_t = t1; }
+                    } else if (h0) cur = c0;
+                    else if (h1) cur = c1;
                     else cur = kDone;
                 }
                 while (cur == kDone && sp) {           // nearest deferred entry that still starts before the bound
                     --sp;
-                    if (tstack[sp] <= bound) { cur = stack[sp]; cur_t = tstack[sp]; }
+                    if (tstack[sp] <= bound) cur = stack[sp];
                 }
             }
             if (over) {
@@ -1395,9 +1327,6 @@ __global__ void __launch_bounds__(LGB_BEAM_THREADS, 1024 / LGB_BEAM_THREADS) k_b
 }
 
 // One thread per sample slot (the centre sample is already done): the leaves of its pixel's beam, nearest first.
-#ifndef LGB_LEAFP_PREFETCH
-#define LGB_LEAFP_PREFETCH 0
-#endif
 #ifndef LGB_LEAFP_THREADS
 #define LGB_LEAFP_THREADS 64         // a block waits for its slowest ray before it frees its slots: 256 -> 64 threads, 55.15 -> 53.97 ms/frame
 #endif
@@ -1421,15 +1350,8 @@ __global__ void __launch_bounds__(LGB_LEAFP_THREADS, 1024 / LGB_LEAFP_THREADS) k
             const float bound = V.beam_bound[p];
             Ray64 ray; RayF f; Trav T;
             enter_root<false>(S, world, ray, f, T, CUDART_INF);
-#if LGB_LEAFP_PREFETCH
-            uint2 e_next = n ? __ldg(&V.beam_list[p]) : make_uint2(0u, 0u);
-            for (uint32_t i = 0; i < n; i++) {
-                const uint2 e = e_next;
-                if (i + 1 < n) e_next = __ldg(&V.beam_list[(size_t)(i + 1) * W.n_pixels + p]);       // in flight while this leaf is tested
-#else
             for (uint32_t i = 0; i < n; i++) {
                 const uint2 e = __ldg(&V.beam_list[(size_t)i * W.n_pixels + p]);
-#endif
                 if (__uint_as_float(e.y) > T.best_up) continue;            // starts beyond the best hit (the list is only nearly sorted)
                 leaf_prims<false, STATS, false>(S, world, ray, f, T, (e.x >> 29) & 3u, ((e.x >> 24) & 31u) + 1u, e.x & kLeafFirstMask, CUDART_INF, lc);
             }
@@ -1477,14 +1399,9 @@ __device__ __forceinline__ uint32_t light_gates(const DevScene& S, const Ray64& 
     return gate;
 }
 
-// The rare slot whose sign decisions lean_surface leaves to the reference's own sequence (k_gshadow<SETUP>), out of line.
-__device__ __noinline__ void setup_generic(const DevScene& S, const Ray64& ray, double t, uint32_t ref, D3& ps, D3& ng, double& wo_ng) {
-    ShadePoint P; uint32_t id;
-    shade_point<false, false>(S, ray, t, ref, P, id);
-    ps = P.ps; ng = P.ng; wo_ng = dot(P.wo, P.ng);
-}
-// The same for k_cprimary<SETUP>, written so that nothing of the kernel's own state has its address taken: the scene record is read
-// from global memory (DevScene::self), the ray goes by value, the results go straight to the slot's wavefront entries.  With
+// The rare slot whose sign decisions lean_surface leaves to the reference's own sequence (k_cprimary<SETUP>), out of line.
+// Written so that nothing of the kernel's own state has its address taken: the scene record is read from global memory
+// (DevScene::self), the ray goes by value, the results go straight to the slot's wavefront entries.  With
 // `const DevScene& S` bound to the kernel's parameter block every thread copied the 350-byte record to its stack at entry (28 STL.64
 // per thread: 30 GB of local stores per mixed4k frame, through L1 into L2), and the ray after it -- for a call one slot in a million makes.
 __device__ __noinline__ void setup_generic_slot(const DevScene* Sg, double ox, double oy, double oz, double dx, double dy, double dz, double t, uint32_t ref,
@@ -1527,36 +1444,6 @@ __global__ void __launch_bounds__(LGB_CPRIMARY_THREADS, LGB_CPRIMARY_BLOCKS) k_c
     const size_t cell = (size_t)(y >> W.cg_shift) * W.cg_nx + (size_t)(x >> W.cg_shift);
     uint32_t b = 0, e = 0;
     if (valid) { b = __ldg(W.cg_start + cell); e = __ldg(W.cg_start + cell + 1); }
-#if LGB_CP_STAGE
-    // A warp holds the samples of 32 / spp neighbouring pixels, so at >= 8 spp all its lanes walk the SAME tile's list.  Then the lanes
-    // fetch its first 32 entries and their f32 filter records side by side, one entry each, into the warp's slab of shared memory, and
-    // the walk reads them from there: the dependent chain list -> entry -> record (two L1 / L2 round trips per entry and lane) becomes
-    // one parallel fetch per warp.  Warps whose lanes disagree (1 spp: 32 pixels, two tiles) walk from global memory as before.
-    constexpr uint32_t kStage = 32;
-    __shared__ uint2 s_ent[LGB_CPRIMARY_THREADS / 32][kStage];
-    __shared__ float4 s_rec[LGB_CPRIMARY_THREADS / 32][kStage][3];
-    const unsigned wid = threadIdx.x >> 5;
-    uint32_t ns = 0;
-    {
-        const unsigned vmask = __ballot_sync(0xFFFFFFFFu, valid);
-        if (vmask) {
-            const int lead = __ffs(vmask) - 1;
-            const unsigned long long cell0 = __shfl_sync(0xFFFFFFFFu, (unsigned long long)cell, lead);
-            const uint32_t b0 = __shfl_sync(0xFFFFFFFFu, b, lead), e0 = __shfl_sync(0xFFFFFFFFu, e, lead);
-            if (__all_sync(0xFFFFFFFFu, !valid || (unsigned long long)cell == cell0)) {
-                ns = min(e0 - b0, kStage);
-                if (lane < ns) {
-                    const uint2 r = __ldg(W.cg_entries + b0 + lane);
-                    float4 q0, q1 = make_float4(0.f, 0.f, 0.f, 0.f), q2 = q1;
-                    prim_record(S, r.x >> 30, r.x & 0x3FFFFFFFu, q0, q1, q2);
-                    s_ent[wid][lane] = r;
-                    s_rec[wid][lane][0] = q0; s_rec[wid][lane][1] = q1; s_rec[wid][lane][2] = q2;
-                }
-                __syncwarp();
-            }
-        }
-    }
-#endif
     if (valid) {
         {
             const Ray64 world = camera_ray(C, W, x, y, s);
@@ -1565,53 +1452,20 @@ __global__ void __launch_bounds__(LGB_CPRIMARY_THREADS, LGB_CPRIMARY_BLOCKS) k_c
             primary++;
             const float to_t = f.inv_len * (1.0f - 2e-6f);                   // an entry's distance from the eye -> a lower bound of its ray parameter
             const bool sorted = e - b <= kGridSortMax;                       // (longer lists are not sorted: lgb_grid.cu)
-#if LGB_WALK_SPLIT
             // positions [b, e) are the tile's list, [e, e2) the large list (both nearest first)
             const uint32_t e2 = e + W.cg_n_large;
             for (uint32_t i = b;;) {
                 uint32_t cand = 0xFFFFFFFFu;
                 while (i < e2) {
                     const bool in_cell = i < e;
-#if LGB_CP_STAGE
-                    const uint32_t k = i - b;
-                    const bool staged = k < ns;
-                    const uint2 r = staged ? s_ent[wid][k] : __ldg(in_cell ? W.cg_entries + i : W.cg_large + (i - e));
-                    i++;
-                    if (__uint_as_float(r.y) * to_t > T.best_up) { if (!in_cell) i = e2; else if (sorted) i = e; continue; }    // nearest first: nothing behind the best hit can beat it
-                    const uint32_t type = r.x >> 30;
-                    float4 q0, q1 = make_float4(0.f, 0.f, 0.f, 0.f), q2 = q1;
-                    if (staged) { q0 = s_rec[wid][k][0]; if (type != LGB_PRIM_SPHERE) { q1 = s_rec[wid][k][1]; q2 = s_rec[wid][k][2]; } }
-                    else prim_record(S, type, r.x & 0x3FFFFFFFu, q0, q1, q2);
-                    if (prim_filter_rec<STATS>(f, T.best_tf, type, q0, q1, q2, lc)) { cand = r.x; break; }
-#else
                     const uint2 r = __ldg(in_cell ? W.cg_entries + i : W.cg_large + (i - e));
                     i++;
                     if (__uint_as_float(r.y) * to_t > T.best_up) { if (!in_cell) i = e2; else if (sorted) i = e; continue; }    // nearest first: nothing behind the best hit can beat it
                     if (prim_filter<STATS>(S, f, T.best_tf, r.x >> 30, r.x & 0x3FFFFFFFu, lc)) { cand = r.x; break; }
-#endif
                 }
                 if (cand == 0xFFFFFFFFu) break;
                 prim_exact<false, STATS>(S, world, ray, f, T, cand >> 30, cand & 0x3FFFFFFFu, CUDART_INF, lc);
             }
-#else
-#if LGB_WALK_PREFETCH
-            uint2 nxt = b < e ? __ldg(W.cg_entries + b) : make_uint2(0u, 0u);
-            for (uint32_t i = b; i < e; i++) {
-                const uint2 r = nxt;
-                if (i + 1 < e) nxt = __ldg(W.cg_entries + i + 1);            // in flight while this entry is tested
-#else
-            for (uint32_t i = b; i < e; i++) {
-                const uint2 r = __ldg(W.cg_entries + i);
-#endif
-                if (__uint_as_float(r.y) * to_t > T.best_up) { if (sorted) break; else continue; }    // nearest first: nothing behind the best hit can beat it
-                leaf_prims<false, STATS, false>(S, world, ray, f, T, r.x >> 30, 1u, r.x & 0x3FFFFFFFu, CUDART_INF, lc);
-            }
-            for (uint32_t i = 0; i < W.cg_n_large; i++) {
-                const uint2 r = __ldg(W.cg_large + i);
-                if (__uint_as_float(r.y) * to_t > T.best_up) break;
-                leaf_prims<false, STATS, false>(S, world, ray, f, T, r.x >> 30, 1u, r.x & 0x3FFFFFFFu, CUDART_INF, lc);
-            }
-#endif
             const bool hit = T.best.ref != LGB_MISS;
             wst(&V.hit_t[g], (double)(hit ? T.best.t : CUDART_INF)); wst(&V.hit_ref[g], (uint32_t)(T.best.ref));
             hits += hit ? 1u : 0u;
@@ -1801,9 +1655,6 @@ __global__ void __launch_bounds__(kAppendThreads) k_pretest(DevScene S, DevWork 
 // them against the listed primitives only (f32 filter + exact f64 test) and removes them from queue B.  Whatever is left (pixels
 // whose anchor is blocked -- k_pretest tries its occluder on the other samples first, as before --, overflowing lists, pixels
 // without an anchor ray) goes the old way: k_pretest, then k_shadow over queue C.
-#ifndef LGB_SHADOW_BEAMS
-#define LGB_SHADOW_BEAMS 1           // 48.45 -> 45.50 ms/frame on mixed4k (bundles only for pixels whose anchor ray is free; with every anchor as a bundle: 54.3)
-#endif
 template <bool STATS>
 __global__ void __launch_bounds__(LGB_SBEAM_THREADS_, 1024 / LGB_SBEAM_THREADS_) k_sbeam(DevScene S, DevWork W, DevOut O, DevWave V, uint32_t light,
                                                                                      uint2* list_out, uint32_t* count_out) {
@@ -1999,31 +1850,10 @@ __device__ __forceinline__ bool grid_blocked(const DevScene& S, D3 o, uint32_t l
     const bool sorted = e - b <= kGridSortMax;                         // (longer lists are not sorted: lgb_grid.cu)
     const uint2* en = G->entries;
     const uint2* lg = G->large;
-#if LGB_WALK_SPLIT_SHADOW
-    // positions [b, e) are the cell's list, [e, e2) the light's large list (both nearest first)
-    const uint32_t e2 = e + n_large;
-    for (uint32_t i = b;;) {
-        uint32_t cand = 0xFFFFFFFFu;
-        while (i < e2) {
-            const bool in_cell = i < e;
-            const uint2 r = __ldg(in_cell ? en + i : lg + (i - e));
-            i++;
-            if (__uint_as_float(r.y) > len_up) { if (!in_cell) i = e2; else if (sorted) i = e; continue; }
-            if (prim_filter<STATS>(S, f, T.best_tf, r.x >> 30, r.x & 0x3FFFFFFFu, lc)) { cand = r.x; break; }
-        }
-        if (cand == 0xFFFFFFFFu) break;
-        if (prim_exact<true, STATS>(S, world, ray, f, T, cand >> 30, cand & 0x3FFFFFFFu, 1.0, lc)) { hit = true; break; }
-    }
-#else
-#if LGB_WALK_PREFETCH
-    uint2 nxt = b < e ? __ldg(en + b) : make_uint2(0u, 0u);
-    for (uint32_t i = b; i < e && !hit; i++) {
-        const uint2 r = nxt;
-        if (i + 1 < e) nxt = __ldg(en + i + 1);                          // in flight while this entry is tested
-#else
+    // The fused walk (filter and exact test in one loop body), not k_cprimary's split form: at 40-48 registers the split walk took
+    // 6.02 ms against 5.75 on mixed4k.  An any-hit walk ends at its first exact hit, so there is less for the warp to converge on.
     for (uint32_t i = b; i < e && !hit; i++) {
         const uint2 r = __ldg(en + i);
-#endif
         if (__uint_as_float(r.y) > len_up) { if (sorted) break; else continue; }
         hit = leaf_prims<true, STATS, false>(S, world, ray, f, T, r.x >> 30, 1u, r.x & 0x3FFFFFFFu, 1.0, lc);
     }
@@ -2032,13 +1862,10 @@ __device__ __forceinline__ bool grid_blocked(const DevScene& S, D3 o, uint32_t l
         if (__uint_as_float(r.y) > len_up) break;
         hit = leaf_prims<true, STATS, false>(S, world, ray, f, T, r.x >> 30, 1u, r.x & 0x3FFFFFFFu, 1.0, lc);
     }
-#endif
     return hit;
 }
 
-// SETUP (camera rays of a plain capture): the thread also does k_setup's work for its slot -- surface record, sign byte, gates -- so
-// that the shadow origin goes from registers into the walk and is never stored (k_setup and its 24 B/slot of ps drop out of the frame).
-template <bool STATS, bool ALL_SHADOWS, bool SETUP = false>
+template <bool STATS, bool ALL_SHADOWS>
 __global__ void __launch_bounds__(LGB_GSHADOW_THREADS, LGB_GSHADOW_MIN_BLOCKS) k_gshadow(DevScene S, DevCamera C, DevWork W, DevOut O, DevWave V) {
     const uint64_t total = W.n_pixels * W.spp;
     const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2049,32 +1876,11 @@ __global__ void __launch_bounds__(LGB_GSHADOW_THREADS, LGB_GSHADOW_MIN_BLOCKS) k
         const uint32_t ref = wld(&V.hit_ref[g]);
         uint32_t mask = 0;
         D3 ps = d3(0, 0, 0);
-        if (SETUP) {
-            const double t = V.hit_t[g];
-            Ray64 ray; uint32_t x, y, s;
-            if (ref != LGB_MISS && ref != kSlotUnused && slot_ray<false>(C, W, g, ray, x, y, s)) {
-                if (S.specular && (material_flags(S, ref) & kMatSpecular)) { V.occl[g] = 0; V.gate[g] = 0; }     // glass, mirror: BSDF::f is zero (bxdf/mod.rs:172)
-                else {
-                    LeanSurf Ls;
-                    lean_surface<true>(S, ray, t, ref, 0u, Ls);
-                    D3 ng; double wo_ng = 1.0;
-                    if (Ls.flags & kSfGeneric) setup_generic(S, ray, t, ref, ps, ng, wo_ng);
-                    else {
-                        ng = (Ls.flags & kSfNgFlip) ? -Ls.n : Ls.n;
-                        ps = ray.o + ray.d * t + ng * (2.220446049250313e-16 * 65536.0);       // surface.rs:168, integrate.rs:40
-                    }
-                    mask = light_gates(S, ray, ps, ng, wo_ng, !(Ls.flags & kSfGeneric));
-                    V.gate[g] = mask; V.sflags[g] = (unsigned char)Ls.flags;
-                    if (!mask) V.occl[g] = 0;
-                }
-            }
-        } else {
-            // gate and shadow origin are requested together with the hit word, not one after the other (three dependent round trips
-            // were 18 % of this kernel's stall samples); for a miss they hold stale values nobody looks at
-            const uint32_t gate = ALL_SHADOWS ? (S.n_lights >= 32u ? 0xFFFFFFFFu : (1u << S.n_lights) - 1u) : wld(&V.gate[g]);
-            ps = d3(wld(&V.ps[3 * g]), wld(&V.ps[3 * g + 1]), wld(&V.ps[3 * g + 2]));
-            if (ref != LGB_MISS && ref != kSlotUnused) mask = gate;
-        }
+        // gate and shadow origin are requested together with the hit word, not one after the other (three dependent round trips
+        // were 18 % of this kernel's stall samples); for a miss they hold stale values nobody looks at
+        const uint32_t gate = ALL_SHADOWS ? (S.n_lights >= 32u ? 0xFFFFFFFFu : (1u << S.n_lights) - 1u) : wld(&V.gate[g]);
+        ps = d3(wld(&V.ps[3 * g]), wld(&V.ps[3 * g + 1]), wld(&V.ps[3 * g + 2]));
+        if (ref != LGB_MISS && ref != kSlotUnused) mask = gate;
         if (mask) {
             uint32_t occl = 0;
             for (uint32_t l = 0; l < S.n_lights; l++) {
@@ -2110,29 +1916,14 @@ __global__ void __launch_bounds__(LGB_TRAV_THREADS, LGB_MIN_BLOCKS) k_shadow(Dev
     const unsigned lane = threadIdx.x & 31u;
     LocalCounters lc = {};
     unsigned int occluded = 0;
-#if LGB_SMEM_STACK
-    extern __shared__ uint32_t dyn_smem[];
-    uint32_t* stack = dyn_smem + threadIdx.x;
-    constexpr int kStride = LGB_TRAV_THREADS;
-#else
     uint32_t stack[kStackDepth];
-    constexpr int kStride = 1;
-#endif
-#if LGB_SMEM_TOP
-    __shared__ float4 s_top[4 * LGB_SMEM_TOP];
-    for (uint32_t i = threadIdx.x; i < 4u * min((uint32_t)LGB_SMEM_TOP, S.n_nodes); i += blockDim.x) s_top[i] = __ldg(S.nodes + i);
-    __syncthreads();
-    const float4* top = s_top;
-#else
-    const float4* top = nullptr;
-#endif
     Ray64 world, ray; RayF f; Trav T;
     uint32_t g = 0;
     bool active = false, drained = false;
     for (;;) {
         if (!drained) {
             const unsigned idle = __ballot_sync(0xFFFFFFFFu, !active);
-            if (idle == 0xFFFFFFFFu || __popc(idle) > 32 - LGB_REFILL_BELOW) {
+            if (idle == 0xFFFFFFFFu) {
                 const unsigned long long idx = warp_fetch(V.queue_fetch + light * 3 + which, !active, lane);
                 if (!active && idx < total) {
                     g = q[idx];
@@ -2148,7 +1939,7 @@ __global__ void __launch_bounds__(LGB_TRAV_THREADS, LGB_MIN_BLOCKS) k_shadow(Dev
         const unsigned oct0 = __shfl_sync(0xFFFFFFFFu, f.oct, __ffs(amask) - 1);
         const unsigned octw = __all_sync(0xFFFFFFFFu, !active || f.oct == oct0) ? oct0 : 8u;
         if (active) {
-            const bool done = trav_run<true, STATS, true, INST>(S, world, ray, f, T, stack, nullptr, 1.0, lc, drained ? 0 : LGB_REFILL_BELOW, octw, top, kStride);
+            const bool done = trav_run<true, STATS, true, INST>(S, world, ray, f, T, stack, nullptr, 1.0, lc, 0, octw);
             if (done) {
                 if (T.best.ref != LGB_MISS) { atomicOr(&V.occl[g], 1u << light); occluded++; }
                 if (record) V.occluder[(size_t)light * W.n_pixels + fdiv(g, W.fd_spp)] = T.best.ref;
@@ -2183,9 +1974,6 @@ __global__ void __launch_bounds__(LGB_TRAV_THREADS, LGB_MIN_BLOCKS) k_shadow(Dev
 #endif
 #ifndef LGB_FUSED_THREADS
 #define LGB_FUSED_THREADS 128u          // blocks of 256 / 128 threads (whole pixels): k_shade_lean 4.05 / 3.88 ms on mixed4k
-#endif
-#ifndef LGB_WARP_RESOLVE
-#define LGB_WARP_RESOLVE 0           // 1: fused resolve through warp shuffles instead of shared memory + barrier (measured 0.4 ms slower, DESIGN.md §6)
 #endif
 #ifndef LGB_GSHADE_MIN_BLOCKS
 #define LGB_GSHADE_MIN_BLOCKS 2      // the GENERAL variants (every material, spawn of the specular rays)
@@ -2307,20 +2095,6 @@ __global__ void __launch_bounds__(256, GENERAL ? LGB_GSHADE_MIN_BLOCKS : LGB_SHA
         if (have) { O.radiance[3 * g + 0] = output.x; O.radiance[3 * g + 1] = output.y; O.radiance[3 * g + 2] = output.z; }
         return;
     }
-#if LGB_WARP_RESOLVE
-    if (32u % W.spp == 0u) {          // the samples of a pixel sit in one warp: sum them with shuffles, in sample order, no block barrier
-        const unsigned lane = threadIdx.x & 31u, base = lane - lane % W.spp;
-        D3 c = d3(0, 0, 0);
-        for (uint32_t k = 0; k < W.spp; k++)
-            c = c + d3(__shfl_sync(0xFFFFFFFFu, output.x, base + k), __shfl_sync(0xFFFFFFFFu, output.y, base + k), __shfl_sync(0xFFFFFFFFu, output.z, base + k));
-        if (mine && lane == base && have) {
-            c = c * (1.0 / (double)W.spp);
-            const uint64_t p = (uint32_t)g / W.spp;
-            reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x] = quantise(c);
-        }
-        return;
-    }
-#endif
     rad[3 * threadIdx.x] = output.x; rad[3 * threadIdx.x + 1] = output.y; rad[3 * threadIdx.x + 2] = output.z;
     valid[threadIdx.x] = have ? 1 : 0;
     __syncthreads();
@@ -2491,12 +2265,10 @@ __global__ void __launch_bounds__(256, LGB_LEAN_MIN_BLOCKS) k_shade_lean(DevScen
             }
         }
     }
-#ifndef LGB_LEAN_NO_GENERIC       // (experiments: the register need of the lean code alone)
     if (generic) {
         const Ray64 ray = camera_ray(C, W, x, y, s);
         output = shade_generic_plastic(S, sh, ray, V.hit_t[g], V.hit_ref[g], V.occl[g]);
     }
-#endif
     if constexpr (!FUSED) {
         if (have) { O.radiance[3 * g + 0] = output.x; O.radiance[3 * g + 1] = output.y; O.radiance[3 * g + 2] = output.z; }
     } else {
@@ -2524,113 +2296,6 @@ __global__ void __launch_bounds__(256, LGB_LEAN_MIN_BLOCKS) k_shade_lean(DevScen
         reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)py * W.w + px] = o;
     }
     }
-}
-
-// ================================================================== hit -> film in ONE kernel (plastic scenes with light grids)
-// k_setup + k_gshadow + k_shade_lean for one sample slot without the trip through HBM between them: the surface record and the sign
-// decisions (lean_surface), the per-light gates, the shadow rays through the light grids, the radiance and the film resolve.  Neither
-// ps, nor the gate / sign bytes, nor the occlusion bits are ever stored, and the camera ray and the unit normal are formed once.
-// The same device functions in the same order as the three kernels, so the film is theirs byte for byte (the AOV captures, which need
-// the per-sample buffers, keep the three-kernel form and the tests compare the two).
-#ifndef LGB_SURFACE_MIN_BLOCKS
-#define LGB_SURFACE_MIN_BLOCKS 4
-#endif
-template <bool STATS>
-__device__ __noinline__ D3 surface_generic(const DevScene& S, const DevShade& sh, const Ray64& ray, double t, uint32_t ref, LocalCounters& lc, unsigned& traced, unsigned& occluded) {
-    ShadePoint P; uint32_t id;
-    shade_point<false, false>(S, ray, t, ref, P, id);
-    const uint32_t gate = light_gates(S, ray, P.ps, P.ng, dot(P.wo, P.ng), false);
-    uint32_t occl = ~gate;
-    for (uint32_t l = 0; l < S.n_lights; l++) {
-        if (!((gate >> l) & 1u)) continue;
-        traced++;
-        if (grid_blocked<STATS>(S, P.ps, l, lc)) { occl |= 1u << l; occluded++; }
-    }
-    return shade_generic_plastic(S, sh, ray, t, ref, occl);
-}
-#ifndef LGB_SURFACE_THREADS
-#define LGB_SURFACE_THREADS 256u     // whole pixels per block (spp <= this, else 256)
-#endif
-template <bool STATS>
-__global__ void __launch_bounds__(256, LGB_SURFACE_MIN_BLOCKS) k_surface(DevScene S, DevCamera C, DevShade sh, DevWork W, DevOut O, DevWave V) {
-    const double PI = 3.14159265358979323846264338327950288;
-    __shared__ double rad[3 * kRadStride];
-    __shared__ unsigned char valid[256];
-    __shared__ unsigned char bytes[256 * 3];
-    const unsigned lane = threadIdx.x & 31u;
-    const uint32_t ppb = fdiv(blockDim.x, W.fd_spp);                 // pixels per block
-    const uint32_t tp = fdiv(threadIdx.x, W.fd_spp), s = threadIdx.x - tp * W.spp;
-    const uint64_t p = (uint64_t)blockIdx.x * ppb + tp;
-    const bool mine = tp < ppb && p < W.n_pixels;
-    const uint64_t g = p * W.spp + s;
-    LocalCounters lc = {};
-    unsigned traced = 0, occluded = 0;
-    D3 output = d3(0, 0, 0);
-    bool have = false, generic = false;
-    uint32_t x = 0, y = 0;
-    if (mine) {
-        const uint32_t ref = V.hit_ref[g];
-        const double t = V.hit_t[g];
-        if (ref != kSlotUnused && slot_to_pixel(W, (uint32_t)p, x, y)) {
-            const Ray64 ray = camera_ray(C, W, x, y, s);
-            have = true;
-            if (ref == LGB_MISS) output = background_of(sh, ray.d);                          // background.rs:25-34
-            else {
-                LeanSurf Ls;
-                lean_surface<true>(S, ray, t, ref, 0u, Ls);
-                if (Ls.flags & kSfGeneric) generic = true;
-                else {
-                    const D3 ng = (Ls.flags & kSfNgFlip) ? -Ls.n : Ls.n;
-                    const D3 ps = ray.o + ray.d * t + ng * (2.220446049250313e-16 * 65536.0);   // surface.rs:168, integrate.rs:40 (k_setup's own expression)
-                    uint32_t lit = light_gates(S, ray, ps, ng, 1.0, true);
-                    for (uint32_t l = 0; l < S.n_lights; l++) {
-                        if (!((lit >> l) & 1u)) continue;
-                        traced++;
-                        if (grid_blocked<STATS>(S, ps, l, lc)) { lit &= ~(1u << l); occluded++; }
-                    }
-                    output = lean_radiance(S, sh, ray, t, Ls, Ls.flags, lit);
-                }
-            }
-        }
-    }
-    if (generic) {               // (rare: a sign decision within rounding of a tie -- the reference's own sequence, out of line)
-        const Ray64 ray = camera_ray(C, W, x, y, s);
-        output = surface_generic<STATS>(S, sh, ray, V.hit_t[g], V.hit_ref[g], lc, traced, occluded);
-    }
-    {
-        const uint32_t at = threadIdx.x + (threadIdx.x >> 4);
-        rad[at] = output.x; rad[kRadStride + at] = output.y; rad[2 * kRadStride + at] = output.z;
-        valid[threadIdx.x] = have ? 1 : 0;
-    }
-    __syncthreads();
-    for (uint32_t j = threadIdx.x; j < 3u * ppb; j += blockDim.x) {        // item j: channel j / ppb of pixel j % ppb
-        const uint32_t ch = j >= 2u * ppb ? 2u : (j >= ppb ? 1u : 0u), q = j - ch * ppb, t0 = q * W.spp;
-        if (!valid[t0]) continue;
-        const double* r = rad + ch * kRadStride;
-        double c = 0.0;
-        for (uint32_t k = 0; k < W.spp; k++) c = c + r[t0 + k + ((t0 + k) >> 4)];
-        c = c * (1.0 / (double)W.spp);
-        bytes[3 * q + ch] = (unsigned char)round(fmin(fmax(c, 0.0), 1.0) * 255.0);      // img.rs:56-67
-    }
-    __syncthreads();
-    if (threadIdx.x < ppb && valid[threadIdx.x * W.spp]) {
-        const uint64_t pp = (uint64_t)blockIdx.x * ppb + threadIdx.x;
-        uint32_t px, py;
-        slot_to_pixel(W, pp, px, py);
-        uchar4 o; o.x = bytes[3 * threadIdx.x]; o.y = bytes[3 * threadIdx.x + 1]; o.z = bytes[3 * threadIdx.x + 2]; o.w = 255;
-        reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + pp : (uint64_t)py * W.w + px] = o;
-    }
-    if (O.counters) {
-        const unsigned long long v0 = warp_sum(traced), v1 = warp_sum(occluded);
-        if (lane == 0 && v0) { atomicAdd(&ctr(O)->shadow_traced, v0); atomicAdd(&ctr(O)->shadow_occluded, v1); }
-        if (STATS) {
-            for (int k = 0; k < 3; k++) {
-                unsigned long long a = warp_sum(lc.filter[k]), b = warp_sum(lc.exact[k]);
-                if (lane == 0) { atomicAdd(&ctr(O)->filter[k], a); atomicAdd(&ctr(O)->exact[k], b); }
-            }
-        }
-    }
-    (void)PI;
 }
 
 // Whitted recursion (integrate.rs:69-132) below the closest hits that carry specular lobes (glass, mirror), one thread per listed
@@ -2910,25 +2575,8 @@ cudaError_t launch_fastmath(const double* x, uint64_t n, double* rcp, double* rs
     return cudaGetLastError();
 }
 
-constexpr size_t kPrimarySmem = LGB_SMEM_STACK ? (size_t)2 * kStackDepth * LGB_TRAV_THREADS * 4 : 0;      // dynamic shared memory of the stack variants
-constexpr size_t kShadowSmem = LGB_SMEM_STACK ? (size_t)kStackDepth * LGB_TRAV_THREADS * 4 : 0;
 // ------------------------------------------------------------------ launch wrappers (called from lgb_api.cu)
 bool render_fused(uint32_t spp) { return spp >= 1 && spp <= 256; }      // and !S.general: see launch_render
-#ifndef LGB_SURFACE_FUSED
-#define LGB_SURFACE_FUSED 0          // measured (mixed4k): k_surface 16.0 ms against 2.7 + 7.4 + 4.0 ms for k_setup + k_gshadow + k_shade_lean -- the walk's
-#endif                               // spills on top of the shading state leave L1 (29.6 GB of DRAM writes per frame, profiles/r2_v8_ncu_k_surface.txt)
-#ifndef LGB_SETUP_FUSED
-#define LGB_SETUP_FUSED 0            // measured (mixed4k): k_gshadow<SETUP> 11.5 ms against k_setup 2.7 + k_gshadow 7.4 ms -- like k_surface, the walk
-#endif                               // kernel pays more for the added live state than the 48 B/slot of ps traffic it saves
-// k_gshadow<SETUP> does the hit setup itself for camera rays of scenes with light grids, unless a per-sample buffer is asked for
-bool setup_fused(const DevScene& S, const DevWork& W, const DevOut& O, bool all_shadows) {
-    return LGB_SETUP_FUSED && S.grids && !S.instanced && !all_shadows && !O.aov_id && !O.aov_t && !O.aov_occl && W.mode != 3;
-}
-// k_surface serves plastic scenes with light grids and flat-shaded meshes whenever no per-sample buffer is asked for
-bool surface_fused(const DevScene& S, const DevWork& W, const DevOut& O, bool all_shadows) {
-    return LGB_SURFACE_FUSED && S.grids && !S.instanced && !S.general && !S.tri_nrm && !all_shadows && render_fused(W.spp) &&
-           !O.aov_li && !O.aov_id && !O.aov_t && !O.aov_occl && W.mode != 3;
-}
 
 // `ev` (optional): kRenderEvents events recorded around the phases: start | primary | setup | anchor shadow rays |
 // pretest + remaining shadow rays | shade | resolve.
@@ -2942,18 +2590,6 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
                           KernelLog* klog, ShadeChunks* chunks) {
     if (chunks) chunks->launched = 0;
     auto mark = [&](int i) { if (ev) cudaEventRecord(ev[i], stream); };
-#if LGB_SMEM_STACK
-    {   // the shared-memory stack variant needs more than the default 48 KB of dynamic shared memory (per device: cheap, idempotent)
-        cudaFuncSetAttribute(k_primary<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrimarySmem);
-        cudaFuncSetAttribute(k_primary<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrimarySmem);
-        cudaFuncSetAttribute(k_primary<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrimarySmem);
-        cudaFuncSetAttribute(k_primary<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrimarySmem);
-        cudaFuncSetAttribute(k_shadow<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kShadowSmem);
-        cudaFuncSetAttribute(k_shadow<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kShadowSmem);
-        cudaFuncSetAttribute(k_shadow<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kShadowSmem);
-        cudaFuncSetAttribute(k_shadow<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kShadowSmem);
-    }
-#endif
     const uint64_t total = W.n_pixels * W.spp;
     const bool cache = W.spp > 1;
     const unsigned pblocks = (unsigned)std::min<uint64_t>((total + LGB_TRAV_THREADS - 1) / LGB_TRAV_THREADS, (uint64_t)sms * LGB_MIN_BLOCKS);
@@ -2979,10 +2615,10 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
             KL("k_beam", -1, stream, if (stats) k_beam<true><<<bb, LGB_BEAM_THREADS, 0, stream>>>(S, C, W, O, V); else k_beam<false><<<bb, LGB_BEAM_THREADS, 0, stream>>>(S, C, W, O, V));
             KL("k_leafp", -1, stream, if (stats) k_leafp<true><<<lb, LGB_LEAFP_THREADS, 0, stream>>>(S, C, W, O, V); else k_leafp<false><<<lb, LGB_LEAFP_THREADS, 0, stream>>>(S, C, W, O, V));
             DevWork Wf = W; Wf.slot_list = V.fallback_list; Wf.n_list = 0; Wf.n_list_dev = V.fallback_count;
-            KL("k_primary(fallback)", -1, stream, if (stats) k_primary<true, false><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, Wf, O, V); else k_primary<false, false><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, Wf, O, V));
+            KL("k_primary(fallback)", -1, stream, if (stats) k_primary<true, false><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, Wf, O, V); else k_primary<false, false><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, Wf, O, V));
         } else if (pb) {
-            if (inst) KL("k_primary", -1, stream, if (stats) k_primary<true, true><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, W, O, V); else k_primary<false, true><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, W, O, V));
-            else KL("k_primary", -1, stream, if (stats) k_primary<true, false><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, W, O, V); else k_primary<false, false><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, W, O, V));
+            if (inst) KL("k_primary", -1, stream, if (stats) k_primary<true, true><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, W, O, V); else k_primary<false, true><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, W, O, V));
+            else KL("k_primary", -1, stream, if (stats) k_primary<true, false><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, W, O, V); else k_primary<false, false><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, W, O, V));
         }
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
@@ -2990,22 +2626,9 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
     if (total == 0) return cudaSuccess;
     mark(1);
     const unsigned blocks = (unsigned)((total + 255) / 256), ablocks = (unsigned)((total + kAppendThreads - 1) / kAppendThreads);
-    if (surface_fused(S, W, O, all_shadows)) {      // hit -> film in one kernel (k_surface)
-        const unsigned ft = W.spp <= LGB_SURFACE_THREADS ? LGB_SURFACE_THREADS : 256u;
-        const unsigned fb = (unsigned)((W.n_pixels + (ft / W.spp) - 1) / (ft / W.spp));
-        mark(2); mark(3); mark(4);
-        KL("k_surface(+film)", -1, stream, if (stats) k_surface<true><<<fb, ft, 0, stream>>>(S, C, sh, W, O, V); else k_surface<false><<<fb, ft, 0, stream>>>(S, C, sh, W, O, V));
-        mark(5); mark(6);
-        return cudaGetLastError();
-    }
-    const bool setup_in_gshadow = !W.setup_in_primary && setup_fused(S, W, O, all_shadows);
     if (W.setup_in_primary) {           // k_cprimary<SETUP> has written ps / gate / sign byte: straight to the shadow rays
         mark(2);
         KL("k_gshadow", -1, stream, if (stats) k_gshadow<true, false><<<(unsigned)((total + LGB_GSHADOW_THREADS - 1) / LGB_GSHADOW_THREADS), LGB_GSHADOW_THREADS, 0, stream>>>(S, C, W, O, V); else k_gshadow<false, false><<<(unsigned)((total + LGB_GSHADOW_THREADS - 1) / LGB_GSHADOW_THREADS), LGB_GSHADOW_THREADS, 0, stream>>>(S, C, W, O, V));
-        mark(3);
-    } else if (setup_in_gshadow) {             // hit setup inside the shadow kernel: ps never leaves the registers
-        mark(2);
-        KL("k_gshadow(+setup)", -1, stream, if (stats) k_gshadow<true, false, true><<<(unsigned)((total + LGB_GSHADOW_THREADS - 1) / LGB_GSHADOW_THREADS), LGB_GSHADOW_THREADS, 0, stream>>>(S, C, W, O, V); else k_gshadow<false, false, true><<<(unsigned)((total + LGB_GSHADOW_THREADS - 1) / LGB_GSHADOW_THREADS), LGB_GSHADOW_THREADS, 0, stream>>>(S, C, W, O, V));
         mark(3);
     } else {
     if (inst) KL("k_setup", -1, stream, if (all_shadows) k_setup<true, true><<<ablocks, kAppendThreads, 0, stream>>>(S, C, sh, W, O, V); else k_setup<false, true><<<ablocks, kAppendThreads, 0, stream>>>(S, C, sh, W, O, V));
@@ -3025,7 +2648,7 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
         const int lane = nside ? (int)(l % (uint32_t)(nside + 1)) : 0;
         cudaStream_t ls = lane ? side->s[lane - 1] : stream;
         uint2* blist = lane ? V.beam_list2 : V.beam_list; uint32_t* bcount = lane ? V.beam_count2 : V.beam_count;
-        const bool sbeams = LGB_SHADOW_BEAMS && W.beams && cache && !inst && blist && lane < 2;
+        const bool sbeams = W.beams && cache && !inst && blist && lane < 2;
         for (int which = kQueueA; which <= (cache ? kQueueC : kQueueA); which += 2) {
             const unsigned sb = which == kQueueA ? (unsigned)std::min<uint64_t>((W.n_pixels + LGB_TRAV_THREADS - 1) / LGB_TRAV_THREADS, pblocks) : pblocks;
             if (which == kQueueC) {
@@ -3040,8 +2663,8 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
                 KL("k_pretest", (int)l, ls, if (inst) k_pretest<true><<<tb, kAppendThreads, 0, ls>>>(S, W, O, V, l); else k_pretest<false><<<tb, kAppendThreads, 0, ls>>>(S, W, O, V, l));
             }
             const char* sname = which == kQueueA ? "k_shadow(anchors)" : "k_shadow(rest)";
-            if (inst) KL(sname, (int)l, ls, if (stats) k_shadow<true, true><<<sb, LGB_TRAV_THREADS, kShadowSmem, ls>>>(S, W, O, V, l, which); else k_shadow<false, true><<<sb, LGB_TRAV_THREADS, kShadowSmem, ls>>>(S, W, O, V, l, which));
-            else KL(sname, (int)l, ls, if (stats) k_shadow<true, false><<<sb, LGB_TRAV_THREADS, kShadowSmem, ls>>>(S, W, O, V, l, which); else k_shadow<false, false><<<sb, LGB_TRAV_THREADS, kShadowSmem, ls>>>(S, W, O, V, l, which));
+            if (inst) KL(sname, (int)l, ls, if (stats) k_shadow<true, true><<<sb, LGB_TRAV_THREADS, 0, ls>>>(S, W, O, V, l, which); else k_shadow<false, true><<<sb, LGB_TRAV_THREADS, 0, ls>>>(S, W, O, V, l, which));
+            else KL(sname, (int)l, ls, if (stats) k_shadow<true, false><<<sb, LGB_TRAV_THREADS, 0, ls>>>(S, W, O, V, l, which); else k_shadow<false, false><<<sb, LGB_TRAV_THREADS, 0, ls>>>(S, W, O, V, l, which));
             if (which == kQueueA && l == 0) mark(3);      // (the anchor / rest split of the first light only)
         }
     }
@@ -3095,15 +2718,15 @@ cudaError_t launch_level(const DevScene& S, const DevCamera& C, const DevShade& 
     const unsigned pb = (unsigned)std::min<uint64_t>((total + LGB_TRAV_THREADS - 1) / LGB_TRAV_THREADS, (uint64_t)sms * LGB_MIN_BLOCKS);
     const unsigned blocks = (unsigned)((total + 255) / 256), ablocks = (unsigned)((total + kAppendThreads - 1) / kAppendThreads);
     if (S.instanced) {
-        k_primary<false, true, true><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, W, O, V);
+        k_primary<false, true, true><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, W, O, V);
         k_setup<false, true, true><<<ablocks, kAppendThreads, 0, stream>>>(S, C, sh, W, O, V);
-        for (uint32_t l = 0; l < S.n_lights; l++) k_shadow<false, true><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, W, O, V, l, kQueueA);
+        for (uint32_t l = 0; l < S.n_lights; l++) k_shadow<false, true><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, W, O, V, l, kQueueA);
         k_shade<true, false, true, true><<<blocks, 256, 0, stream>>>(S, C, sh, W, O, V);
     } else {
-        k_primary<false, false, true><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, C, W, O, V);
+        k_primary<false, false, true><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, C, W, O, V);
         k_setup<false, false, true><<<ablocks, kAppendThreads, 0, stream>>>(S, C, sh, W, O, V);
         if (S.grids) { DevOut Os = O; Os.counters = shadow_counters; k_gshadow<false, false><<<(unsigned)((total + LGB_GSHADOW_THREADS - 1) / LGB_GSHADOW_THREADS), LGB_GSHADOW_THREADS, 0, stream>>>(S, C, W, Os, V); }
-        else for (uint32_t l = 0; l < S.n_lights; l++) k_shadow<false, false><<<pb, LGB_TRAV_THREADS, kPrimarySmem, stream>>>(S, W, O, V, l, kQueueA);
+        else for (uint32_t l = 0; l < S.n_lights; l++) k_shadow<false, false><<<pb, LGB_TRAV_THREADS, 0, stream>>>(S, W, O, V, l, kQueueA);
         k_shade<false, false, true, true><<<blocks, 256, 0, stream>>>(S, C, sh, W, O, V);
     }
     return cudaGetLastError();
