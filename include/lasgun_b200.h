@@ -297,6 +297,15 @@ int lgb_capture_aov(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, uint
 int lgb_capture_device(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, uint32_t tile_rank,
                        uint32_t tile_ranks, void* d_film, void* stream, lgb_stats* stats);
 
+/* Linear film: the colour the RGBA8 film quantises (in-order sum of the samples of a pixel times 1/spp, integrate.rs:16-20),
+ * rounded to nearest float32, NOT clamped and NOT quantised.  Row-major (h, w, 3) float32, 12 bytes per pixel, pixel (x, y) at
+ * d_rgb[3 * (y * w + x)].  Otherwise the contract of lgb_capture_device: tiles of tile_rank / tile_ranks (other pixels untouched),
+ * d_rgb may be a peer pointer, a device group splits the tiles over its devices, asynchronous on `stream` unless stats != NULL.
+ * d_rgb == NULL is LGB_ERR_INVALID (there is no context-owned float film).  An addition beyond the reference API: the shading
+ * is computed in f64 on the device anyway, so light above 1.0 and steps finer than 1/255 reach the caller without a host trip. */
+int lgb_capture_linear(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, uint32_t tile_rank, uint32_t tile_ranks,
+                       float* d_rgb, void* stream, lgb_stats* stats);
+
 /* Per-kernel timing of one frame (bench / roofline): the frame of lgb_capture_device (all tiles) with a pair of CUDA events around
  * EVERY kernel launch, all launches on one stream (the shadow chains of different lights do not overlap in this call), and, with
  * LGB_OPT_COUNT_WORK set, each launch's share of the work counters.  Entries come in launch order; *n_out is the number of

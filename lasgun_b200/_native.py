@@ -16,13 +16,14 @@ _lib = None
 
 LGB_OK, LGB_ERR_INVALID, LGB_ERR_CUDA, LGB_ERR_UNSUPPORTED, LGB_ERR_NOMEM, LGB_ERR_NO_DEVICE = 0, -1, -2, -3, -4, -5
 LGB_MISS = 0xFFFFFFFF
+CUDA_STREAM_LEGACY = 0x1                 # cudaStreamLegacy (driver_types.h): the legacy default stream as a stream handle
 LGB_LEAF_FLAG = 0x80000000
 
 # Every symbol include/lasgun_b200.h declares (checked by tests/test_abi.py without a GPU).
 ABI_SYMBOLS = [
     "lgb_build_probe", "lgb_device_count", "lgb_init", "lgb_init_devices", "lgb_context_devices", "lgb_set_option", "lgb_shutdown", "lgb_last_error", "lgb_status_string", "lgb_scene_create",
     "lgb_film_alloc_shared", "lgb_film_open_shared", "lgb_film_release_shared", "lgb_film_signal", "lgb_film_wait", "lgb_scene_destroy", "lgb_scene_layout_bytes", "lgb_scene_export", "lgb_scene_import", "lgb_scene_verify", "lgb_scene_device_bytes", "lgb_scene_build_ms", "lgb_scene_node_count", "lgb_capture", "lgb_capture_subset", "lgb_capture_aov",
-    "lgb_capture_device", "lgb_capture_profile", "lgb_trace_rays", "lgb_debug_fastmath", "lgb_measure_l2_read_gbs", "lgb_measure_fp32_gops", "lgb_measure_fp64_gops",
+    "lgb_capture_device", "lgb_capture_linear", "lgb_capture_profile", "lgb_trace_rays", "lgb_debug_fastmath", "lgb_measure_l2_read_gbs", "lgb_measure_fp32_gops", "lgb_measure_fp64_gops",
 ]
 
 
@@ -125,6 +126,7 @@ def lib():
         "lgb_capture_subset": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, u8p, C.POINTER(Stats)]),
         "lgb_capture_aov": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, u8p, u32p, dp, u32p, dp, C.POINTER(Stats)]),
         "lgb_capture_device": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, C.POINTER(Stats)]),
+        "lgb_capture_linear": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, fp, vp, C.POINTER(Stats)]),
         "lgb_capture_profile": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, vp, C.POINTER(KernelTime), C.c_uint32, u32p, C.POINTER(Stats)]),
         "lgb_trace_rays": (C.c_int, [vp, vp, dp, C.c_uint64, u32p, dp, dp, dp]),
         "lgb_debug_fastmath": (C.c_int, [vp, dp, C.c_uint64, dp, dp]),
@@ -487,6 +489,27 @@ class DeviceScene:
         self.ctx.check(lib().lgb_capture_device(self.ctx.h, self.h, w, h, rank, ranks, C.c_void_p(d_film_ptr),
                                                 C.c_void_p(stream) if stream else None, C.byref(st) if want_stats else None))
         return st.as_dict() if want_stats else None
+
+    def capture_linear(self, w, h, out=None, rank=0, ranks=1, stream=None, want_stats=False):
+        """lgb_capture_linear: the linear film (the colour the RGBA8 film quantises, as float32, neither clamped nor quantised) as a
+        torch.float32 CUDA tensor of shape (h, w, 3), on the context's device unless `out` is given.  Enqueued on `stream` (a
+        torch.cuda.Stream; default torch.cuda.current_stream()) and asynchronous unless want_stats.  Returns the tensor, or
+        (tensor, stats dict) with want_stats."""
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        if out is None:
+            out = torch.empty((h, w, 3), dtype=torch.float32, device=dev)
+        elif out.dtype != torch.float32 or out.device != dev or tuple(out.shape) != (h, w, 3) or not out.is_contiguous():
+            raise ValueError(f"capture_linear: out must be a contiguous float32 tensor of shape ({h}, {w}, 3) on {dev}, "
+                             f"got {out.dtype} {tuple(out.shape)} on {out.device}{'' if out.is_contiguous() else ', not contiguous'}")
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        # torch's default stream is the legacy one (handle 0); NULL would mean the context's private stream, so pass cudaStreamLegacy
+        handle = stream.cuda_stream or CUDA_STREAM_LEGACY
+        st = Stats() if want_stats else None
+        self.ctx.check(lib().lgb_capture_linear(self.ctx.h, self.h, w, h, rank, ranks, C.cast(C.c_void_p(out.data_ptr()), C.POINTER(C.c_float)),
+                                                C.c_void_p(handle), C.byref(st) if want_stats else None))
+        return (out, st.as_dict()) if want_stats else out
 
     def capture_profile(self, w, h, d_film_ptr=0):
         """lgb_capture_profile: (list of per-launch dicts in launch order, frame stats)."""

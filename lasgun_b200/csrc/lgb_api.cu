@@ -20,11 +20,11 @@
 
 namespace lgb {
 constexpr int kRenderEvents = 7;
-cudaError_t launch_render(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, bool stats, bool all_shadows, int sms, cudaStream_t, cudaEvent_t* ev, int part, const SideStreams* side, KernelLog* klog, ShadeChunks* chunks = nullptr);
+cudaError_t launch_render(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, bool stats, bool all_shadows, int sms, cudaStream_t, cudaEvent_t* ev, int part, const SideStreams* side, KernelLog* klog, ShadeChunks* chunks = nullptr, bool linear = false);
 bool render_fused(uint32_t spp);
 cudaError_t launch_level(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, int sms, cudaStream_t, DevCounters* shadow_counters);
 cudaError_t launch_gather(const SpawnRec* recs, const uint32_t* nspec, double* rad_parent, const double* rad_child, uint64_t n_upper, cudaStream_t);
-cudaError_t launch_resolve(const DevWork&, const DevOut&, cudaStream_t);
+cudaError_t launch_resolve(const DevWork&, const DevOut&, cudaStream_t, bool linear);
 cudaError_t launch_export_li(const DevWork&, const DevOut&, const DevWave&, cudaStream_t);
 cudaError_t launch_trace(const DevScene&, const TraceBox&, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns, cudaStream_t);
 cudaError_t launch_l2_read(const void* buf, uint64_t bytes, int iters, float* sink, int sms, cudaStream_t);
@@ -1383,6 +1383,7 @@ struct CaptureArgs {
     bool klog_no_camgrid = false;
     void* host_film = nullptr;   // lgb_capture: the caller's film; where the frame allows it the read-back starts behind the first slice of the shade kernel
     KernelLog* klog = nullptr;   // lgb_capture_profile: events and counter snapshots around every launch (one stream)
+    bool linear = false;         // lgb_capture_linear: d_film is the (h, w, 3) f32 linear film, not RGBA8
 };
 
 // Wavefront buffers of `nslots` sample slots carved out of one allocation (layout: DevWave, lgb_types.cuh).
@@ -1645,15 +1646,15 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
                 CU(c, launch_render(s->dev, s->cam, s->shade, W2, O, V, st_on, a.aov, c->sm_count, st, ties <= V.tie_cap ? nullptr : pev, 1, side, a.klog));
             }
             if (int rc = sync_scene_copy(c, s, st)) return rc;
-            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 2 | wf, side, a.klog, chunks));
+            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 2 | wf, side, a.klog, chunks, a.linear));
         } else {
             if (int rc = sync_scene_copy(c, s, st)) return rc;
-            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 3 | wf, side, a.klog, chunks));
+            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 3 | wf, side, a.klog, chunks, a.linear));
         }
         if (wf && total) {                     // materials beyond plastic: the levels of the specular ray trees, then the film
             if (S.specular && S.recursion > 0) if (int rc = run_whitted_levels(c, s, O, total, st, stats != nullptr, &level_rays, &level_launches)) return rc;
             if (pev) CU(c, cudaEventRecord(pev[5], st));
-            CU(c, launch_resolve(W, O, st));
+            CU(c, launch_resolve(W, O, st, a.linear));
             if (pev) CU(c, cudaEventRecord(pev[6], st));
         }
         if (O.aov_li) CU(c, launch_export_li(W, O, V, st));
@@ -1731,7 +1732,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
 // into the leader's film -- the peers' uchar4 stores cross NVLink while their other tiles are still being shaded, no collective
 // and no gather pass -- each on its own host thread (a capture holds short synchronisation points: tile-list upload, the
 // lazy-tree tie count, the statistics), and the call returns when every device's stream is drained.
-static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void* film, lgb_stats* stats) {
+static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void* film, lgb_stats* stats, bool linear = false) {
     const uint32_t n = 1 + (uint32_t)c->peers.size();
     if (s->replicas.size() != c->peers.size()) return fail(c, LGB_ERR_INVALID, "capture: the scene was not created on this device group");
     if (!s->dev.nodes && s->deferred.scratch) {          // deferred BVH: the leader decides for the group before anybody renders
@@ -1747,10 +1748,12 @@ static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void*
     for (uint32_t k = 1; k < n; k++)
         workers.emplace_back([&, k] {
             CaptureArgs a{w, h, 0, k, n, 0, 0, false, film, nullptr};
+            a.linear = linear;
             rc[k] = run_capture(c->peers[k - 1], s->replicas[k - 1], a, &st[k], true);
         });
     {
         CaptureArgs a{w, h, 0, 0, n, 0, 0, false, film, nullptr};
+        a.linear = linear;
         rc[0] = run_capture(c, s, a, &st[0], true);
     }
     for (std::thread& t : workers) t.join();
@@ -1776,15 +1779,26 @@ static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void*
     return LGB_OK;
 }
 
-int lgb_capture_device(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t rank, uint32_t ranks, void* d_film, void* stream, lgb_stats* stats) {
-    if (!d_film) return fail(c, LGB_ERR_INVALID, "lgb_capture_device: d_film is NULL");
+// lgb_capture_device and lgb_capture_linear: the frame (or the tiles of tile_rank) into a caller's device buffer, RGBA8 or linear f32.
+static int capture_to_device(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t rank, uint32_t ranks, void* d_film, void* stream, lgb_stats* stats, bool linear) {
     if (c && !c->peers.empty() && ranks == 1) {              // device group: the whole frame, split over the group; blocking
         if (stream) CU(c, cudaStreamSynchronize((cudaStream_t)stream));        // the caller's earlier work on the film (a clear) is done
         lgb_stats local;
-        return group_capture(c, s, w, h, d_film, stats ? stats : &local);
+        return group_capture(c, s, w, h, d_film, stats ? stats : &local, linear);
     }
     CaptureArgs a{w, h, 0, rank, ranks, 0, 0, false, d_film, (cudaStream_t)stream};
+    a.linear = linear;
     return run_capture(c, s, a, stats, stats != nullptr);
+}
+
+int lgb_capture_device(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t rank, uint32_t ranks, void* d_film, void* stream, lgb_stats* stats) {
+    if (!d_film) return fail(c, LGB_ERR_INVALID, "lgb_capture_device: d_film is NULL");
+    return capture_to_device(c, s, w, h, rank, ranks, d_film, stream, stats, false);
+}
+
+int lgb_capture_linear(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t tile_rank, uint32_t tile_ranks, float* d_rgb, void* stream, lgb_stats* stats) {
+    if (!d_rgb) return fail(c, LGB_ERR_INVALID, "lgb_capture_linear: d_rgb is NULL");
+    return capture_to_device(c, s, w, h, tile_rank, tile_ranks, d_rgb, stream, stats, true);
 }
 
 // The film goes to the caller's buffer.  A pageable one (the reference's Film is a Vec, film.rs:22-45) makes cudaMemcpy bounce through

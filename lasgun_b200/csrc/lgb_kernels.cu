@@ -1986,9 +1986,15 @@ __device__ __forceinline__ uchar4 quantise(D3 c) {                     // img.rs
     px.w = 255;
     return px;
 }
+// The linear film (lgb_capture_linear): the colour quantise() would receive, rounded to nearest f32, 3 floats per pixel.
+__device__ __forceinline__ void store_linear(uint8_t* film, uint64_t i, D3 c) {
+    float* f = reinterpret_cast<float*>(film) + 3 * i;
+    f[0] = __double2float_rn(c.x); f[1] = __double2float_rn(c.y); f[2] = __double2float_rn(c.z);
+}
 // Radiance of every sample slot (integrate.rs:23-80) and, FUSED (spp <= 256: a block holds whole pixels), the film:
 // the samples of a pixel meet in shared memory and are summed in sample order (integrate.rs:16-20), so the
 // 24 B/sample radiance buffer and k_resolve drop out.  Thread t of a block: pixel t / spp of the block, sample t % spp.
+// LINEAR (FUSED only): the film is the linear f32 one (store_linear) instead of RGBA8.
 // The rays below one specular hit (specular_reflect / specular_transmit, integrate.rs:82-132) appended to the next level of the
 // wavefront: reflected rays fill the level's slots from 0, transmitted ones from V.next_t_base, so each kind stays with its own
 // (neighbouring rays of a warp then point the same way); one record per hit tells k_gather where the children are.
@@ -2031,7 +2037,7 @@ __device__ __forceinline__ void spawn_children(const ShadePoint& P, const DevWav
 
 // GENERAL (scenes with Oren-Nayar, metal, glass or mirror; never FUSED): every material's BSDF::f, and the slots whose closest hit
 // carries specular lobes are listed for k_secondary.
-template <bool INST, bool FUSED, bool GENERAL = false, bool RAYBUF = false>
+template <bool INST, bool FUSED, bool GENERAL = false, bool RAYBUF = false, bool LINEAR = false>
 __global__ void __launch_bounds__(256, GENERAL ? LGB_GSHADE_MIN_BLOCKS : LGB_SHADE_MIN_BLOCKS) k_shade(DevScene S, DevCamera C, DevShade sh, DevWork W, DevOut O, DevWave V) {
     const double PI = 3.14159265358979323846264338327950288;
     const uint64_t total = W.n_pixels * W.spp;
@@ -2103,7 +2109,8 @@ __global__ void __launch_bounds__(256, GENERAL ? LGB_GSHADE_MIN_BLOCKS : LGB_SHA
         for (uint32_t k = 0; k < W.spp; k++) c = c + d3(rad[3 * (threadIdx.x + k)], rad[3 * (threadIdx.x + k) + 1], rad[3 * (threadIdx.x + k) + 2]);
         c = c * (1.0 / (double)W.spp);
         const uint64_t p = (uint32_t)g / W.spp;
-        reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x] = quantise(c);
+        if constexpr (LINEAR) store_linear(O.film, W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x, c);
+        else reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x] = quantise(c);
     }
 }
 
@@ -2216,14 +2223,14 @@ __device__ __forceinline__ D3 shade_generic_plastic(const DevScene& S, const Dev
 #endif
 // FUSED (spp <= 256): a block holds whole pixels (thread t: pixel t / spp of the block, sample t % spp); the samples meet in shared
 // memory, one thread per (pixel, channel) sums them in sample order (integrate.rs:16-20) and quantises (img.rs:56-67), one thread per
-// pixel stores the uchar4.
+// pixel stores the uchar4.  LINEAR (FUSED only): the thread that sums a (pixel, channel) stores its f32 to the linear film itself.
 constexpr int kRadStride = 256 + 16 + 1;           // per channel; index t + t / 16 keeps the per-pixel runs on different banks
-template <bool FUSED>
+template <bool FUSED, bool LINEAR = false>
 __global__ void __launch_bounds__(256, LGB_LEAN_MIN_BLOCKS) k_shade_lean(DevScene S, DevCamera C, DevShade sh, DevWork W, DevOut O, DevWave V) {
     const double PI = 3.14159265358979323846264338327950288;
     __shared__ double rad[FUSED ? 3 * kRadStride : 3];
     __shared__ unsigned char valid[FUSED ? 256 : 1];
-    __shared__ unsigned char bytes[FUSED ? 256 * 3 : 1];
+    __shared__ unsigned char bytes[FUSED && !LINEAR ? 256 * 3 : 1];
     uint64_t g;
     uint32_t p32, s;
     bool mine;
@@ -2285,8 +2292,16 @@ __global__ void __launch_bounds__(256, LGB_LEAN_MIN_BLOCKS) k_shade_lean(DevScen
         double c = 0.0;
         for (uint32_t k = 0; k < W.spp; k++) c = c + r[t0 + k + ((t0 + k) >> 4)];
         c = c * (1.0 / (double)W.spp);
-        bytes[3 * q + ch] = (unsigned char)round(fmin(fmax(c, 0.0), 1.0) * 255.0);      // img.rs:56-67
+        if constexpr (LINEAR) {
+            const uint64_t p = ((uint64_t)blockIdx.x + W.block_off) * ppb + q;
+            uint32_t px, py;
+            slot_to_pixel(W, p, px, py);
+            reinterpret_cast<float*>(O.film)[3 * (W.compact_out ? W.compact_base + p : (uint64_t)py * W.w + px) + ch] = __double2float_rn(c);
+        } else {
+            bytes[3 * q + ch] = (unsigned char)round(fmin(fmax(c, 0.0), 1.0) * 255.0);      // img.rs:56-67
+        }
     }
+    if constexpr (!LINEAR) {
     __syncthreads();
     if (threadIdx.x < ppb && valid[threadIdx.x * W.spp]) {
         const uint64_t p = ((uint64_t)blockIdx.x + W.block_off) * ppb + threadIdx.x;
@@ -2294,6 +2309,7 @@ __global__ void __launch_bounds__(256, LGB_LEAN_MIN_BLOCKS) k_shade_lean(DevScen
         slot_to_pixel(W, p, px, py);
         uchar4 o; o.x = bytes[3 * threadIdx.x]; o.y = bytes[3 * threadIdx.x + 1]; o.z = bytes[3 * threadIdx.x + 2]; o.w = 255;
         reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)py * W.w + px] = o;
+    }
     }
     }
 }
@@ -2407,7 +2423,8 @@ __global__ void __launch_bounds__(256) k_gather(const SpawnRec* recs, const uint
     rad_parent[3 * (size_t)r.slot] = output.x; rad_parent[3 * (size_t)r.slot + 1] = output.y; rad_parent[3 * (size_t)r.slot + 2] = output.z;
 }
 
-// integrate.rs:16-20 + img.rs:56-67: in-order sum of the samples, weight, quantise, store.
+// integrate.rs:16-20 + img.rs:56-67: in-order sum of the samples, weight, quantise, store.  LINEAR: the f32 store of store_linear instead.
+template <bool LINEAR>
 __global__ void __launch_bounds__(256) k_resolve(DevWork W, DevOut O) {
     const uint64_t p = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= W.n_pixels) return;
@@ -2418,7 +2435,8 @@ __global__ void __launch_bounds__(256) k_resolve(DevWork W, DevOut O) {
     const double* r = O.radiance + 3 * p * W.spp;
     for (uint32_t s = 0; s < W.spp; s++) c = c + d3(r[3 * s], r[3 * s + 1], r[3 * s + 2]);
     c = c * weight;
-    reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x] = quantise(c);
+    if constexpr (LINEAR) store_linear(O.film, W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x, c);
+    else reinterpret_cast<uchar4*>(O.film)[W.compact_out ? W.compact_base + p : (uint64_t)y * W.w + x] = quantise(c);
 }
 
 // Per-sample radiance for lgb_capture_aov: radiance buffer (slot order) -> caller's order ((y * w + x) * spp + s).
@@ -2587,7 +2605,7 @@ bool render_fused(uint32_t spp) { return spp >= 1 && spp <= 256; }      // and !
 #define KL(nm, light, st, ...) do { if (klog) klog->begin(nm, light, st); __VA_ARGS__; if (klog) klog->end(st, O.counters); } while (0)
 cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade& sh, const DevWork& W, const DevOut& O,
                           const DevWave& V, bool stats, bool all_shadows, int sms, cudaStream_t stream, cudaEvent_t* ev, int part, const SideStreams* side,
-                          KernelLog* klog, ShadeChunks* chunks) {
+                          KernelLog* klog, ShadeChunks* chunks, bool linear) {
     if (chunks) chunks->launched = 0;
     auto mark = [&](int i) { if (ev) cudaEventRecord(ev[i], stream); };
     const uint64_t total = W.n_pixels * W.spp;
@@ -2680,11 +2698,11 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
         }
         mark(5);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
-        KL("k_resolve", -1, stream, k_resolve<<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O));
+        KL("k_resolve", -1, stream, if (linear) k_resolve<true><<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O); else k_resolve<false><<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O));
     } else if (render_fused(W.spp) && !O.aov_li) {   // whole pixels per block: shade and resolve in one kernel, no radiance buffer
         const unsigned ft = W.spp <= LGB_FUSED_THREADS ? LGB_FUSED_THREADS : 256u;        // threads per block: whole pixels, as few of them as the option allows
         const unsigned fb = (unsigned)((W.n_pixels + (ft / W.spp) - 1) / (ft / W.spp));
-        if (chunks && chunks->want > 1 && !inst && !klog && fb >= 64u * chunks->want) {
+        if (chunks && chunks->want > 1 && !inst && !klog && !linear && fb >= 64u * chunks->want) {      // (the RGBA8 read-back of lgb_capture)
             // slices of consecutive blocks = consecutive pixel slots = (single-rank tile lists are row-major) consecutive rows of macro tiles
             const unsigned K = std::min<unsigned>(chunks->want, 8u), ppb = ft / W.spp;
             for (unsigned k = 0; k < K; k++) {
@@ -2695,7 +2713,9 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
                 chunks->done_pixels[k] = std::min<uint64_t>((uint64_t)b1 * ppb, W.n_pixels);
             }
             chunks->launched = K;
-        } else
+        } else if (linear)
+        KL(inst ? "k_shade(+linear film)" : "k_shade_lean(+linear film)", -1, stream, if (inst) k_shade<true, true, false, false, true><<<fb, ft, 0, stream>>>(S, C, sh, W, O, V); else k_shade_lean<true, true><<<fb, ft, 0, stream>>>(S, C, sh, W, O, V));
+        else
         KL(inst ? "k_shade(+film)" : "k_shade_lean(+film)", -1, stream, if (inst) k_shade<true, true><<<fb, ft, 0, stream>>>(S, C, sh, W, O, V); else k_shade_lean<true><<<fb, ft, 0, stream>>>(S, C, sh, W, O, V));
         mark(5);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
@@ -2703,7 +2723,7 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
         KL(inst ? "k_shade" : "k_shade_lean", -1, stream, if (inst) k_shade<true, false><<<blocks, 256, 0, stream>>>(S, C, sh, W, O, V); else k_shade_lean<false><<<blocks, 256, 0, stream>>>(S, C, sh, W, O, V));
         mark(5);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
-        KL("k_resolve", -1, stream, k_resolve<<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O));
+        KL("k_resolve", -1, stream, if (linear) k_resolve<true><<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O); else k_resolve<false><<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O));
     }
     mark(6);
     return cudaGetLastError();
@@ -2742,9 +2762,10 @@ cudaError_t launch_export_li(const DevWork& W, const DevOut& O, const DevWave& V
     k_export_li<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(W, O, V);
     return cudaGetLastError();
 }
-cudaError_t launch_resolve(const DevWork& W, const DevOut& O, cudaStream_t stream) {
+cudaError_t launch_resolve(const DevWork& W, const DevOut& O, cudaStream_t stream, bool linear) {
     if (W.n_pixels == 0) return cudaSuccess;
-    k_resolve<<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O);
+    if (linear) k_resolve<true><<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O);
+    else k_resolve<false><<<(unsigned)((W.n_pixels + 255) / 256), 256, 0, stream>>>(W, O);
     return cudaGetLastError();
 }
 cudaError_t launch_trace(const DevScene& S, const TraceBox& B, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ng, double* ns, cudaStream_t stream) {

@@ -267,7 +267,7 @@ struct DevOut {
     uint32_t* aov_occl;
     double* aov_li;                  // optional: the radiance of every sample (li, integrate.rs:23), global sample index
     DevCounters* counters;           // optional
-    uint8_t* film;                   // row-major RGBA8 (may be a peer pointer)
+    uint8_t* film;                   // row-major RGBA8, or the (h, w, 3) f32 linear film of lgb_capture_linear (may be a peer pointer)
 };
 
 }  // namespace lgb

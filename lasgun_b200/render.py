@@ -22,6 +22,10 @@ class Accel:
     def from_scene(scene: Scene, **kw):
         return Accel(scene, **kw)
 
+    def capture_linear(self, w: int, h: int, out=None):
+        """The linear film of this resident scene: a float32 CUDA tensor (h, w, 3), enqueued on torch.cuda.current_stream()."""
+        return self.dev.capture_linear(w, h, out=out)
+
     def close(self):
         self.dev.destroy()
 
@@ -34,6 +38,19 @@ def capture(scene: Scene, film: Film, ctx: N.Context | None = None):
     finally:
         root.close()
     return stats
+
+
+def capture_linear(scene: Scene, w: int, h: int, ctx: N.Context | None = None):
+    """The linear film of `capture`: the in-order sample sum times 1/spp (integrate.rs:16-20) of every pixel as float32, neither
+    clamped to [0, 1] nor quantised -- a torch.float32 CUDA tensor of shape (h, w, 3), returned once the frame is complete."""
+    import torch
+    root = Accel(scene, ctx, lazy=True)
+    try:
+        rgb = root.capture_linear(w, h)
+        torch.cuda.current_stream(rgb.device).synchronize()
+    finally:
+        root.close()
+    return rgb
 
 
 def capture_subset(k: int, n: int, root: Accel, film: Film):
