@@ -306,6 +306,32 @@ int lgb_capture_device(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, u
 int lgb_capture_linear(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, uint32_t tile_rank, uint32_t tile_ranks,
                        float* d_rgb, void* stream, lgb_stats* stats);
 
+/* Guides: per-pixel geometry of the camera rays' closest hits, for denoisers, losses and datasets on the GPU.  Row-major device
+ * buffers, pixel (x, y) at index y * w + x; every pointer may be NULL (not written) and may be a peer pointer:
+ *   normal    (h, w, 3) the world-space shading normal ns of each sample's hit, exactly as lgb_trace_rays returns it (transformed,
+ *             swap_backface applied, interpolated for meshes with vertex normals, NOT flipped toward the ray), summed in sample
+ *             order (camera.rs:137-145), times 1/spp, rounded to nearest float32; not renormalised, a miss adds (0, 0, 0)
+ *   depth     (h, w) t of the anchor sample's hit (camera.rs:143) times |view|, rounded to nearest float32; +inf on a miss.  look_at
+ *             keeps up and aux unit and orthogonal to view, so this is the hit's distance along the view axis, perspective or
+ *             orthographic.  |view| = sqrt((vx vx + vy vy) + vz vz) in f64, and t |view| is one f64 product
+ *   prim_id   (h, w) canonical id of the anchor sample's hit (as lgb_capture_aov reports it), or LGB_MISS
+ *   coverage  (h, w) samples of the pixel that hit something / spp, as (float)((double)hits / spp)
+ *   rgb       (h, w, 3) the linear film of lgb_capture_linear, from the same frame; NULL: a geometry pass -- primary rays only,
+ *             no shadow, shading or Whitted work is launched at all (lgb_stats: shadow_rays, shadow_rays_traced,
+ *             shadow_occluded and secondary_rays are 0)
+ * All of them describe the camera ray's first hit: mirrors and glass do not forward what they show.  Otherwise the contract of
+ * lgb_capture_linear (tiles of tile_rank / tile_ranks, every other element untouched; device groups; asynchronous on `stream`
+ * unless stats != NULL).  out == NULL or all five pointers NULL is LGB_ERR_INVALID, and nothing is written. */
+typedef struct lgb_guides {
+    float* rgb;                      /* (h, w, 3) linear film, or NULL */
+    float* normal;                   /* (h, w, 3) or NULL */
+    float* depth;                    /* (h, w)    or NULL */
+    uint32_t* prim_id;               /* (h, w)    or NULL */
+    float* coverage;                 /* (h, w)    or NULL */
+} lgb_guides;
+int lgb_capture_guides(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, uint32_t tile_rank, uint32_t tile_ranks,
+                       const lgb_guides* out, void* stream, lgb_stats* stats);
+
 /* Per-kernel timing of one frame (bench / roofline): the frame of lgb_capture_device (all tiles) with a pair of CUDA events around
  * EVERY kernel launch, all launches on one stream (the shadow chains of different lights do not overlap in this call), and, with
  * LGB_OPT_COUNT_WORK set, each launch's share of the work counters.  Entries come in launch order; *n_out is the number of

@@ -23,7 +23,7 @@ LGB_LEAF_FLAG = 0x80000000
 ABI_SYMBOLS = [
     "lgb_build_probe", "lgb_device_count", "lgb_init", "lgb_init_devices", "lgb_context_devices", "lgb_set_option", "lgb_shutdown", "lgb_last_error", "lgb_status_string", "lgb_scene_create",
     "lgb_film_alloc_shared", "lgb_film_open_shared", "lgb_film_release_shared", "lgb_film_signal", "lgb_film_wait", "lgb_scene_destroy", "lgb_scene_layout_bytes", "lgb_scene_export", "lgb_scene_import", "lgb_scene_verify", "lgb_scene_device_bytes", "lgb_scene_build_ms", "lgb_scene_node_count", "lgb_capture", "lgb_capture_subset", "lgb_capture_aov",
-    "lgb_capture_device", "lgb_capture_linear", "lgb_capture_profile", "lgb_trace_rays", "lgb_debug_fastmath", "lgb_measure_l2_read_gbs", "lgb_measure_fp32_gops", "lgb_measure_fp64_gops",
+    "lgb_capture_device", "lgb_capture_linear", "lgb_capture_guides", "lgb_capture_profile", "lgb_trace_rays", "lgb_debug_fastmath", "lgb_measure_l2_read_gbs", "lgb_measure_fp32_gops", "lgb_measure_fp64_gops",
 ]
 
 
@@ -74,6 +74,11 @@ class BuildInfo(C.Structure):
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}
+
+
+class Guides(C.Structure):
+    """lgb_guides: the device buffers of lgb_capture_guides (NULL = not written)."""
+    _fields_ = [("rgb", C.c_void_p), ("normal", C.c_void_p), ("depth", C.c_void_p), ("prim_id", C.c_void_p), ("coverage", C.c_void_p)]
 
 
 class KernelTime(C.Structure):
@@ -127,6 +132,7 @@ def lib():
         "lgb_capture_aov": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, u8p, u32p, dp, u32p, dp, C.POINTER(Stats)]),
         "lgb_capture_device": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, C.POINTER(Stats)]),
         "lgb_capture_linear": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, fp, vp, C.POINTER(Stats)]),
+        "lgb_capture_guides": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Guides), vp, C.POINTER(Stats)]),
         "lgb_capture_profile": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32, vp, C.POINTER(KernelTime), C.c_uint32, u32p, C.POINTER(Stats)]),
         "lgb_trace_rays": (C.c_int, [vp, vp, dp, C.c_uint64, u32p, dp, dp, dp]),
         "lgb_debug_fastmath": (C.c_int, [vp, dp, C.c_uint64, dp, dp]),
@@ -510,6 +516,47 @@ class DeviceScene:
         self.ctx.check(lib().lgb_capture_linear(self.ctx.h, self.h, w, h, rank, ranks, C.cast(C.c_void_p(out.data_ptr()), C.POINTER(C.c_float)),
                                                 C.c_void_p(handle), C.byref(st) if want_stats else None))
         return (out, st.as_dict()) if want_stats else out
+
+    GUIDES = ("rgb", "normal", "depth", "prim_id", "coverage")
+
+    def capture_guides(self, w, h, rgb=True, normal=True, depth=True, prim_id=True, coverage=True, out=None, rank=0, ranks=1, stream=None,
+                       want_stats=False):
+        """lgb_capture_guides: per-pixel geometry of the camera rays' closest hits as CUDA tensors, in a dict keyed by the requested
+        outputs: normal (h, w, 3) float32, depth (h, w) float32, prim_id (h, w) int32 holding the u32 id (LGB_MISS reads as -1),
+        coverage (h, w) float32, and rgb (h, w, 3) float32, the linear film of the same frame.  rgb=False renders a geometry pass
+        (primary rays only).  `out` (optional): a dict of caller tensors for some of the requested outputs, checked as
+        capture_linear checks its `out`.  Enqueued on `stream` (default torch.cuda.current_stream()), asynchronous unless want_stats.
+        Returns the dict, or (dict, stats dict) with want_stats."""
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        want = {"rgb": rgb, "normal": normal, "depth": depth, "prim_id": prim_id, "coverage": coverage}
+        shapes = {"rgb": (h, w, 3), "normal": (h, w, 3), "depth": (h, w), "prim_id": (h, w), "coverage": (h, w)}
+        out = dict(out or {})
+        for k in out:
+            if k not in want or not want[k]:
+                raise ValueError(f"capture_guides: out[{k!r}] is not a requested output")
+        res = {}
+        for k in self.GUIDES:
+            if not want[k]:
+                continue
+            dtype = torch.int32 if k == "prim_id" else torch.float32
+            t = out.get(k)
+            if t is None:
+                t = torch.empty(shapes[k], dtype=dtype, device=dev)
+            elif t.dtype != dtype or t.device != dev or tuple(t.shape) != shapes[k] or not t.is_contiguous():
+                raise ValueError(f"capture_guides: out[{k!r}] must be a contiguous {dtype} tensor of shape {shapes[k]} on {dev}, "
+                                 f"got {t.dtype} {tuple(t.shape)} on {t.device}{'' if t.is_contiguous() else ', not contiguous'}")
+            res[k] = t
+        if not res:
+            raise ValueError("capture_guides: no output requested")
+        g = Guides(*[res[k].data_ptr() if k in res else None for k in self.GUIDES])
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        handle = stream.cuda_stream or CUDA_STREAM_LEGACY           # (see capture_linear)
+        st = Stats() if want_stats else None
+        self.ctx.check(lib().lgb_capture_guides(self.ctx.h, self.h, w, h, rank, ranks, C.byref(g), C.c_void_p(handle),
+                                                C.byref(st) if want_stats else None))
+        return (res, st.as_dict()) if want_stats else res
 
     def capture_profile(self, w, h, d_film_ptr=0):
         """lgb_capture_profile: (list of per-launch dicts in launch order, frame stats)."""

@@ -20,7 +20,7 @@
 
 namespace lgb {
 constexpr int kRenderEvents = 7;
-cudaError_t launch_render(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, bool stats, bool all_shadows, int sms, cudaStream_t, cudaEvent_t* ev, int part, const SideStreams* side, KernelLog* klog, ShadeChunks* chunks = nullptr, bool linear = false);
+cudaError_t launch_render(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, bool stats, bool all_shadows, int sms, cudaStream_t, cudaEvent_t* ev, int part, const SideStreams* side, KernelLog* klog, ShadeChunks* chunks = nullptr, bool linear = false, const DevGuides* guides = nullptr);
 bool render_fused(uint32_t spp);
 cudaError_t launch_level(const DevScene&, const DevCamera&, const DevShade&, const DevWork&, const DevOut&, const DevWave&, int sms, cudaStream_t, DevCounters* shadow_counters);
 cudaError_t launch_gather(const SpawnRec* recs, const uint32_t* nspec, double* rad_parent, const double* rad_child, uint64_t n_upper, cudaStream_t);
@@ -1384,6 +1384,7 @@ struct CaptureArgs {
     void* host_film = nullptr;   // lgb_capture: the caller's film; where the frame allows it the read-back starts behind the first slice of the shade kernel
     KernelLog* klog = nullptr;   // lgb_capture_profile: events and counter snapshots around every launch (one stream)
     bool linear = false;         // lgb_capture_linear: d_film is the (h, w, 3) f32 linear film, not RGBA8
+    const lgb_guides* guides = nullptr;   // lgb_capture_guides: d_film = guides->rgb (linear), NULL for a geometry pass
 };
 
 // Wavefront buffers of `nslots` sample slots carved out of one allocation (layout: DevWave, lgb_types.cuh).
@@ -1531,11 +1532,12 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
         if (!a.klog_no_camgrid) if (int rc = ensure_camgrid(c, s, a.w, a.h, total_all, W, st)) return rc;
     }
     const bool grid_shadows = S.grids && !S.instanced;                 // no shadow queues, no occluder cache
+    const bool geometry = a.guides && !a.guides->rgb;                  // lgb_capture_guides without a film: primary rays and k_guides only
     // hit setup inside the camera-grid kernel (no k_setup launch): plain captures whose shadows go through the light grids
-    W.setup_in_primary = (c->setup_in_primary && W.cg_start && grid_shadows && !a.aov && a.mode != 3) ? 1u : 0u;
+    W.setup_in_primary = (c->setup_in_primary && W.cg_start && grid_shadows && !a.aov && a.mode != 3 && !geometry) ? 1u : 0u;
     const bool beam_lists = W.beams && (!W.cg_start || !grid_shadows); // pixel beams (primary) and / or shadow beams
     const bool two_lists = beam_lists && !grid_shadows && S.n_lights > 1 && c->side_streams && c->side.n;
-    const bool need_radiance = !render_fused(W.spp) || S.general || a.want_li;
+    const bool need_radiance = !geometry && (!render_fused(W.spp) || S.general || a.want_li);
     const bool lazy_ties = s->lazy_fn && !s->dev.rank;
     // the queue area also lends its first words to the pixel beams' fallback list and to k_shade's list of specular slots (one u32 per slot)
     const uint32_t queue_nl = grid_shadows ? ((beam_lists || S.specular) ? 1u : 0u) : nl;
@@ -1560,7 +1562,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
     DevOut O{};
     O.radiance = (double*)c->radiance.p;
     O.counters = (DevCounters*)c->counters.p;
-    if (a.d_film) O.film = (uint8_t*)a.d_film;
+    if (a.d_film || a.guides) O.film = (uint8_t*)a.d_film;
     else {
         CU(c, c->film.reserve(std::max<uint64_t>(a.mode == 0 ? area : units_all, 1) * 4));
         O.film = (uint8_t*)c->film.p;
@@ -1570,6 +1572,13 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
         O.aov_id = (uint32_t*)c->aov_id.p; O.aov_t = (double*)c->aov_t.p; O.aov_occl = (uint32_t*)c->aov_occl.p;
         if (a.want_li) { CU(c, c->aov_li.reserve(std::max<uint64_t>(area * W.spp, 1) * 24)); O.aov_li = (double*)c->aov_li.p; }
     }
+    DevGuides G{};
+    if (a.guides) {
+        G.normal = a.guides->normal; G.depth = a.guides->depth; G.prim_id = a.guides->prim_id; G.coverage = a.guides->coverage;
+        const double* v = s->cam.view;
+        G.view_len = std::sqrt((v[0] * v[0] + v[1] * v[1]) + v[2] * v[2]);      // (no contraction in this file)
+    }
+    const DevGuides* guides = a.guides ? &G : nullptr;
     CU(c, cudaMemsetAsync(c->counters.p, 0, kCtrBytes, st));
     CU(c, cudaEventRecord(c->ev0, st));
     cudaEvent_t* pev = (stats && sync_stats && total_all) ? c->phase : nullptr;
@@ -1611,7 +1620,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
             V.tie_list = (uint32_t*)c->ties.p; V.tie_cap = kTieCap;
             if (const char* e = std::getenv("LGB_TIE_CAP")) V.tie_cap = std::min<uint32_t>(kTieCap, (uint32_t)std::strtoul(e, nullptr, 10));   // tests: force the whole-frame re-trace
         }
-        wf = (S.general && c->whitted_wavefront) ? 4 : 0;               // launch_render stops after k_shade; the levels and the resolve follow here
+        wf = (S.general && c->whitted_wavefront && !geometry) ? 4 : 0;  // launch_render stops after k_shade; the levels and the resolve follow here
         if (wf && S.specular && S.recursion > 0 && total) {             // k_shade of the camera wave spawns level 1
             CU(c, c->lvl_ctr.reserve(4 * (kMaxRecursion + 2) * 4));
             CU(c, cudaMemsetAsync(c->lvl_ctr.p, 0, 4 * (kMaxRecursion + 2) * 4, st));
@@ -1646,10 +1655,10 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
                 CU(c, launch_render(s->dev, s->cam, s->shade, W2, O, V, st_on, a.aov, c->sm_count, st, ties <= V.tie_cap ? nullptr : pev, 1, side, a.klog));
             }
             if (int rc = sync_scene_copy(c, s, st)) return rc;
-            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 2 | wf, side, a.klog, chunks, a.linear));
+            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 2 | wf, side, a.klog, chunks, a.linear, guides));
         } else {
             if (int rc = sync_scene_copy(c, s, st)) return rc;
-            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 3 | wf, side, a.klog, chunks, a.linear));
+            CU(c, launch_render(s->dev, s->cam, s->shade, W, O, V, st_on, a.aov, c->sm_count, st, pev, 3 | wf, side, a.klog, chunks, a.linear, guides));
         }
         if (wf && total) {                     // materials beyond plastic: the levels of the specular ray trees, then the film
             if (S.specular && S.recursion > 0) if (int rc = run_whitted_levels(c, s, O, total, st, stats != nullptr, &level_rays, &level_launches)) return rc;
@@ -1692,7 +1701,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
         CU(c, cudaStreamSynchronize(st));
         std::memset(stats, 0, sizeof *stats);
         stats->primary_rays = hc.primary_rays; stats->primary_hits = hc.primary_hits;
-        stats->shadow_rays = hc.primary_hits * s->dev.n_lights;
+        stats->shadow_rays = geometry ? 0 : hc.primary_hits * s->dev.n_lights;
         stats->shadow_rays_traced = hc.shadow_traced; stats->shadow_occluded = hc.shadow_occluded; stats->shadow_cache_hits = hc.shadow_cached;
         stats->node_tests = hc.node_tests; stats->primary_node_tests = hc.p_node_tests;
         for (int k = 0; k < 3; k++) { stats->primary_filter_tests[k] = hc.p_filter[k]; stats->primary_exact_tests[k] = hc.p_exact[k]; }
@@ -1706,7 +1715,9 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
         const uint32_t primary_launches = W.cg_start ? 1u : (W.beams && W.spp >= 4 && !S.instanced) ? 3u : 1u;           // k_cprimary | k_beam + k_leafp + fallback | k_primary
         const uint32_t shade_launches = S.general ? (S.specular && S.recursion && !wf ? 3u : 2u) : (render_fused(W.spp) && !O.aov_li) ? 1u : 2u;
         const uint32_t setup_launches = W.setup_in_primary ? 0u : 1u;                                                                           // 0 when k_cprimary<SETUP> did it
-        stats->kernel_launches = total_all ? level_launches + (uint32_t)n_bands * (primary_launches + setup_launches + shadow_launches + shade_launches) : 0;
+        const uint32_t guide_launches = a.guides ? 1u : 0u;                                                                                   // k_guides
+        stats->kernel_launches = !total_all ? 0 : geometry ? (uint32_t)n_bands * (primary_launches + guide_launches)
+                                 : level_launches + (uint32_t)n_bands * (primary_launches + guide_launches + setup_launches + shadow_launches + shade_launches);
         if (chunks && chunks->launched) stats->kernel_launches += chunks->launched - 1;
         stats->bands = (uint32_t)n_bands;
         float ms = 0.f; CU(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
@@ -1732,7 +1743,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
 // into the leader's film -- the peers' uchar4 stores cross NVLink while their other tiles are still being shaded, no collective
 // and no gather pass -- each on its own host thread (a capture holds short synchronisation points: tile-list upload, the
 // lazy-tree tie count, the statistics), and the call returns when every device's stream is drained.
-static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void* film, lgb_stats* stats, bool linear = false) {
+static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void* film, lgb_stats* stats, bool linear = false, const lgb_guides* guides = nullptr) {
     const uint32_t n = 1 + (uint32_t)c->peers.size();
     if (s->replicas.size() != c->peers.size()) return fail(c, LGB_ERR_INVALID, "capture: the scene was not created on this device group");
     if (!s->dev.nodes && s->deferred.scratch) {          // deferred BVH: the leader decides for the group before anybody renders
@@ -1748,12 +1759,12 @@ static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void*
     for (uint32_t k = 1; k < n; k++)
         workers.emplace_back([&, k] {
             CaptureArgs a{w, h, 0, k, n, 0, 0, false, film, nullptr};
-            a.linear = linear;
+            a.linear = linear; a.guides = guides;
             rc[k] = run_capture(c->peers[k - 1], s->replicas[k - 1], a, &st[k], true);
         });
     {
         CaptureArgs a{w, h, 0, 0, n, 0, 0, false, film, nullptr};
-        a.linear = linear;
+        a.linear = linear; a.guides = guides;
         rc[0] = run_capture(c, s, a, &st[0], true);
     }
     for (std::thread& t : workers) t.join();
@@ -1779,15 +1790,17 @@ static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void*
     return LGB_OK;
 }
 
-// lgb_capture_device and lgb_capture_linear: the frame (or the tiles of tile_rank) into a caller's device buffer, RGBA8 or linear f32.
-static int capture_to_device(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t rank, uint32_t ranks, void* d_film, void* stream, lgb_stats* stats, bool linear) {
+// lgb_capture_device, lgb_capture_linear and lgb_capture_guides: the frame (or the tiles of tile_rank) into a caller's device buffers,
+// RGBA8 or linear f32, and the guides.
+static int capture_to_device(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t rank, uint32_t ranks, void* d_film, void* stream, lgb_stats* stats, bool linear,
+                             const lgb_guides* guides = nullptr) {
     if (c && !c->peers.empty() && ranks == 1) {              // device group: the whole frame, split over the group; blocking
         if (stream) CU(c, cudaStreamSynchronize((cudaStream_t)stream));        // the caller's earlier work on the film (a clear) is done
         lgb_stats local;
-        return group_capture(c, s, w, h, d_film, stats ? stats : &local, linear);
+        return group_capture(c, s, w, h, d_film, stats ? stats : &local, linear, guides);
     }
     CaptureArgs a{w, h, 0, rank, ranks, 0, 0, false, d_film, (cudaStream_t)stream};
-    a.linear = linear;
+    a.linear = linear; a.guides = guides;
     return run_capture(c, s, a, stats, stats != nullptr);
 }
 
@@ -1799,6 +1812,11 @@ int lgb_capture_device(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_
 int lgb_capture_linear(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t tile_rank, uint32_t tile_ranks, float* d_rgb, void* stream, lgb_stats* stats) {
     if (!d_rgb) return fail(c, LGB_ERR_INVALID, "lgb_capture_linear: d_rgb is NULL");
     return capture_to_device(c, s, w, h, tile_rank, tile_ranks, d_rgb, stream, stats, true);
+}
+
+int lgb_capture_guides(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint32_t tile_rank, uint32_t tile_ranks, const lgb_guides* out, void* stream, lgb_stats* stats) {
+    if (!out || !(out->rgb || out->normal || out->depth || out->prim_id || out->coverage)) return fail(c, LGB_ERR_INVALID, "lgb_capture_guides: no output requested");
+    return capture_to_device(c, s, w, h, tile_rank, tile_ranks, out->rgb, stream, stats, true, out);
 }
 
 // The film goes to the caller's buffer.  A pageable one (the reference's Film is a Vec, film.rs:22-45) makes cudaMemcpy bounce through

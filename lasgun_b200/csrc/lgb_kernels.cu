@@ -2464,6 +2464,17 @@ __device__ __forceinline__ double entry_param(const TraceBox& B, const Ray64& r)
     }
     return tn <= tf ? tn : 0.0;
 }
+// The world-space surface record of the closest hit `ref` on `ray` (formed in the primitive's own space, then brought back:
+// bvh.rs:508-518), and its shading normal RayIntersection::ns() (surface.rs:107-118): lgb_trace_rays and lgb_capture_guides.
+template <bool INST>
+__device__ __forceinline__ void world_record(const DevScene& S, const Ray64& ray, uint32_t ref, double& t, Surf& sf) {
+    if (INST) {
+        const uint32_t space = space_of(S, ref);
+        surface_of(S, ray_to_space(S, space, ray), ref, t, sf);
+        record_to_world(S.spaces, space, sf);
+    } else surface_of(S, ray, ref, t, sf);
+}
+__device__ __forceinline__ D3 shading_normal(const Surf& sf) { return sf.has_n ? normalize(sf.n) : normalize(cross(sf.s_dpdu, sf.s_dpdv)); }
 template <bool INST>
 __global__ void __launch_bounds__(128) k_trace(DevScene S, TraceBox B, const double* rays, uint64_t n, uint32_t* ids, double* ts, double* ngs, double* nss) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2493,19 +2504,81 @@ __global__ void __launch_bounds__(128) k_trace(DevScene S, TraceBox B, const dou
     uint32_t id = LGB_MISS; D3 ng = d3(0, 0, 0), ns = d3(0, 0, 0);
     if (h.ref != LGB_MISS) {
         Surf sf; double t = h.t;
-        if (INST) {
-            const uint32_t space = space_of(S, h.ref);
-            surface_of(S, ray_to_space(S, space, ray), h.ref, t, sf);
-            record_to_world(S.spaces, space, sf);
-        } else surface_of(S, ray, h.ref, t, sf);
+        world_record<INST>(S, ray, h.ref, t, sf);
         id = sf.id;
         ng = normalize(cross(sf.g_dpdu, sf.g_dpdv));
-        ns = sf.has_n ? normalize(sf.n) : normalize(cross(sf.s_dpdu, sf.s_dpdv));
+        ns = shading_normal(sf);
     }
     if (ids) ids[i] = id;
     if (ts) ts[i] = h.ref != LGB_MISS ? h.t : CUDART_INF;
     if (ngs) { ngs[3 * i] = ng.x; ngs[3 * i + 1] = ng.y; ngs[3 * i + 2] = ng.z; }
     if (nss) { nss[3 * i] = ns.x; nss[3 * i + 1] = ns.y; nss[3 * i + 2] = ns.z; }
+}
+
+// lgb_capture_guides: per-pixel geometry of the camera rays' closest hits, read from the wave (hit_t / hit_ref) after the primary
+// phase and before anything overwrites it.  A block holds whole pixels (kGuideThreads / spp of them; above kGuideThreads samples,
+// one pixel in passes of kGuideThreads samples): each thread takes one sample slot, rebuilds its camera ray and derives the shading
+// normal of its hit as lgb_trace_rays does; the normals meet in shared memory, one thread per pixel sums them in sample order
+// (camera.rs:137-145), counts the hits and stores every requested output.  The anchor sample (camera.rs:143) gives depth and id.
+constexpr uint32_t kGuideThreads = 256;
+constexpr int kGuideStride = kGuideThreads + kGuideThreads / 16;      // per component; index t + t / 16 as in k_shade_lean
+template <bool INST>
+__global__ void __launch_bounds__(kGuideThreads) k_guides(DevScene S, DevCamera C, DevWork W, DevWave V, DevGuides G) {
+    __shared__ double nrm[3 * kGuideStride];
+    __shared__ unsigned char hit[kGuideThreads];
+    const bool passes_of_one = W.spp > kGuideThreads;
+    const uint32_t ppb = passes_of_one ? 1u : fdiv(kGuideThreads, W.fd_spp);          // pixels per block
+    const uint32_t tp = passes_of_one ? 0u : fdiv(threadIdx.x, W.fd_spp);              // this thread's pixel in the block
+    const uint64_t p = (uint64_t)blockIdx.x * ppb + tp;
+    uint32_t x = 0, y = 0;
+    const bool on_film = tp < ppb && p < W.n_pixels && slot_to_pixel(W, p, x, y);
+    // the thread that reduces pixel threadIdx.x of the block
+    const uint64_t rp = (uint64_t)blockIdx.x * ppb + threadIdx.x;
+    uint32_t rx = 0, ry = 0;
+    const bool reducer = threadIdx.x < ppb && rp < W.n_pixels && slot_to_pixel(W, rp, rx, ry);
+    D3 sum = d3(0, 0, 0);
+    uint32_t hits = 0;
+    for (uint32_t s0 = 0; s0 < W.spp; s0 += passes_of_one ? kGuideThreads : W.spp) {
+        const uint32_t s = passes_of_one ? s0 + threadIdx.x : threadIdx.x - tp * W.spp;
+        D3 n = d3(0, 0, 0);
+        bool h = false;
+        if (on_film && s < W.spp) {
+            const uint64_t g = p * W.spp + s;
+            const uint32_t ref = V.hit_ref[g];
+            if (ref != LGB_MISS && ref != kSlotUnused) {
+                Surf sf; double t = V.hit_t[g];
+                world_record<INST>(S, camera_ray(C, W, x, y, s), ref, t, sf);
+                n = shading_normal(sf);
+                h = true;
+            }
+        }
+        const uint32_t at = threadIdx.x + (threadIdx.x >> 4);
+        nrm[at] = n.x; nrm[kGuideStride + at] = n.y; nrm[2 * kGuideStride + at] = n.z;
+        hit[threadIdx.x] = h ? 1 : 0;
+        __syncthreads();
+        if (reducer) {
+            const uint32_t t0 = passes_of_one ? 0u : threadIdx.x * W.spp, cnt = passes_of_one ? min(kGuideThreads, W.spp - s0) : W.spp;
+            for (uint32_t k = t0; k < t0 + cnt; k++) {
+                const uint32_t i = k + (k >> 4);
+                sum = sum + d3(nrm[i], nrm[kGuideStride + i], nrm[2 * kGuideStride + i]);
+                hits += hit[k];
+            }
+        }
+        __syncthreads();
+    }
+    if (!reducer) return;
+    const uint64_t o = W.compact_out ? W.compact_base + rp : (uint64_t)ry * W.w + rx;
+    if (G.normal) {
+        const D3 c = sum * (1.0 / (double)W.spp);
+        G.normal[3 * o] = __double2float_rn(c.x); G.normal[3 * o + 1] = __double2float_rn(c.y); G.normal[3 * o + 2] = __double2float_rn(c.z);
+    }
+    if (G.coverage) G.coverage[o] = __double2float_rn((double)hits / (double)W.spp);
+    if (G.depth || G.prim_id) {
+        const uint64_t ga = rp * W.spp + W.anchor;
+        const uint32_t ref = V.hit_ref[ga];
+        if (G.depth) G.depth[o] = ref == LGB_MISS ? CUDART_INF_F : __double2float_rn(__dmul_rn(V.hit_t[ga], G.view_len));
+        if (G.prim_id) G.prim_id[o] = ref == LGB_MISS ? LGB_MISS : canonical_id(S, ref);
+    }
 }
 
 // ------------------------------------------------------------------ end-of-frame flags of a shared film (multi-GPU, one process per GPU)
@@ -2599,13 +2672,14 @@ bool render_fused(uint32_t spp) { return spp >= 1 && spp <= 256; }      // and !
 // `ev` (optional): kRenderEvents events recorded around the phases: start | primary | setup | anchor shadow rays |
 // pretest + remaining shadow rays | shade | resolve.
 // part 1 = k_primary (every slot, or W.slot_list: the re-trace of tied slots), 2 = everything after it, 3 = both.
+// `guides` (optional, part 2): k_guides first, in the primary phase of `ev`; with O.film == NULL the frame ends there (a geometry pass).
 // `side` (optional): the shadow chains of the lights are independent of each other (own queues, own fetch counters, own occluder
 // table, one bit each in `occl`), so they are dealt round-robin over the launch stream and the side streams: the blocks of one
 // light's persistent kernel fill the SMs that the tail of another's has left idle.
 #define KL(nm, light, st, ...) do { if (klog) klog->begin(nm, light, st); __VA_ARGS__; if (klog) klog->end(st, O.counters); } while (0)
 cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade& sh, const DevWork& W, const DevOut& O,
                           const DevWave& V, bool stats, bool all_shadows, int sms, cudaStream_t stream, cudaEvent_t* ev, int part, const SideStreams* side,
-                          KernelLog* klog, ShadeChunks* chunks, bool linear) {
+                          KernelLog* klog, ShadeChunks* chunks, bool linear, const DevGuides* guides) {
     if (chunks) chunks->launched = 0;
     auto mark = [&](int i) { if (ev) cudaEventRecord(ev[i], stream); };
     const uint64_t total = W.n_pixels * W.spp;
@@ -2642,6 +2716,14 @@ cudaError_t launch_render(const DevScene& S, const DevCamera& C, const DevShade&
     }
     if (!(part & 2)) return cudaSuccess;
     if (total == 0) return cudaSuccess;
+    if (guides) {                       // every slot's final hit is in the wave (the tie re-trace, if any, is done); nothing has overwritten it yet
+        const unsigned gppb = W.spp <= kGuideThreads ? kGuideThreads / W.spp : 1u, gb = (unsigned)((W.n_pixels + gppb - 1) / gppb);
+        KL("k_guides", -1, stream, if (inst) k_guides<true><<<gb, kGuideThreads, 0, stream>>>(S, C, W, V, *guides); else k_guides<false><<<gb, kGuideThreads, 0, stream>>>(S, C, W, V, *guides));
+        if (!O.film) {                  // a geometry pass: no setup, shadow, shade or resolve work
+            for (int k = 1; k <= 6; k++) mark(k);
+            return cudaGetLastError();
+        }
+    }
     mark(1);
     const unsigned blocks = (unsigned)((total + 255) / 256), ablocks = (unsigned)((total + kAppendThreads - 1) / kAppendThreads);
     if (W.setup_in_primary) {           // k_cprimary<SETUP> has written ps / gate / sign byte: straight to the shadow rays

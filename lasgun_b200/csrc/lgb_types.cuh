@@ -270,4 +270,13 @@ struct DevOut {
     uint8_t* film;                   // row-major RGBA8, or the (h, w, 3) f32 linear film of lgb_capture_linear (may be a peer pointer)
 };
 
+// lgb_capture_guides: per-pixel geometry of the camera rays' closest hits (k_guides), row-major; NULL outputs are not written.
+struct DevGuides {
+    float* normal;                   // (h, w, 3): in-order sum of the samples' shading normals times 1/spp
+    float* depth;                    // (h, w): t of the anchor sample times |view|, +inf on a miss
+    uint32_t* prim_id;               // (h, w): canonical id of the anchor sample's hit, or LGB_MISS
+    float* coverage;                 // (h, w): samples that hit / spp
+    double view_len;                 // |view| (host, f64)
+};
+
 }  // namespace lgb

@@ -26,6 +26,11 @@ class Accel:
         """The linear film of this resident scene: a float32 CUDA tensor (h, w, 3), enqueued on torch.cuda.current_stream()."""
         return self.dev.capture_linear(w, h, out=out)
 
+    def capture_guides(self, w: int, h: int, rgb: bool = True, **kw):
+        """Per-pixel normal, depth, prim_id and coverage of this resident scene (and, with rgb, the linear film of the same frame):
+        a dict of CUDA tensors, enqueued on torch.cuda.current_stream() (DeviceScene.capture_guides)."""
+        return self.dev.capture_guides(w, h, rgb=rgb, **kw)
+
     def close(self):
         self.dev.destroy()
 
@@ -51,6 +56,20 @@ def capture_linear(scene: Scene, w: int, h: int, ctx: N.Context | None = None):
     finally:
         root.close()
     return rgb
+
+
+def capture_guides(scene: Scene, w: int, h: int, rgb: bool = True, ctx: N.Context | None = None):
+    """Per-pixel geometry of the camera rays' closest hits -- shading normal summed over the samples times 1/spp, depth along the
+    view axis, primitive id and coverage of every pixel -- and, with rgb, the linear film of `capture_linear` from the same frame:
+    a dict of CUDA tensors, returned once the frame is complete."""
+    import torch
+    root = Accel(scene, ctx, lazy=True)
+    try:
+        out = root.capture_guides(w, h, rgb=rgb)
+        torch.cuda.current_stream(next(iter(out.values())).device).synchronize()
+    finally:
+        root.close()
+    return out
 
 
 def capture_subset(k: int, n: int, root: Accel, film: Film):
