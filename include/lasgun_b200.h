@@ -13,7 +13,8 @@
  *
  * Conventions: every function returns LGB_OK (0) or a negative lgb_status; nothing aborts or
  * unwinds across this boundary.  Host arrays passed in are borrowed for the duration of the
- * call only.  One capture at a time per context.  One context drives one GPU; multi-GPU
+ * call only.  One capture at a time per context (a capture enqueued on another stream than the previous one waits there for
+ * it).  One context drives one GPU; multi-GPU
  * renders use one context per GPU (one process per GPU) and the tile-rank arguments.
  */
 #ifndef LASGUN_B200_H
@@ -25,7 +26,7 @@
 extern "C" {
 #endif
 
-#define LGB_ABI_VERSION 5
+#define LGB_ABI_VERSION 6
 
 typedef enum lgb_status {
     LGB_OK = 0,
@@ -154,7 +155,10 @@ typedef struct lgb_scene_desc {
     lgb_reference_tree_fn reference_tree;                    /* lazy mode (nodes == NULL), else NULL */
     void* reference_tree_user;
     double bounds_lo[3], bounds_hi[3];                       /* lazy mode: world box of all primitives */
+    double view_lo[3], view_hi[3];                           /* with LGB_SCENE_VIEW_BOX: world box of every camera origin lgb_scene_set_camera will
+                                                              * be given (see there); ignored without the flag */
 } lgb_scene_desc;
+#define LGB_SCENE_VIEW_BOX 1u       /* lgb_scene_desc.flags: view_lo / view_hi are valid (finite, lo <= hi) */
 
 #define LGB_MAX_LIGHTS 32
 /* The caller's tree is the REFERENCE tree.  lgb_scene_create uses it (a) to validate the scene and bound
@@ -235,7 +239,8 @@ void lgb_shutdown(lgb_ctx* ctx);
                                      * env LGB_LIGHT_GRIDS presets it. */
 #define LGB_OPT_CAMERA_GRID 6       /* primary rays of a perspective camera through a grid of pixel tiles, each listing the primitives its
                                      * samples can see (csrc/lgb_grid.cu), instead of the BVH / pixel beams.  Same hits.  1 on, 0 off,
-                                     * -1 (default) automatic.  Built at the first capture of a film size and kept with the scene.
+                                     * -1 (default) automatic.  Built at the first capture of a film size and camera (lgb_scene_set_camera)
+                                     * and kept with the scene.
                                      * env LGB_CAMERA_GRID presets it. */
 #define LGB_OPT_WAVE_BUDGET_MB 7    /* memory (MB, default 16384) the per-sample wavefront buffers of one capture may take: a frame that needs more
                                      * is rendered in bands of macro tiles on the same buffers (any frame size in bounded memory).
@@ -252,6 +257,17 @@ const char* lgb_status_string(int status);
 int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* desc, lgb_scene** out);
 void lgb_scene_destroy(lgb_scene* scene);
 uint64_t lgb_scene_device_bytes(const lgb_scene* scene);
+/* A new view of a resident scene: every capture enqueued after this call renders with `camera` (a look_at camera as in
+ * lgb_scene_desc.camera; captures already enqueued keep the camera they were enqueued with).  Host-side, never synchronises; one
+ * capture or set_camera at a time per scene.  The geometry, lights, grids and every decision lgb_scene_create took stay; the
+ * camera grid is rebuilt at the next capture that uses one, in stream order behind the scene's earlier captures.
+ * The f32 error bound of the scene was derived from its world box: the scene, the creation camera's origin and, with
+ * LGB_SCENE_VIEW_BOX, the desc's view box (an orthographic origin widened by 2.5 |image_plane_height| on every axis).  A camera
+ * whose origin, widened the same way, is not inside that box is refused with LGB_ERR_UNSUPPORTED and lgb_last_error names the
+ * box: declare the region an orbit or a fly-through will visit as the view box at creation.  LGB_ERR_INVALID: NULL argument,
+ * supersampling_root outside 1..256, or a component that is not finite.  A refused call leaves the scene's camera unchanged.
+ * On a device group's scene it moves every device's copy; an imported scene checks against the box of its layout. */
+int lgb_scene_set_camera(lgb_ctx* ctx, lgb_scene* scene, const lgb_camera* camera);
 /* Replication across GPUs (one process per GPU): the device scene is ONE relocatable arena plus a small layout
  * record.  The rank that built it exports both; the others receive the arena bytes over NVLink (NCCL broadcast, or
  * a peer copy) into memory they own and import it -- the BVH is built once, not once per GPU.
@@ -350,7 +366,7 @@ int lgb_capture_profile(lgb_ctx* ctx, lgb_scene* scene, uint32_t w, uint32_t h, 
 /* Trace caller-supplied rays (o[3], d[3] f64 each) through the scene: closest-hit id, t and the world-space
  * RayIntersection::ng() / ns() (surface.rs:107-118; any output pointer may be NULL).
  * The f32 error bound of the traversal is derived from the world box of the scene and its camera (the reference root box,
- * through the root transform, united with the camera origin).  The f32 culling ray of an origin outside that box starts where
+ * through the root transform, united with the creation camera's origin and, with LGB_SCENE_VIEW_BOX, the view box).  The f32 culling ray of an origin outside that box starts where
  * the ray enters it (grown by 1/64 of its extent), and a direction with max |d_k| outside [2^-40, 2^40] is traced scaled by
  * an exact power of two; the exact f64 tests give the reference's t either way.  Precondition: every origin lies within one
  * box extent of that box (so no coordinate is NaN or infinite); otherwise the whole batch is refused with LGB_ERR_UNSUPPORTED

@@ -18,10 +18,11 @@ LGB_OK, LGB_ERR_INVALID, LGB_ERR_CUDA, LGB_ERR_UNSUPPORTED, LGB_ERR_NOMEM, LGB_E
 LGB_MISS = 0xFFFFFFFF
 CUDA_STREAM_LEGACY = 0x1                 # cudaStreamLegacy (driver_types.h): the legacy default stream as a stream handle
 LGB_LEAF_FLAG = 0x80000000
+LGB_SCENE_VIEW_BOX = 1
 
 # Every symbol include/lasgun_b200.h declares (checked by tests/test_abi.py without a GPU).
 ABI_SYMBOLS = [
-    "lgb_build_probe", "lgb_device_count", "lgb_init", "lgb_init_devices", "lgb_context_devices", "lgb_set_option", "lgb_shutdown", "lgb_last_error", "lgb_status_string", "lgb_scene_create",
+    "lgb_build_probe", "lgb_device_count", "lgb_init", "lgb_init_devices", "lgb_context_devices", "lgb_set_option", "lgb_shutdown", "lgb_last_error", "lgb_status_string", "lgb_scene_create", "lgb_scene_set_camera",
     "lgb_film_alloc_shared", "lgb_film_open_shared", "lgb_film_release_shared", "lgb_film_signal", "lgb_film_wait", "lgb_scene_destroy", "lgb_scene_layout_bytes", "lgb_scene_export", "lgb_scene_import", "lgb_scene_verify", "lgb_scene_device_bytes", "lgb_scene_build_ms", "lgb_scene_node_count", "lgb_capture", "lgb_capture_subset", "lgb_capture_aov",
     "lgb_capture_device", "lgb_capture_linear", "lgb_capture_guides", "lgb_capture_profile", "lgb_trace_rays", "lgb_debug_fastmath", "lgb_measure_l2_read_gbs", "lgb_measure_fp32_gops", "lgb_measure_fp64_gops",
 ]
@@ -64,6 +65,7 @@ class SceneDesc(C.Structure):
         ("ambient", C.c_double * 3), ("bg_inner", C.c_double * 3), ("bg_outer", C.c_double * 3), ("bg_scale", C.c_double),
         ("recursion", C.c_uint32), ("expected_film_pixels", C.c_uint32),
         ("reference_tree", C.c_void_p), ("reference_tree_user", C.c_void_p), ("bounds_lo", C.c_double * 3), ("bounds_hi", C.c_double * 3),
+        ("view_lo", C.c_double * 3), ("view_hi", C.c_double * 3),
     ]
 
 
@@ -116,6 +118,7 @@ def lib():
         "lgb_build_probe": (C.c_int, [C.POINTER(SceneDesc), C.POINTER(BuildInfo)]),
         "lgb_last_error": (C.c_char_p, [vp]), "lgb_status_string": (C.c_char_p, [C.c_int]),
         "lgb_scene_create": (C.c_int, [vp, C.POINTER(SceneDesc), C.POINTER(vp)]), "lgb_scene_destroy": (None, [vp]),
+        "lgb_scene_set_camera": (C.c_int, [vp, vp, C.POINTER(CameraDesc)]),
         "lgb_film_alloc_shared": (C.c_int, [vp, C.c_uint64, C.POINTER(C.c_void_p), u8p]),
         "lgb_film_open_shared": (C.c_int, [vp, u8p, C.POINTER(C.c_void_p)]),
         "lgb_film_release_shared": (C.c_int, [vp, vp, C.c_int]),
@@ -142,6 +145,7 @@ def lib():
         "lgh_last_error": (C.c_char_p, []), "lgh_scene_new": (vp, []), "lgh_scene_free": (None, [vp]),
         "lgh_set_perspective_camera": (None, [vp, C.c_double]), "lgh_set_orthographic_camera": (None, [vp, C.c_double]),
         "lgh_look_at": (None, [vp, dp, dp, dp]), "lgh_set_supersampling": (C.c_int, [vp, C.c_int]),
+        "lgh_camera_describe": (C.c_int, [C.c_int, C.c_double, dp, dp, dp, C.c_int, C.POINTER(CameraDesc)]),
         "lgh_set_ambient_light": (None, [vp, dp]), "lgh_set_radial_background": (None, [vp, dp, dp, C.c_double]),
         "lgh_set_mesh_smoothing": (None, [vp, C.c_int]), "lgh_add_point_light": (None, [vp, dp, dp, dp]),
         "lgh_add_mesh": (C.c_int, [vp, fp, C.c_uint64, u32p, C.c_uint64, fp, C.c_uint64, u32p, C.POINTER(C.c_int64)]),
@@ -175,6 +179,17 @@ def _d3(v):
 
 def _ptr(a, ty):
     return a.ctypes.data_as(C.POINTER(ty)) if a is not None and a.size else None
+
+
+def camera_desc(cam: api.Camera) -> CameraDesc:
+    """The lgb_camera of an api.Camera, set up as HostScene sets up a scene's camera (constructor, look_at, set_supersampling):
+    bit for bit the camera a scene built with `cam` carries in its desc."""
+    out = CameraDesc()
+    look = [_d3(v) for v in cam.look] if cam.look is not None else [None, None, None]
+    rc = lib().lgh_camera_describe(1 if cam.perspective else 0, cam.param, *look, cam.supersampling, C.byref(out))
+    if rc != LGB_OK:
+        raise LasgunError(rc, lib().lgh_last_error().decode())
+    return out
 
 
 class HostScene:
@@ -258,18 +273,27 @@ class HostScene:
 class FlatScene:
     """Host-side flattened scene (Accel::from without the upload): owns the arrays of an lgb_scene_desc."""
 
-    def __init__(self, scene, keep_levels=False, lazy=False):
+    def __init__(self, scene, keep_levels=False, lazy=False, view_box=None):
         """lazy=True: the reference BVH is not built now; the device asks for it (reference_tree callback) only if a
-        closest-hit ray meets two primitives at bit-identical t.  Accessors that need the tree build it."""
+        closest-hit ray meets two primitives at bit-identical t.  Accessors that need the tree build it.
+        view_box=(lo, hi): world box of every camera origin DeviceScene.set_camera will be given (LGB_SCENE_VIEW_BOX); the scene's
+        f32 error bound then covers it.  None: the scene and its own camera only."""
         L = lib()
         self.host = scene if isinstance(scene, HostScene) else HostScene(scene)
         self.h = L.lgh_flatten(self.host.h, 1 if keep_levels else 0, 1 if lazy else 0)
         if not self.h:
             msg = L.lgh_last_error().decode()
             raise LasgunError(LGB_ERR_UNSUPPORTED if "not on the device path" in msg or "outside the device" in msg else LGB_ERR_INVALID, msg)
+        self.view_box = None if view_box is None else (_d3(view_box[0]), _d3(view_box[1]))
         self.desc = SceneDesc()
-        L.lgh_flat_describe(self.h, C.byref(self.desc))
+        self._describe()
         self.spp = self.desc.camera.supersampling_root ** 2
+
+    def _describe(self):
+        lib().lgh_flat_describe(self.h, C.byref(self.desc))
+        if self.view_box is not None:
+            self.desc.flags |= LGB_SCENE_VIEW_BOX
+            self.desc.view_lo, self.desc.view_hi = self.view_box
 
     @property
     def tree_built(self):
@@ -280,7 +304,7 @@ class FlatScene:
         L = lib()
         if L.lgh_flat_build_tree(self.h):
             raise LasgunError(LGB_ERR_INVALID, L.lgh_last_error().decode())
-        L.lgh_flat_describe(self.h, C.byref(self.desc))
+        self._describe()
         self.n_lights = self.desc.n_lights
 
     @property
@@ -432,6 +456,15 @@ class DeviceScene:
         ctx.check(L.lgb_scene_create(ctx.h, C.byref(flat.desc), C.byref(h)))
         self.h = h
         self.spp = flat.spp
+
+    def set_camera(self, camera):
+        """lgb_scene_set_camera: captures enqueued from now on render with `camera` (an api.Camera or a CameraDesc); captures already
+        enqueued keep theirs.  A camera whose origin leaves the scene's world box (the scene, its creation camera and the view box of
+        its FlatScene) raises LasgunError with LGB_ERR_UNSUPPORTED, and the scene keeps its camera.  Returns self."""
+        desc = camera if isinstance(camera, CameraDesc) else camera_desc(camera)
+        self.ctx.check(lib().lgb_scene_set_camera(self.ctx.h, self.h, C.byref(desc)))
+        self.spp = desc.supersampling_root ** 2
+        return self
 
     def verify(self):
         """Structural check of the resident device BVH (lgb_scene_verify)."""

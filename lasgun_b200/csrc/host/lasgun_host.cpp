@@ -655,6 +655,16 @@ struct Emitter {
 
 }  // namespace
 
+// lasgun::Camera -> lgb_camera: what lgb_scene_desc.camera and lgb_scene_set_camera take
+static lgb_camera to_lgb_camera(const Camera& c) {
+    lgb_camera o{};
+    std::memcpy(o.origin, c.origin, 24); std::memcpy(o.view, c.view, 24);
+    std::memcpy(o.up, c.up, 24); std::memcpy(o.aux, c.aux, 24);
+    o.image_plane_height = c.image_plane_height; o.pixel_separation = c.pixel_separation;
+    o.sample_distance = c.distance; o.supersampling_root = (uint32_t)c.root;
+    return o;
+}
+
 FlatScene flatten(const Scene& scene, const BuildOptions& opt) {
     auto t0 = std::chrono::steady_clock::now();
     FlatScene out;
@@ -683,11 +693,7 @@ FlatScene flatten(const Scene& scene, const BuildOptions& opt) {
         lgb_light q; std::memcpy(q.position, l.position, 24); std::memcpy(q.intensity, l.intensity, 24); std::memcpy(q.falloff, l.falloff, 24);
         out.lights.push_back(q);
     }
-    const Camera& c = scene.camera;
-    std::memcpy(out.camera.origin, c.origin, 24); std::memcpy(out.camera.view, c.view, 24);
-    std::memcpy(out.camera.up, c.up, 24); std::memcpy(out.camera.aux, c.aux, 24);
-    out.camera.image_plane_height = c.image_plane_height; out.camera.pixel_separation = c.pixel_separation;
-    out.camera.sample_distance = c.distance; out.camera.supersampling_root = (uint32_t)c.root;
+    out.camera = to_lgb_camera(scene.camera);
     std::memcpy(out.ambient, scene.ambient, 24); std::memcpy(out.bg_inner, scene.bg_inner, 24); std::memcpy(out.bg_outer, scene.bg_outer, 24);
     out.bg_scale = scene.bg_scale; out.recursion = scene.recursion;
     out.build_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -817,6 +823,16 @@ void lgh_set_perspective_camera(void* s, double fov) { ((HostScene*)s)->scene.se
 void lgh_set_orthographic_camera(void* s, double h) { ((HostScene*)s)->scene.set_orthographic_camera(h); }
 void lgh_look_at(void* s, const double* o, const double* l, const double* u) { ((HostScene*)s)->scene.camera.look_at(o, l, u); }
 int lgh_set_supersampling(void* s, int base) { return guarded([&] { ((HostScene*)s)->scene.camera.set_supersampling((uint8_t)base); }); }
+// The lgb_camera of a camera set up as a scene's: the perspective or orthographic constructor, look_at if origin, look and up are
+// given, then set_supersampling -- the reference's arithmetic, so a camera moved to later equals a scene built with it, bit for bit.
+int lgh_camera_describe(int perspective, double param, const double* origin, const double* look, const double* up, int supersampling, lgb_camera* out) {
+    return guarded([&] {
+        Camera c = perspective ? Camera::perspective(param) : Camera::orthographic(param);
+        if (origin && look && up) c.look_at(origin, look, up);
+        c.set_supersampling((uint8_t)supersampling);
+        *out = to_lgb_camera(c);
+    });
+}
 void lgh_set_ambient_light(void* s, const double* c) { ((HostScene*)s)->scene.set_ambient_light(c); }
 void lgh_set_radial_background(void* s, const double* in, const double* out, double scale) { ((HostScene*)s)->scene.set_radial_background(in, out, scale); }
 void lgh_set_max_recursion_depth(void* s, uint32_t depth) { ((HostScene*)s)->scene.set_max_recursion_depth(depth); }

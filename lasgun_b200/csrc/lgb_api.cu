@@ -65,6 +65,8 @@ struct lgb_ctx {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr;
     cudaEvent_t phase[kRenderEvents] = {};
+    // recorded behind every capture: the next one, on whatever stream, waits for it before it touches the context's buffers
+    cudaEvent_t last_capture = nullptr;
     std::string error;
     DevBuf aov_li, beam2;
     DevBuf radiance, film, counters, tiles, aov_id, aov_t, aov_occl, scratch, wave, wave_ctr, ties, beam;
@@ -130,8 +132,9 @@ struct lgb_scene {
     void* rank_buf = nullptr;                        // rank tables uploaded later live outside the arena
     uint64_t tie_retraces = 0;
     uint64_t bytes = 0;
-    // camera grid (lgb_grid.cu) of the film size it was last built for; rebuilt when the film changes
-    struct CamGrid { uint32_t w = 0, h = 0, shift = 0, nx = 0, n_large = 0; bool valid = false, refused = false; void* starts = nullptr; void* entries = nullptr; void* large = nullptr; uint64_t bytes = 0; double build_ms = 0; } camgrid;
+    // camera grid (lgb_grid.cu) of the film size and camera (cam_gen) it was last built for; rebuilt when either changes
+    struct CamGrid { uint32_t w = 0, h = 0, shift = 0, nx = 0, n_large = 0; uint64_t gen = 0; bool valid = false, refused = false; void* starts = nullptr; void* entries = nullptr; void* large = nullptr; uint64_t bytes = 0; double build_ms = 0; } camgrid;
+    uint64_t cam_gen = 0;              // incremented by every lgb_scene_set_camera
     CamGrid& cam_grid() { return camgrid; }
     std::vector<void*> grid_allocs;    // light grids (lgb_grid.cu): table + per-light cell starts / entries / large lists, outside the arena
     struct GridHost { void* starts; void* entries; void* large; size_t starts_bytes, entries_bytes, large_bytes; uint32_t res, n_large; };
@@ -151,8 +154,9 @@ struct lgb_scene {
     DevCamera cam{};
     DevShade shade{};
     double max_abs = 0.0;      // max |coordinate| over geometry, camera origin and lights
-    // world box (scene and camera) the f32 error bound of every space was derived from: the traversal is conservative for rays
-    // whose f32 origin lies inside it, so lgb_trace_rays starts the f32 ray of a caller-supplied origin outside where it enters it
+    // world box (scene, creation camera, declared view box) the f32 error bound of every space was derived from: the traversal is
+    // conservative for rays whose f32 origin lies inside it, so lgb_trace_rays starts the f32 ray of a caller-supplied origin outside
+    // where it enters it, and lgb_scene_set_camera refuses a camera whose origins leave it
     double origin_lo[3] = {0, 0, 0}, origin_hi[3] = {0, 0, 0};
     double build_ms = 0.0;     // host time of the device-BVH build inside lgb_scene_create
     double t_validate = 0, t_rank = 0, t_build = 0, t_convert_upload = 0, t_total = 0;   // ms, lgb_scene_create phases
@@ -167,6 +171,22 @@ static int cuda_fail(lgb_ctx* ctx, cudaError_t e, const char* what) {
     return fail(ctx, LGB_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
 #define CU(ctx, call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return cuda_fail(ctx, e__, #call); } while (0)
+
+// The checks lgb_scene_create and lgb_scene_set_camera both apply to a camera; NULL if it passes.
+static const char* camera_problem(const lgb_camera& c) {
+    if (c.supersampling_root == 0 || c.supersampling_root > 256) return "supersampling_root out of range";
+    return nullptr;
+}
+// orthographic origins move across the image plane (camera.rs:126-128) by at most this much on every axis, for aspect <= 4 (checked
+// per capture); 0 for a perspective camera
+static double origin_slack(const lgb_camera& c) { return 2.5 * std::fabs(c.image_plane_height) * std::fabs(c.pixel_separation); }
+static DevCamera dev_camera(const lgb_camera& c) {
+    DevCamera d{};
+    for (int k = 0; k < 3; k++) { d.origin[k] = c.origin[k]; d.view[k] = c.view[k]; d.up[k] = c.up[k]; d.aux[k] = c.aux[k]; }
+    d.image_plane_height = c.image_plane_height; d.pixel_separation = c.pixel_separation; d.sample_distance = c.sample_distance;
+    d.root = c.supersampling_root;
+    return d;
+}
 
 extern "C" {
 
@@ -365,6 +385,7 @@ void lgb_shutdown(lgb_ctx* c) {
     for (cudaEvent_t e : c->chunk_ev) cudaEventDestroy(e);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); cudaEventDestroy(c->ev2);
+    if (c->last_capture) cudaEventDestroy(c->last_capture);
     for (auto& e : c->phase) cudaEventDestroy(e);
     for (int k = 0; k < c->side.n; k++) { cudaStreamDestroy(c->side.s[k]); cudaEventDestroy(c->side.join[k]); }
     cudaEventDestroy(c->side.fork);
@@ -890,7 +911,10 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
         return fail(ctx, LGB_ERR_INVALID, "lgb_scene_create: array too large for 30-bit primitive references");
     if (d->n_lights > LGB_MAX_LIGHTS) return fail(ctx, LGB_ERR_UNSUPPORTED, "lgb_scene_create: more than LGB_MAX_LIGHTS point lights");
     if (d->n_materials == 0 && (d->n_spheres || d->n_cuboids || d->n_triangles)) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_create: no materials");
-    if (d->camera.supersampling_root == 0 || d->camera.supersampling_root > 256) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_create: supersampling_root out of range");
+    if (const char* p = camera_problem(d->camera)) return fail(ctx, LGB_ERR_INVALID, std::string("lgb_scene_create: ") + p);
+    if (d->flags & LGB_SCENE_VIEW_BOX)
+        for (int k = 0; k < 3; k++)
+            if (!(std::isfinite(d->view_lo[k]) && std::isfinite(d->view_hi[k]) && d->view_lo[k] <= d->view_hi[k])) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_create: bad view box");
     CU(ctx, cudaSetDevice(ctx->device));
 
     auto tc0 = std::chrono::steady_clock::now();
@@ -967,11 +991,13 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
                 wlo[r] = l; whi[r] = h;
             }
         } else for (int k = 0; k < 3; k++) { wlo[k] = rlo[k]; whi[k] = rhi[k]; }
-        // orthographic origins move across the image plane (camera.rs:126-128); aspect <= 4 assumed, checked per capture
-        const double slack = 2.5 * std::fabs(d->camera.image_plane_height) * std::fabs(d->camera.pixel_separation);
+        const double slack = origin_slack(d->camera);
         for (int k = 0; k < 3; k++) {
             if (std::isfinite(d->camera.origin[k])) { wlo[k] = std::min(wlo[k], d->camera.origin[k] - slack); whi[k] = std::max(whi[k], d->camera.origin[k] + slack); }
         }
+        // the region the caller's later cameras will visit (lgb_scene_set_camera accepts origins inside this box only)
+        if (d->flags & LGB_SCENE_VIEW_BOX)
+            for (int k = 0; k < 3; k++) { wlo[k] = std::min(wlo[k], d->view_lo[k]); whi[k] = std::max(whi[k], d->view_hi[k]); }
         for (int k = 0; k < 3; k++) { s->origin_lo[k] = wlo[k]; s->origin_hi[k] = whi[k]; }
     }
 
@@ -1267,14 +1293,8 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
     }
     s->t_convert_upload = ms_since(tc3);
     }
-    for (int k = 0; k < 3; k++) {
-        s->cam.origin[k] = d->camera.origin[k]; s->cam.view[k] = d->camera.view[k]; s->cam.up[k] = d->camera.up[k]; s->cam.aux[k] = d->camera.aux[k];
-        s->shade.ambient[k] = d->ambient[k]; s->shade.bg_inner[k] = d->bg_inner[k]; s->shade.bg_outer[k] = d->bg_outer[k];
-    }
-    s->cam.image_plane_height = d->camera.image_plane_height;
-    s->cam.pixel_separation = d->camera.pixel_separation;
-    s->cam.sample_distance = d->camera.sample_distance;
-    s->cam.root = d->camera.supersampling_root;
+    s->cam = dev_camera(d->camera);
+    for (int k = 0; k < 3; k++) { s->shade.ambient[k] = d->ambient[k]; s->shade.bg_inner[k] = d->bg_inner[k]; s->shade.bg_outer[k] = d->bg_outer[k]; }
     s->shade.bg_scale = d->bg_scale;
     cudaError_t e = cudaStreamSynchronize(ctx->stream);     // the staging buffer is free for the next scene
     if (e != cudaSuccess) { cuda_fail(ctx, e, "scene upload"); return bail(LGB_ERR_CUDA); }
@@ -1284,6 +1304,33 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
     if (ctx->peers.empty()) { if (int rc = build_light_grids(ctx, s)) return bail(rc); }
     else if (int rc = replicate_to_peers(ctx, s)) return bail(rc);       // (builds the leader's grids too, while the peers copy)
     *out = s;
+    return LGB_OK;
+}
+
+// Captures take the camera by value (DevWork constants, beams, tile lists, kernel arguments) when they are enqueued; the one piece
+// of per-view state kept with the scene is the camera grid, keyed on cam_gen and rebuilt in stream order (ensure_camgrid).
+int lgb_scene_set_camera(lgb_ctx* ctx, lgb_scene* s, const lgb_camera* cam) {
+    if (!ctx || !s || !cam) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_camera: NULL argument");
+    if (s->ctx != ctx) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_camera: scene does not belong to this context");
+    if (const char* p = camera_problem(*cam)) return fail(ctx, LGB_ERR_INVALID, std::string("lgb_scene_set_camera: ") + p);
+    const double comps[] = {cam->origin[0], cam->origin[1], cam->origin[2], cam->view[0], cam->view[1], cam->view[2], cam->up[0], cam->up[1], cam->up[2],
+                            cam->aux[0], cam->aux[1], cam->aux[2], cam->image_plane_height, cam->pixel_separation, cam->sample_distance};
+    for (double v : comps) if (!std::isfinite(v)) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_camera: a camera component is not finite");
+    // the f32 error bound of every space, the padding of the device BVH and of both grid kinds were derived from origin_lo/hi: the
+    // conservativeness argument (DESIGN §4, items 1-2) holds for ray origins inside that box only
+    const double slack = origin_slack(*cam);
+    for (int k = 0; k < 3; k++) {
+        if (cam->origin[k] - slack >= s->origin_lo[k] && cam->origin[k] + slack <= s->origin_hi[k]) continue;
+        char msg[768];
+        std::snprintf(msg, sizeof msg, "lgb_scene_set_camera: the camera origin (%.17g, %.17g, %.17g), widened by %.17g (the reach of an orthographic camera's origins), is not inside the box "
+                      "[%.17g, %.17g] x [%.17g, %.17g] x [%.17g, %.17g] of the scene, its creation camera and its view box, from which its f32 error bound "
+                      "was derived (declare the region with LGB_SCENE_VIEW_BOX at lgb_scene_create)", cam->origin[0], cam->origin[1], cam->origin[2], slack,
+                      s->origin_lo[0], s->origin_hi[0], s->origin_lo[1], s->origin_hi[1], s->origin_lo[2], s->origin_hi[2]);
+        return fail(ctx, LGB_ERR_UNSUPPORTED, msg);
+    }
+    const DevCamera d = dev_camera(*cam);
+    s->cam = d; s->cam_gen++;
+    for (lgb_scene* r : s->replicas) { r->cam = d; r->cam_gen++; }     // device group: every peer rebuilds its own camera grid
     return LGB_OK;
 }
 
@@ -1309,11 +1356,14 @@ static int ensure_camgrid(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, uint
     const bool want = c->camera_grid == 1 || (c->camera_grid < 0 && large_scene(S) && samples >= 4ull * prims);
     if (!want || S.instanced || s->cam.pixel_separation != 0.0 || prims == 0) return LGB_OK;
     lgb_scene::CamGrid& G = s->cam_grid();
-    if (G.refused && G.w == w && G.h == h) return LGB_OK;
-    if (!(G.valid && G.w == w && G.h == h)) {
+    const bool same_key = G.w == w && G.h == h && G.gen == s->cam_gen;
+    if (G.refused && same_key) return LGB_OK;
+    if (!(G.valid && same_key)) {
         auto t0 = std::chrono::steady_clock::now();
+        // a capture of the previous film size or view may still read the old grid on another stream
+        if (s->last_use) CU(c, cudaStreamWaitEvent(st, s->last_use, 0));
         for (void** q : {&G.starts, &G.entries, &G.large}) if (*q) { cudaFreeAsync(*q, st); *q = nullptr; }
-        G.valid = false; G.refused = false; G.w = w; G.h = h;
+        G.valid = false; G.refused = false; G.w = w; G.h = h; G.gen = s->cam_gen;
         CamGridParams P{};
         const DevCamera& cam = s->cam;
         // (a w, b w, w) = [aux | up | view]^-1 (X - origin)
@@ -1488,6 +1538,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
     if (a.w == 0 || a.h == 0 || (uint64_t)a.w * a.h >= (1ull << 32)) return fail(c, LGB_ERR_INVALID, "capture: bad film size");
     CU(c, cudaSetDevice(c->device));
     cudaStream_t st = a.stream ? a.stream : c->stream;
+    if (c->last_capture) CU(c, cudaStreamWaitEvent(st, c->last_capture, 0));    // one capture at a time per context, in stream order
     DevWork W{};
     W.mode = a.mode; W.w = a.w; W.h = a.h;
     W.winv = 1.0 / (double)a.w; W.hinv = 1.0 / (double)a.h; W.aspect = (double)a.w / (double)a.h;   // film.rs:36-45
@@ -1675,6 +1726,8 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
     CU(c, cudaEventRecord(c->ev1, st));
     if (!s->last_use) CU(c, cudaEventCreateWithFlags(&s->last_use, cudaEventDisableTiming));
     CU(c, cudaEventRecord(s->last_use, st));
+    if (!c->last_capture) CU(c, cudaEventCreateWithFlags(&c->last_capture, cudaEventDisableTiming));
+    CU(c, cudaEventRecord(c->last_capture, st));
     uint32_t copy_rows[9] = {0};                 // film rows [copy_rows[k], copy_rows[k + 1]) leave behind slice k
     bool copy_bounce = false;
     if (chunks && chunks->launched) {

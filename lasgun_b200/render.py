@@ -12,15 +12,22 @@ from .api import Film, Scene
 class Accel:
     """`Accel::from(&scene)` (lib.rs:42, bvh.rs:135): the scene's BVH, flattened and resident on the GPU."""
 
-    def __init__(self, scene: Scene, ctx: N.Context | None = None, lazy: bool = False):
+    def __init__(self, scene: Scene, ctx: N.Context | None = None, lazy: bool = False, view_box=None):
+        """view_box=(lo, hi): the world box every camera origin set_camera will be given lies in (an orbit, a fly-through)."""
         self.scene = scene
         self.ctx = ctx or N.default_context()
-        self.flat = N.FlatScene(scene, lazy=lazy)
+        self.flat = N.FlatScene(scene, lazy=lazy, view_box=view_box)
         self.dev = N.DeviceScene(self.ctx, self.flat)
 
     @staticmethod
     def from_scene(scene: Scene, **kw):
         return Accel(scene, **kw)
+
+    def set_camera(self, camera):
+        """A new view of this resident scene (api.Camera): captures from now on render it, without rebuilding anything but the camera
+        grid.  Its origin must lie in the box of the scene, the first camera and view_box.  Returns self."""
+        self.dev.set_camera(camera)
+        return self
 
     def capture_linear(self, w: int, h: int, out=None):
         """The linear film of this resident scene: a float32 CUDA tensor (h, w, 3), enqueued on torch.cuda.current_stream()."""
