@@ -235,7 +235,8 @@ void lgb_shutdown(lgb_ctx* ctx);
                                      * env LGB_BEAMS presets it. */
 #define LGB_OPT_LIGHT_GRIDS 5       /* shadow rays through per-light cube-map grids of primitive lists instead of the BVH (csrc/lgb_grid.cu;
                                      * scenes without transformed aggregates).  Same occlusion bits.  1 on, 0 off, -1 (default)
-                                     * automatic: device BVH of >= 1024 nodes and at most 8 lights.  Read at lgb_scene_create.
+                                     * automatic: device BVH of >= 1024 nodes and at most 8 lights.  Read at lgb_scene_create (and when
+                                     * lgb_scene_set_lights moves a light).
                                      * env LGB_LIGHT_GRIDS presets it. */
 #define LGB_OPT_CAMERA_GRID 6       /* primary rays of a perspective camera through a grid of pixel tiles, each listing the primitives its
                                      * samples can see (csrc/lgb_grid.cu), instead of the BVH / pixel beams.  Same hits.  1 on, 0 off,
@@ -259,7 +260,7 @@ void lgb_scene_destroy(lgb_scene* scene);
 uint64_t lgb_scene_device_bytes(const lgb_scene* scene);
 /* A new view of a resident scene: every capture enqueued after this call renders with `camera` (a look_at camera as in
  * lgb_scene_desc.camera; captures already enqueued keep the camera they were enqueued with).  Host-side, never synchronises; one
- * capture or set_camera at a time per scene.  The geometry, lights, grids and every decision lgb_scene_create took stay; the
+ * capture or set_* call at a time per scene.  The geometry, lights, grids and every decision lgb_scene_create took stay; the
  * camera grid is rebuilt at the next capture that uses one, in stream order behind the scene's earlier captures.
  * The f32 error bound of the scene was derived from its world box: the scene, the creation camera's origin and, with
  * LGB_SCENE_VIEW_BOX, the desc's view box (an orthographic origin widened by 2.5 |image_plane_height| on every axis).  A camera
@@ -268,6 +269,21 @@ uint64_t lgb_scene_device_bytes(const lgb_scene* scene);
  * supersampling_root outside 1..256, or a component that is not finite.  A refused call leaves the scene's camera unchanged.
  * On a device group's scene it moves every device's copy; an imported scene checks against the box of its layout. */
 int lgb_scene_set_camera(lgb_ctx* ctx, lgb_scene* scene, const lgb_camera* camera);
+/* Relighting a resident scene: every capture enqueued after this call renders with these `n_lights` point lights (0 ...
+ * LGB_MAX_LIGHTS, any count, not only the creation count) and this ambient term (lgb_scene_desc.ambient); captures already enqueued
+ * keep what they were enqueued with.  Host-side, never synchronises; one capture or set_* call at a time per scene.  The geometry,
+ * camera and every other decision lgb_scene_create took stay.  The records go into the scene's light slot, and if a light moved or
+ * the count changed the light grids are rebuilt (or dropped: the same rule as at creation, e.g. more than 8 lights), both at the
+ * next capture (or lgb_scene_export), in stream order behind the scene's earlier captures; a new intensity, falloff or ambient term
+ * rebuilds nothing.  The frames are those of a scene created with these lights.
+ * The shadow beams' f32 cull starts at the light, so a light position must satisfy |position[k]| <= 4 M on every axis, M being the
+ * largest |coordinate| of the world box the f32 error bound was derived from (see lgb_scene_set_camera); a light beyond it is
+ * refused with LGB_ERR_UNSUPPORTED and lgb_last_error names the box: a view box (LGB_SCENE_VIEW_BOX) holding the lights enlarges it.
+ * LGB_ERR_UNSUPPORTED also for n_lights > LGB_MAX_LIGHTS.  LGB_ERR_INVALID: NULL ctx, scene or ambient, lights == NULL with
+ * n_lights > 0, a scene of another context, or a component that is not finite.  A refused call leaves the scene unchanged.
+ * On a device group's scene every device follows.  An imported scene accepts it too: the call writes the light slot of the
+ * borrowed arena and rebuilds the importer's own grids. */
+int lgb_scene_set_lights(lgb_ctx* ctx, lgb_scene* scene, const lgb_light* lights, uint64_t n_lights, const double ambient[3]);
 /* Replication across GPUs (one process per GPU): the device scene is ONE relocatable arena plus a small layout
  * record.  The rank that built it exports both; the others receive the arena bytes over NVLink (NCCL broadcast, or
  * a peer copy) into memory they own and import it -- the BVH is built once, not once per GPU.

@@ -22,7 +22,7 @@ LGB_SCENE_VIEW_BOX = 1
 
 # Every symbol include/lasgun_b200.h declares (checked by tests/test_abi.py without a GPU).
 ABI_SYMBOLS = [
-    "lgb_build_probe", "lgb_device_count", "lgb_init", "lgb_init_devices", "lgb_context_devices", "lgb_set_option", "lgb_shutdown", "lgb_last_error", "lgb_status_string", "lgb_scene_create", "lgb_scene_set_camera",
+    "lgb_build_probe", "lgb_device_count", "lgb_init", "lgb_init_devices", "lgb_context_devices", "lgb_set_option", "lgb_shutdown", "lgb_last_error", "lgb_status_string", "lgb_scene_create", "lgb_scene_set_camera", "lgb_scene_set_lights",
     "lgb_film_alloc_shared", "lgb_film_open_shared", "lgb_film_release_shared", "lgb_film_signal", "lgb_film_wait", "lgb_scene_destroy", "lgb_scene_layout_bytes", "lgb_scene_export", "lgb_scene_import", "lgb_scene_verify", "lgb_scene_device_bytes", "lgb_scene_build_ms", "lgb_scene_node_count", "lgb_capture", "lgb_capture_subset", "lgb_capture_aov",
     "lgb_capture_device", "lgb_capture_linear", "lgb_capture_guides", "lgb_capture_profile", "lgb_trace_rays", "lgb_debug_fastmath", "lgb_measure_l2_read_gbs", "lgb_measure_fp32_gops", "lgb_measure_fp64_gops",
 ]
@@ -42,6 +42,11 @@ class CameraDesc(C.Structure):
     _fields_ = [("origin", C.c_double * 3), ("view", C.c_double * 3), ("up", C.c_double * 3), ("aux", C.c_double * 3),
                 ("image_plane_height", C.c_double), ("pixel_separation", C.c_double), ("sample_distance", C.c_double),
                 ("supersampling_root", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class LightDesc(C.Structure):
+    """lgb_light (PointLight, src/light/point.rs:14-18)."""
+    _fields_ = [("position", C.c_double * 3), ("intensity", C.c_double * 3), ("falloff", C.c_double * 3)]
 
 
 class InstanceDesc(C.Structure):
@@ -119,6 +124,7 @@ def lib():
         "lgb_last_error": (C.c_char_p, [vp]), "lgb_status_string": (C.c_char_p, [C.c_int]),
         "lgb_scene_create": (C.c_int, [vp, C.POINTER(SceneDesc), C.POINTER(vp)]), "lgb_scene_destroy": (None, [vp]),
         "lgb_scene_set_camera": (C.c_int, [vp, vp, C.POINTER(CameraDesc)]),
+        "lgb_scene_set_lights": (C.c_int, [vp, vp, C.POINTER(LightDesc), C.c_uint64, dp]),
         "lgb_film_alloc_shared": (C.c_int, [vp, C.c_uint64, C.POINTER(C.c_void_p), u8p]),
         "lgb_film_open_shared": (C.c_int, [vp, u8p, C.POINTER(C.c_void_p)]),
         "lgb_film_release_shared": (C.c_int, [vp, vp, C.c_int]),
@@ -190,6 +196,13 @@ def camera_desc(cam: api.Camera) -> CameraDesc:
     if rc != LGB_OK:
         raise LasgunError(rc, lib().lgh_last_error().decode())
     return out
+
+
+def light_descs(lights):
+    """The lgb_light records of (position, intensity, falloff) triples, as api.Scene.lights holds them: the array FlatScene puts in
+    the desc for a scene with these lights."""
+    lights = [tuple(api._v3(v) for v in l) for l in lights]
+    return (LightDesc * len(lights))(*[LightDesc(*(_d3(v) for v in l)) for l in lights])
 
 
 class HostScene:
@@ -464,6 +477,15 @@ class DeviceScene:
         desc = camera if isinstance(camera, CameraDesc) else camera_desc(camera)
         self.ctx.check(lib().lgb_scene_set_camera(self.ctx.h, self.h, C.byref(desc)))
         self.spp = desc.supersampling_root ** 2
+        return self
+
+    def set_lights(self, lights, ambient):
+        """lgb_scene_set_lights: captures enqueued from now on render with `lights` ((position, intensity, falloff) triples, as
+        api.Scene.lights; 0 to LGB_MAX_LIGHTS of them) and the ambient term `ambient`; captures already enqueued keep theirs.  A light
+        with a coordinate beyond 4 M (M: the largest coordinate of the scene's world box) raises LasgunError with LGB_ERR_UNSUPPORTED,
+        and the scene keeps its lights.  Returns self."""
+        recs = light_descs(lights)
+        self.ctx.check(lib().lgb_scene_set_lights(self.ctx.h, self.h, recs, len(recs), _d3(ambient)))
         return self
 
     def verify(self):

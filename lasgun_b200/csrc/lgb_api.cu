@@ -150,10 +150,15 @@ struct lgb_scene {
     uint64_t grid_bytes = 0;
     std::vector<lgb_scene*> replicas;  // device group: the same scene on every peer, in peer order (arena copied over NVLink, not rebuilt)
     cudaEvent_t last_use = nullptr;   // recorded behind every capture on the stream it ran on: lgb_scene_destroy frees the arena behind it
+    // point lights (9 doubles each: position, intensity, falloff, the layout of the arena's light slot): light_rec holds the ones in
+    // effect for the next capture (lgb_scene_set_lights), light_dev the ones in the slot and in the grids; apply_lights moves
+    // light_dev up to light_rec in stream order when light_gen has moved past light_applied
+    std::vector<double> light_rec, light_dev;
+    uint64_t light_gen = 0, light_applied = 0;
     DevScene dev{};
     DevCamera cam{};
     DevShade shade{};
-    double max_abs = 0.0;      // max |coordinate| over geometry, camera origin and lights
+    double max_abs = 0.0;      // max |coordinate| of the geometry and the world box below (not of the lights: lgb_scene_set_lights)
     // world box (scene, creation camera, declared view box) the f32 error bound of every space was derived from: the traversal is
     // conservative for rays whose f32 origin lies inside it, so lgb_trace_rays starts the f32 ray of a caller-supplied origin outside
     // where it enters it, and lgb_scene_set_camera refuses a camera whose origins leave it
@@ -187,6 +192,16 @@ static DevCamera dev_camera(const lgb_camera& c) {
     d.root = c.supersampling_root;
     return d;
 }
+// lgb_light -> the arena's light record (lgb_types.cuh: 9 doubles)
+static std::vector<double> light_records(const lgb_light* lights, uint64_t n) {
+    std::vector<double> r(9 * n);
+    for (uint64_t i = 0; i < n; i++)
+        for (int k = 0; k < 3; k++) { r[9 * i + k] = lights[i].position[k]; r[9 * i + 3 + k] = lights[i].intensity[k]; r[9 * i + 6 + k] = lights[i].falloff[k]; }
+    return r;
+}
+// How far from the origin, in units of M (the largest |coordinate| of the world box), a light may lie on any axis: k_sbeam's f32
+// culling ray starts at the light, and its cull is conservative up to about 7.5 M (DESIGN §4, "Lights")
+constexpr double kLightReach = 4.0;
 
 extern "C" {
 
@@ -485,10 +500,11 @@ static int ensure_rank_tables(lgb_ctx* ctx, lgb_scene* s) {
 }
 
 extern "C" { static int ensure_bvh(lgb_ctx* ctx, lgb_scene* s); }      // (defined inside the extern "C" block below)
+extern "C" { static int apply_lights(lgb_ctx* c, lgb_scene* s, cudaStream_t st); }
 // ---- export / import: the arena is position independent once DevScene's pointers are written as offsets
 namespace {
 struct SceneLayout { uint64_t magic, arena_bytes; DevScene dev; DevCamera cam; DevShade shade; double max_abs; double origin_lo[3], origin_hi[3]; };
-constexpr uint64_t kLayoutMagic = 0x4C47423253434E34ull;       // "LGB2SCN4"
+constexpr uint64_t kLayoutMagic = 0x4C47423253434E35ull;       // "LGB2SCN5": the light slot holds LGB_MAX_LIGHTS records
 constexpr uint64_t kNullOffset = ~0ull;
 template <class F> void for_each_pointer(DevScene& d, F f) {
     f((const void*&)d.nodes); f((const void*&)d.sph32); f((const void*&)d.sph64); f((const void*&)d.sph_mat); f((const void*&)d.sph_id);
@@ -653,6 +669,10 @@ int lgb_scene_export(const lgb_scene* s, void* layout_out, uint64_t layout_bytes
     if (!s || !layout_out || layout_bytes < sizeof(SceneLayout) || !arena_dev || !arena_bytes) return LGB_ERR_INVALID;
     if (s->lazy_fn) return LGB_ERR_UNSUPPORTED;       // a lazy scene's rank tables live outside the arena: create it with the tree to replicate it
     if (int rc = ensure_bvh(s->ctx, const_cast<lgb_scene*>(s))) return rc;          // (an importer cannot build the tree: it has no item boxes)
+    if (s->light_applied != s->light_gen) {            // the arena carries the lights in effect, and the caller reads it on its own streams
+        if (int rc = apply_lights(s->ctx, const_cast<lgb_scene*>(s), s->ctx->stream)) return rc;
+        CU(s->ctx, cudaStreamSynchronize(s->ctx->stream));
+    }
     SceneLayout L{};
     L.magic = kLayoutMagic; L.arena_bytes = s->bytes; L.dev = s->dev; L.cam = s->cam; L.shade = s->shade; L.max_abs = s->max_abs;
     std::memcpy(L.origin_lo, s->origin_lo, sizeof L.origin_lo); std::memcpy(L.origin_hi, s->origin_hi, sizeof L.origin_hi);
@@ -663,7 +683,7 @@ int lgb_scene_export(const lgb_scene* s, void* layout_out, uint64_t layout_bytes
     *arena_dev = s->arena; *arena_bytes = s->bytes;
     return LGB_OK;
 }
-static int build_light_grids(lgb_ctx* ctx, lgb_scene* s);
+static int build_light_grids(lgb_ctx* ctx, lgb_scene* s, cudaStream_t st);
 int lgb_scene_import(lgb_ctx* ctx, const void* layout, uint64_t layout_bytes, void* arena_dev, lgb_scene** out) {
     if (!ctx || !layout || layout_bytes < sizeof(SceneLayout) || !arena_dev || !out) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_import: bad argument");
     SceneLayout L; std::memcpy(&L, layout, sizeof L);
@@ -684,7 +704,9 @@ int lgb_scene_import(lgb_ctx* ctx, const void* layout, uint64_t layout_bytes, vo
         return off <= L.arena_bytes && bytes <= L.arena_bytes - off;
     };
     ok = ok && Ld.nodes != (const float4*)kNullOffset && within(Ld.nodes, (uint64_t)Ld.n_nodes * 64) && within(Ld.rank, (uint64_t)8 * Ld.rank_items * 4);
-    ok = ok && within(Ld.materials, 0) && within(Ld.lights, (uint64_t)Ld.n_lights * 72) && within(Ld.spaces, Ld.instanced ? nsp * sizeof(DevSpace) : 0);
+    // (the light slot holds LGB_MAX_LIGHTS records whatever the count: lgb_scene_set_lights writes it in place)
+    ok = ok && Ld.lights != (const double*)kNullOffset && within(Ld.lights, (uint64_t)LGB_MAX_LIGHTS * 72);
+    ok = ok && within(Ld.materials, 0) && within(Ld.spaces, Ld.instanced ? nsp * sizeof(DevSpace) : 0);
     ok = ok && Ld.n_lights <= LGB_MAX_LIGHTS && Ld.rank_items >= P;
     for_each_pointer(s->dev, [&](const void*& p) {
         const uint64_t off = (uint64_t)p;
@@ -692,16 +714,25 @@ int lgb_scene_import(lgb_ctx* ctx, const void* layout, uint64_t layout_bytes, vo
     });
     if (!ok) { delete s; return fail(ctx, LGB_ERR_INVALID, "lgb_scene_import: an array of the layout does not lie inside the arena"); }
     s->dev.grids = nullptr;
-    if (int rc = build_light_grids(ctx, s)) { lgb_scene_destroy(s); return rc; }
+    // the records in the slot: what lgb_scene_set_lights compares new positions with
+    s->light_dev.resize(9 * (size_t)s->dev.n_lights);
+    if (s->dev.n_lights) {
+        cudaError_t e = cudaSetDevice(ctx->device);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(s->light_dev.data(), s->dev.lights, s->light_dev.size() * 8, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) { lgb_scene_destroy(s); return cuda_fail(ctx, e, "lgb_scene_import: light records"); }
+    }
+    s->light_rec = s->light_dev;
+    if (int rc = build_light_grids(ctx, s, ctx->stream)) { lgb_scene_destroy(s); return rc; }
     *out = s;
     return LGB_OK;
 }
 double lgb_scene_build_ms(const lgb_scene* s) { return s ? s->build_ms : 0.0; }
 uint32_t lgb_scene_node_count(const lgb_scene* s) { if (!s) return 0; ensure_bvh(s->ctx, const_cast<lgb_scene*>(s)); return s->dev.n_nodes; }   // (builds a deferred tree)
 
-// Light grids (lgb_grid.cu) of a resident single-space scene, on the scene's own device and the context's stream.  A scene the
-// grids do not suit (transformed aggregates, a tiny BVH, many lights, many huge primitives) simply keeps dev.grids == NULL and its
-// shadow rays traverse the BVH.
+// Light grids (lgb_grid.cu) of a resident single-space scene for the lights in its slot (dev.lights, dev.n_lights), on the scene's
+// own device and stream `st`.  A scene the grids do not suit (transformed aggregates, a tiny BVH, many lights, many huge primitives)
+// simply keeps dev.grids == NULL and its shadow rays traverse the BVH.
 // "a BVH of >= 1024 nodes", also for a scene whose tree is deferred (leaves hold up to 4 primitives: ~n / 2 nodes)
 static bool large_scene(const DevScene& S) { return S.nodes ? S.n_nodes >= 1024u : (S.n_sph + S.n_cub + S.n_tri) / 2 >= 1024u; }
 
@@ -709,10 +740,14 @@ static bool large_scene(const DevScene& S) { return S.nodes ? S.n_nodes >= 1024u
 static cudaError_t shared_alloc(lgb_ctx* ctx, void** p, size_t bytes, cudaStream_t st) {
     return ctx->share_pool ? cudaMallocFromPoolAsync(p, bytes, ctx->share_pool, st) : cudaMallocAsync(p, bytes, st);
 }
-static int build_light_grids(lgb_ctx* ctx, lgb_scene* s) {
+static int build_light_grids(lgb_ctx* ctx, lgb_scene* s, cudaStream_t st) {
     DevScene& S = s->dev;
     S.grids = nullptr;
-    for (void* g : s->grid_allocs) cudaFreeAsync(g, ctx->stream);      // (a rebuild after ensure_bvh re-ordered the primitives)
+    if (!s->grid_allocs.empty()) {             // a rebuild (ensure_bvh re-ordered the primitives, or a light moved): a capture on another
+        CU(ctx, cudaSetDevice(ctx->device));   // stream may still read the old grids
+        if (s->last_use) CU(ctx, cudaStreamWaitEvent(st, s->last_use, 0));
+        for (void* g : s->grid_allocs) cudaFreeAsync(g, st);
+    }
     s->grid_allocs.clear(); s->grid_host.clear(); s->grid_table = nullptr; s->grid_bytes = 0;
     bool want = ctx->light_grids == 1 || (ctx->light_grids < 0 && large_scene(S) && S.n_lights <= 8u);
     // a scene made for ONE frame of known size (capture(scene, film)) must earn its grids within that frame: they cost about as much to
@@ -725,7 +760,6 @@ static int build_light_grids(lgb_ctx* ctx, lgb_scene* s) {
     if (const char* e = std::getenv("LGB_GRID_RES")) res = std::min(4096u, std::max(16u, (uint32_t)std::atoi(e)));
     const uint32_t nl = S.n_lights;
     const size_t nc = grid_cells(res), scan_bytes = grid_scan_bytes(res);
-    cudaStream_t st = ctx->stream;
     std::vector<void*> temp, mine;               // freed at the end | kept by the scene
     auto cleanup = [&](bool keep) {
         for (void* p : temp) cudaFreeAsync(p, st);
@@ -811,11 +845,13 @@ static int build_light_grids(lgb_ctx* ctx, lgb_scene* s) {
 }
 
 static int replicate_to_peers(lgb_ctx* ctx, lgb_scene* s);
+static int copy_grids_to_peers(lgb_ctx* ctx, lgb_scene* s);
 // The device BVH of a scene created without one (lgb_scene::Deferred): binned-SAH build from the kept item boxes, the primitives
 // re-written in leaf order, the grids (which index the primitive arrays) rebuilt, the peers of a device group re-supplied.
 static int ensure_bvh(lgb_ctx* ctx, lgb_scene* s) {
     if (s->dev.nodes || !s->deferred.scratch) return LGB_OK;
     if (ctx->leader) return fail(ctx, LGB_ERR_INVALID, "internal: a device-group replica cannot build its own BVH (the leader re-supplies it)");
+    if (int rc = apply_lights(ctx, s, ctx->stream)) return rc;           // the grids rebuilt below are for the lights in effect
     auto t0 = std::chrono::steady_clock::now();
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
@@ -839,7 +875,7 @@ static int ensure_bvh(lgb_ctx* ctx, lgb_scene* s) {
         for (lgb_scene* r : s->replicas) lgb_scene_destroy(r);
         s->replicas.clear();
         if (int rc = replicate_to_peers(ctx, s)) return rc;                 // (builds the leader's grids too)
-    } else if (int rc = build_light_grids(ctx, s)) return rc;
+    } else if (int rc = build_light_grids(ctx, s, st)) return rc;
     s->build_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (getenv("LGB_TIMING")) fprintf(stderr, "[ensure_bvh] deferred device BVH built on demand: %u nodes, %.2f ms\n", info.n_nodes, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
     return LGB_OK;
@@ -856,23 +892,35 @@ static int replicate_to_peers(lgb_ctx* ctx, lgb_scene* s) {
         lgb_scene* r = new lgb_scene();
         r->ctx = p; r->arena = arena; r->owns_arena = true; r->bytes = s->bytes; r->gpu_built = s->gpu_built;
         r->dev = s->dev; r->cam = s->cam; r->shade = s->shade; r->max_abs = s->max_abs;
+        r->light_rec = r->light_dev = s->light_dev; r->light_gen = r->light_applied = s->light_applied;
         std::memcpy(r->origin_lo, s->origin_lo, sizeof r->origin_lo); std::memcpy(r->origin_hi, s->origin_hi, sizeof r->origin_hi);
         r->lazy_fn = s->lazy_fn; r->lazy_user = s->lazy_user; r->lazy_desc = s->lazy_desc;
         for_each_pointer(r->dev, [&](const void*& q) { if (q) q = (const char*)arena + ((const char*)q - base); });
         s->replicas.push_back(r);
         CU(ctx, cudaMemcpyPeerAsync(arena, p->device, s->arena, ctx->device, s->bytes, p->stream));
     }
-    // the leader builds its light grids while the arenas travel; the grids then travel too (a table and three buffers per light:
-    // 98 MB for `mixed4k`) and only the pointers of the peer's table are rewritten -- rebuilding them per device cost 12 ms at 8 GPUs
-    if (int rc0 = build_light_grids(ctx, s)) return rc0;
+    // the leader builds its light grids while the arenas travel; the grids then travel too
+    if (int rc0 = build_light_grids(ctx, s, ctx->stream)) return rc0;
+    return copy_grids_to_peers(ctx, s);
+}
+
+// Device group: the leader's light grids replace every replica's (a table and three buffers per light: 98 MB for `mixed4k`); only the
+// pointers of the peer's table are rewritten -- rebuilding them per device cost 12 ms at 8 GPUs.  Returns with every peer's stream
+// drained.
+static int copy_grids_to_peers(lgb_ctx* ctx, lgb_scene* s) {
     struct Head { const uint32_t* cell_start; const uint2* entries; const uint2* large; uint32_t res, n_large; };
     std::vector<std::vector<Head>> all_heads(ctx->peers.size());      // (alive until every peer's stream is drained below)
     for (size_t k = 0; k < ctx->peers.size(); k++) {
         lgb_ctx* p = ctx->peers[k];
         lgb_scene* r = s->replicas[k];
+        CU(ctx, cudaSetDevice(p->device));
+        if (!r->grid_allocs.empty()) {                                // a capture of the replica may still read its old grids
+            if (r->last_use) CU(ctx, cudaStreamWaitEvent(p->stream, r->last_use, 0));
+            for (void* g : r->grid_allocs) cudaFreeAsync(g, p->stream);
+        }
+        r->grid_allocs.clear(); r->grid_host.clear(); r->grid_table = nullptr; r->grid_bytes = 0;
         r->dev.grids = nullptr;
         if (!s->dev.grids) continue;
-        CU(ctx, cudaSetDevice(p->device));
         const size_t nl = s->grid_host.size();
         void* tab = nullptr;
         CU(ctx, cudaMallocAsync(&tab, sizeof(DevGrid) * nl, p->stream));
@@ -899,6 +947,35 @@ static int replicate_to_peers(lgb_ctx* ctx, lgb_scene* s) {
     for (lgb_ctx* p : ctx->peers) { CU(ctx, cudaSetDevice(p->device)); CU(ctx, cudaStreamSynchronize(p->stream)); }
     CU(ctx, cudaSetDevice(ctx->device));
     return LGB_OK;
+}
+
+// The lights of lgb_scene_set_lights, applied on `st` by the first entry point that reads them (run_capture, group_capture, ensure_bvh,
+// lgb_scene_export): behind the scene's earlier captures the records go into the arena's light slot, and if a light moved or the count
+// changed the light grids are rebuilt for all of them (the same rule as at creation decides whether there are any).  An intensity,
+// falloff or ambient change rebuilds nothing: the grids list what lies between each light's position and the scene.  A device group's
+// leader applies for every replica: each replica's slot gets the records, and the leader's new grids are copied, as at creation.
+static int apply_lights(lgb_ctx* c, lgb_scene* s, cudaStream_t st) {
+    if (s->light_applied == s->light_gen) return LGB_OK;
+    const std::vector<double>& rec = s->light_rec;
+    const uint32_t n = (uint32_t)(rec.size() / 9);
+    bool moved = rec.size() != s->light_dev.size();
+    for (size_t i = 0; i < rec.size() && !moved; i += 9) moved = std::memcmp(&rec[i], &s->light_dev[i], 24) != 0;
+    CU(c, cudaSetDevice(c->device));
+    if (s->last_use) CU(c, cudaStreamWaitEvent(st, s->last_use, 0));          // captures already enqueued read the old records
+    if (n) CU(c, cudaMemcpyAsync((void*)s->dev.lights, rec.data(), rec.size() * 8, cudaMemcpyHostToDevice, st));   // (pageable: copied before the call returns)
+    s->dev.n_lights = n;
+    for (lgb_scene* r : s->replicas) {
+        CU(c, cudaSetDevice(r->ctx->device));
+        if (r->last_use) CU(c, cudaStreamWaitEvent(r->ctx->stream, r->last_use, 0));
+        if (n) CU(c, cudaMemcpyAsync((void*)r->dev.lights, rec.data(), rec.size() * 8, cudaMemcpyHostToDevice, r->ctx->stream));
+        r->dev.n_lights = n;
+        r->light_rec = r->light_dev = rec; r->light_gen = r->light_applied = s->light_gen;
+    }
+    CU(c, cudaSetDevice(c->device));
+    s->light_dev = rec; s->light_applied = s->light_gen;
+    if (!moved) return LGB_OK;
+    if (int rc = build_light_grids(c, s, st)) return rc;
+    return s->replicas.empty() ? LGB_OK : copy_grids_to_peers(c, s);
 }
 
 int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
@@ -1030,7 +1107,7 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
         const size_t o_s32 = place(ns * 16), o_s64 = place(ns * 32), o_smat = place(ns * 4), o_sid = place(ns * 4);
         const size_t o_c32 = place(ncb * 32), o_c64 = place(ncb * 48), o_cmat = place(ncb * 4), o_cid = place(ncb * 4);
         const size_t o_tri = place(nt * 48), o_nrm = place(any_normals ? nt * 36 : 0);
-        const size_t o_mat = place(mats.size() * 8), o_lights = place(d->n_lights * 72);
+        const size_t o_mat = place(mats.size() * 8), o_lights = place(LGB_MAX_LIGHTS * 72);   // room for any count (lgb_scene_set_lights)
         const size_t o_nodes = place(n * 64);
         const size_t arena_cap = off;
         // scratch: the caller's arrays as they are, the items, the builder's work space
@@ -1145,7 +1222,7 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
         if (ncb) { s->dev.cub32 = la.cub32; s->dev.cub64 = la.cub64; s->dev.cub_mat = la.cub_mat; s->dev.cub_id = la.cub_id; }
         if (nt) { s->dev.tri = la.tri; s->dev.tri_nrm = la.tri_nrm; }
         s->dev.materials = (const double*)(D + o_mat);
-        s->dev.lights = d->n_lights ? (const double*)(D + o_lights) : nullptr; s->dev.n_lights = (uint32_t)d->n_lights;
+        s->dev.lights = (const double*)(D + o_lights); s->dev.n_lights = (uint32_t)d->n_lights;
         s->dev.general = any_general; s->dev.specular = any_specular; s->dev.recursion = d->recursion;
         s->gpu_built = true;
         (void)tg0;
@@ -1182,7 +1259,7 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
     const size_t o_s32 = place(ns * 16), o_s64 = place(ns * 32), o_smat = place(ns * 4), o_sid = place(ns * 4);
     const size_t o_c32 = place(ncb * 32), o_c64 = place(ncb * 48), o_cmat = place(ncb * 4), o_cid = place(ncb * 4);
     const size_t o_tri = place(nt * 48), o_nrm = place(any_normals ? nt * 36 : 0);
-    const size_t o_mat = place(mats.size() * 8), o_lights = place(d->n_lights * 72);
+    const size_t o_mat = place(mats.size() * 8), o_lights = place(LGB_MAX_LIGHTS * 72);   // room for any count (lgb_scene_set_lights)
     const size_t arena_bytes = off;
     {
         cudaError_t e = ctx->reserve_staging(arena_bytes);
@@ -1281,9 +1358,10 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
     s->dev.materials = (const double*)(D + o_mat);
     {
         double* l = (double*)(H + o_lights);
+        std::memset(l, 0, LGB_MAX_LIGHTS * 72);
         for (uint64_t i = 0; i < d->n_lights; i++)
             for (int k = 0; k < 3; k++) { l[9 * i + k] = d->lights[i].position[k]; l[9 * i + 3 + k] = d->lights[i].intensity[k]; l[9 * i + 6 + k] = d->lights[i].falloff[k]; }
-        s->dev.lights = d->n_lights ? (const double*)(D + o_lights) : nullptr;      // (an empty array at the very end of the arena has no valid offset)
+        s->dev.lights = (const double*)(D + o_lights);
         s->dev.n_lights = (uint32_t)d->n_lights;
         s->dev.general = any_general; s->dev.specular = any_specular; s->dev.recursion = d->recursion;
     }
@@ -1296,12 +1374,13 @@ int lgb_scene_create(lgb_ctx* ctx, const lgb_scene_desc* d, lgb_scene** out) {
     s->cam = dev_camera(d->camera);
     for (int k = 0; k < 3; k++) { s->shade.ambient[k] = d->ambient[k]; s->shade.bg_inner[k] = d->bg_inner[k]; s->shade.bg_outer[k] = d->bg_outer[k]; }
     s->shade.bg_scale = d->bg_scale;
+    s->light_rec = s->light_dev = light_records(d->lights, d->n_lights);
     cudaError_t e = cudaStreamSynchronize(ctx->stream);     // the staging buffer is free for the next scene
     if (e != cudaSuccess) { cuda_fail(ctx, e, "scene upload"); return bail(LGB_ERR_CUDA); }
     s->t_total = ms_since(tc0);
     if (getenv("LGB_TIMING")) fprintf(stderr, "[lgb_scene_create] %s build: validate%s %.1f rank %.1f build %.1f (sah %.1f) convert+upload %.1f total %.1f ms, %u threads\n",
                                       s->gpu_built ? "device" : "host", s->gpu_built ? "+stage" : "", s->t_validate, s->t_rank, s->t_build, s->build_ms, s->t_convert_upload, s->t_total, (unsigned)threads);
-    if (ctx->peers.empty()) { if (int rc = build_light_grids(ctx, s)) return bail(rc); }
+    if (ctx->peers.empty()) { if (int rc = build_light_grids(ctx, s, ctx->stream)) return bail(rc); }
     else if (int rc = replicate_to_peers(ctx, s)) return bail(rc);       // (builds the leader's grids too, while the peers copy)
     *out = s;
     return LGB_OK;
@@ -1331,6 +1410,36 @@ int lgb_scene_set_camera(lgb_ctx* ctx, lgb_scene* s, const lgb_camera* cam) {
     const DevCamera d = dev_camera(*cam);
     s->cam = d; s->cam_gen++;
     for (lgb_scene* r : s->replicas) { r->cam = d; r->cam_gen++; }     // device group: every peer rebuilds its own camera grid
+    return LGB_OK;
+}
+
+// Captures take the ambient term by value (DevShade) and read the lights from the arena's slot, sized by dev.n_lights when they are
+// enqueued; the records and the light grids follow in stream order at the next entry point that reads them (apply_lights).
+int lgb_scene_set_lights(lgb_ctx* ctx, lgb_scene* s, const lgb_light* lights, uint64_t n, const double ambient[3]) {
+    if (!ctx || !s || !ambient || (n && !lights)) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_lights: NULL argument");
+    if (s->ctx != ctx) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_lights: scene does not belong to this context");
+    if (n > LGB_MAX_LIGHTS) return fail(ctx, LGB_ERR_UNSUPPORTED, "lgb_scene_set_lights: more than LGB_MAX_LIGHTS point lights");
+    const std::vector<double> rec = light_records(lights, n);
+    for (int k = 0; k < 3; k++) if (!std::isfinite(ambient[k])) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_lights: an ambient component is not finite");
+    for (double v : rec) if (!std::isfinite(v)) return fail(ctx, LGB_ERR_INVALID, "lgb_scene_set_lights: a light component is not finite");
+    // k_sbeam's f32 culling ray starts at the light: conservative for |L_k| <= kLightReach M only (DESIGN §4, "Lights")
+    double M = 0.0;
+    for (int k = 0; k < 3; k++) M = std::max(M, std::max(std::fabs(s->origin_lo[k]), std::fabs(s->origin_hi[k])));
+    const double reach = kLightReach * M;
+    for (uint64_t i = 0; i < n; i++) {
+        const double* p = lights[i].position;
+        if (std::fabs(p[0]) <= reach && std::fabs(p[1]) <= reach && std::fabs(p[2]) <= reach) continue;
+        char msg[900];
+        std::snprintf(msg, sizeof msg, "lgb_scene_set_lights: light %llu at (%.17g, %.17g, %.17g) has a coordinate beyond %.17g = %g M, where M = %.17g is the "
+                      "largest coordinate of the box [%.17g, %.17g] x [%.17g, %.17g] x [%.17g, %.17g] of the scene, its creation camera and its view box, "
+                      "from which its f32 error bound was derived (a view box holding the lights, LGB_SCENE_VIEW_BOX at lgb_scene_create, enlarges it)",
+                      (unsigned long long)i, p[0], p[1], p[2], reach, kLightReach, M,
+                      s->origin_lo[0], s->origin_hi[0], s->origin_lo[1], s->origin_hi[1], s->origin_lo[2], s->origin_hi[2]);
+        return fail(ctx, LGB_ERR_UNSUPPORTED, msg);
+    }
+    s->light_rec = rec; s->light_gen++;
+    for (int k = 0; k < 3; k++) s->shade.ambient[k] = ambient[k];
+    for (lgb_scene* r : s->replicas) for (int k = 0; k < 3; k++) r->shade.ambient[k] = ambient[k];    // (their lights: apply_lights)
     return LGB_OK;
 }
 
@@ -1539,6 +1648,7 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
     CU(c, cudaSetDevice(c->device));
     cudaStream_t st = a.stream ? a.stream : c->stream;
     if (c->last_capture) CU(c, cudaStreamWaitEvent(st, c->last_capture, 0));    // one capture at a time per context, in stream order
+    if (int rc = apply_lights(c, s, st)) return rc;
     DevWork W{};
     W.mode = a.mode; W.w = a.w; W.h = a.h;
     W.winv = 1.0 / (double)a.w; W.hinv = 1.0 / (double)a.h; W.aspect = (double)a.w / (double)a.h;   // film.rs:36-45
@@ -1799,6 +1909,8 @@ static int run_capture(lgb_ctx* c, lgb_scene* s, const CaptureArgs& a, lgb_stats
 static int group_capture(lgb_ctx* c, lgb_scene* s, uint32_t w, uint32_t h, void* film, lgb_stats* stats, bool linear = false, const lgb_guides* guides = nullptr) {
     const uint32_t n = 1 + (uint32_t)c->peers.size();
     if (s->replicas.size() != c->peers.size()) return fail(c, LGB_ERR_INVALID, "capture: the scene was not created on this device group");
+    CU(c, cudaSetDevice(c->device));
+    if (int rc = apply_lights(c, s, c->stream)) return rc;              // the leader, for every device, before anybody renders
     if (!s->dev.nodes && s->deferred.scratch) {          // deferred BVH: the leader decides for the group before anybody renders
         CU(c, cudaSetDevice(c->device));
         DevWork Wp{};

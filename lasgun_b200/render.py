@@ -29,6 +29,13 @@ class Accel:
         self.dev.set_camera(camera)
         return self
 
+    def set_lights(self, lights, ambient):
+        """Relight this resident scene: captures from now on render with `lights` ((position, intensity, falloff) triples, as
+        Scene.add_point_light takes them) and the ambient term `ambient`, without a new scene; only the light grids follow a light
+        that moved.  Returns self."""
+        self.dev.set_lights(lights, ambient)
+        return self
+
     def capture_linear(self, w: int, h: int, out=None):
         """The linear film of this resident scene: a float32 CUDA tensor (h, w, 3), enqueued on torch.cuda.current_stream()."""
         return self.dev.capture_linear(w, h, out=out)
